@@ -25,6 +25,8 @@ hold-out log-likelihood.
           /root/reference/EBEN_orig/src) -- or the oracle's C restatement when that library is
           absent -- on all host cores: the whole 2,000-fit grid when --steps <= 2, else a
           stratified sample of it (every lambda rank, every alpha) per step.
+  --dump-outputs DIR   writes the per-fit tables the last timed step of `value` computed (hold-out error, status,
+          active-set size, iterations) and its grid as DIR/<name>.npy, so that two builds can be compared output by output.
 """
 from __future__ import annotations
 
@@ -55,6 +57,19 @@ def load_workload(which: str = "binomial"):
     if which == "binomial":
         return g["BASISbinomial"].astype(np.float64), g["yBinomial"].astype(np.float64), 5
     return g["BASIS"].astype(np.float64), g["y"].astype(np.float64), 10
+
+
+def dump_outputs(out_dir: str, res, n_folds: int) -> None:
+    """--dump-outputs: what pareben_run_fits returned in the last timed step, merged over the ranks, as float64 .npy files:
+    per-fit tables of shape (grid row, fold) in BuildGrid's row order, and the grid they were computed on (its lambdas
+    come from the device's lambda_max).  The inputs are fixed (bundled data, seeded folds), so two builds compare file by file."""
+    os.makedirs(out_dir, exist_ok=True)
+    grid = res["grid"]
+    tables = {"fold_error": res["table"], "status": res["status"], "n_selected": res["nsel"], "iterations": res["iters"]}
+    for name, a in tables.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64).reshape(grid["alpha"].size, n_folds))
+    for name in ("alpha", "lambda"):
+        np.save(os.path.join(out_dir, "grid_" + name + ".npy"), np.asarray(grid[name], dtype=np.float64))
 
 
 # ------------------------------------------------------------------------------------------------
@@ -262,17 +277,20 @@ def run_gpu(args):
         table = np.zeros(n_grid * n_folds); table[mine] = err
         stat = np.zeros(n_grid * n_folds); stat[mine] = st
         nsel = np.zeros(n_grid * n_folds); nsel[mine] = ns
+        iters = np.zeros(n_grid * n_folds); iters[mine] = it
         if world > 1:
-            t = torch.from_numpy(np.stack([table, stat, nsel])).cuda()
+            t = torch.from_numpy(np.stack([table, stat, nsel, iters])).cuda()
             dist.all_reduce(t)
-            table, stat, nsel = t.cpu().numpy()
+            table, stat, nsel, iters = t.cpu().numpy()
         prob.close()
-        return {"ms_per_step": total_ms / steps, "flops": flops, "table": table, "status": stat, "nsel": nsel, "grid": grid, "folds": folds,
+        return {"ms_per_step": total_ms / steps, "flops": flops, "table": table, "status": stat, "nsel": nsel, "iters": iters, "grid": grid, "folds": folds,
                 "n_fits": n_grid * n_folds, "wall": wall, "clocks": clocks, "avoided": avoided, "gram": gram, "my_ms": float(np.mean(ms_steps)), "my_fits": int(mine.size)}
 
     X, y, n_folds = load_workload()
     n, k = X.shape
     res = resident(X, y, n_folds, "binomial", args.steps, args.warmup, ClockSampler(local))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res, n_folds)
     n_fits = res["n_fits"]
     grid, folds = res["grid"], res["folds"]
     n_grid = grid["alpha"].size
@@ -401,14 +419,23 @@ def run_gpu(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5,
+                    help="timed steps of the headline measurement and of e2e (the Gaussian extra runs min(steps, 3), "
+                         "the streaming extra one)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-extras", action="store_true", help="skip the Gaussian extras")
     ap.add_argument("--no-stream", action="store_true", help="skip the config-5 streaming extra")
     ap.add_argument("--stream-k", type=int, default=0, help="loci of the config-5 streaming extra (0: 20000 on 8 GPUs, else 5000)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the tables the last timed step of the headline measurement computed as DIR/<name>.npy "
+                         "(float64), as soon as that measurement ends; add --no-cpu --no-extras for a quick comparison run")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the CUDA path computed: it needs --impl b200")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,13 +1,14 @@
 """CPU suite: the file readers either side of the hot path (pareben_b200/io.py, rdata.py) and the command line's
-argument handling.  The .rda check runs where the reference checkout exists (this container); the text formats are
-exercised on files written here in the layout of the reference's own inputs (genotype_full.txt, pheno_left.txt)."""
+argument handling.  The .rda reader reads the bundled inputs stored as R data files under tests/golden
+(make_rda_golden.py); the text formats are exercised on files written here in the layout of the reference's own inputs
+(genotype_full.txt, pheno_left.txt)."""
 import os
 import zipfile
 
 import numpy as np
 import pytest
 
-from conftest import ROOT, golden
+from conftest import GOLDEN, golden
 
 
 def _write_genotypes(path, ids, names, M):
@@ -48,9 +49,7 @@ def test_genotype_and_phenotype_text_join(tmp_path):
 
 def test_rda_reader_against_bundled_inputs():
     from pareben_b200 import io as pio
-    d = "/root/reference/data"
-    if not os.path.isdir(d):
-        pytest.skip("reference checkout not present on this box")
+    d = GOLDEN
     g = golden("inputs_bundled.npz")
     X = pio.read_matrix(os.path.join(d, "BASIS.rda"))
     y = pio.read_matrix(os.path.join(d, "y.rda"))

@@ -3,13 +3,10 @@
  * R-layer restatement against the CrossValidate output the reference's authors published
    (paper_materials/.../LooserSubset_10000_ParCV_5-3-2018.RDS -> tests/golden/published_cv_10000.npz).
  * C restatement (oracle/eben_*.c) against golden vectors produced by the reference's own C.
- * Where oracle/_ref is present (build container), restatement vs reference live on fresh inputs.
 """
 import math
-import os
 
 import numpy as np
-import pytest
 
 from conftest import golden
 from oracle import rlayer as R
@@ -114,21 +111,19 @@ def test_local_search_replay_shape_and_rule():
     assert np.all(each[:, 2] <= 1e10)
 
 
-@pytest.mark.skipif(not os.path.exists(R.REF_LIB), reason="oracle/_ref is only built where /root/reference exists")
-def test_port_vs_reference_live_random(built):
-    rng = np.random.default_rng(7)
-    X = rng.choice([-1.0, 0.0, 1.0], size=(80, 30), p=[0.25, 0.5, 0.25])
-    y = 100 + X[:, 3] * 4 - X[:, 11] * 3 + X[:, 5] * X[:, 7] * 3 + rng.normal(0, 2, 80)
-    for epis in (False, True):
-        for lam, a in ((2.0, 1.0), (0.3, 0.5), (0.02, 0.1)):
-            f2 = R.eb_elastic_net_gaussian(X, y, lam, a, epis, R.fit_lib("port"))
-            if epis and f2.weight.shape[0] >= 50:
-                continue    # the reference writes past basisMax = 2K here and corrupts its heap (SURVEY fact 6)
-            f1 = R.eb_elastic_net_gaussian(X, y, lam, a, epis, R.fit_lib("reference"))
-            assert f1.weight.shape == f2.weight.shape
-            assert np.allclose(f1.weight[:, :4], f2.weight[:, :4], rtol=1e-8, atol=1e-12)
-            assert abs(f1.intercept[0] - f2.intercept[0]) < 1e-9 * abs(f1.intercept[0])
-            assert abs(f1.wald - f2.wald) <= 1e-8 * max(1.0, abs(f1.wald))
+def test_port_final_model_matches_reference_golden(bundled, built):
+    """The whole `.C` output of one fit -- weight table with the posterior variances, intercept, Wald statistic, residual
+    variance -- against the reference's own C on config 1 at its optimum (tests/golden/make_golden.py)."""
+    g = golden("final_gaussian_config1.npz")
+    X, y = bundled["BASIS"][:50, :100].astype(float), bundled["y"][:50]
+    f2 = R.eb_elastic_net_gaussian(X, y, float(g["lam"]), float(g["alpha"]), False, R.fit_lib("port"))
+    ref = g["raw_beta"]
+    assert f2.raw_beta.shape == ref.shape and np.array_equal(f2.raw_beta[:, :2], ref[:, :2])
+    assert np.array_equal(f2.raw_beta[:, 2] != 0, ref[:, 2] != 0) and (ref[:, 2] != 0).any()
+    assert np.allclose(f2.raw_beta[:, 2:4], ref[:, 2:4], rtol=1e-8, atol=1e-12)
+    assert abs(f2.intercept[0] - g["intercept"][0]) < 1e-9 * abs(g["intercept"][0])
+    assert abs(f2.wald - float(g["wald"])) <= 1e-8 * max(1.0, abs(float(g["wald"])))
+    assert abs(f2.resid_var - float(g["resid_var"])) <= 1e-8 * float(g["resid_var"])
 
 
 def _port_table_binom(X, y, n_folds, epis, g, rows_idx):
