@@ -18,9 +18,6 @@
 #pragma once
 #include "common.cuh"
 #include "gauss_fit.cuh"
-#ifdef PAREBEN_IMMA
-#include "imma_contract.cuh"      // experiment, off by default: exact but measured slower than the DMMA path (DESIGN.md section 4)
-#endif
 
 namespace pareben {
 
@@ -182,27 +179,6 @@ __device__ inline void binom_full_stat(const Problem &P, const FoldData &F, Slab
     //   bb = sum_h w[h] x_c[h]^2                        (BBsquare, :1728-1729)   -> S_in
     //   ze = sum_h x_c[h] e[h]                          (tempZE,  :1731-1732)    -> Q_in
     //   G[p][c] = sum_h x_c[h] phi_p[h] w[h] / s_c      (BPvector, :1693-1702)   -- kept as the action cache
-#ifdef PAREBEN_IMMA
-    if (!EPIS && F.XT8f && s.bslice) {
-        // genotype codes: the same sums on the INT8 tensor cores, exact to FP64 (imma_contract.cuh).  Columns 0..M-1 are
-        // w o phi_p, column M is e; column 0 (phi_0 = 1, the intercept) is w itself and also multiplies the squared codes.
-        __syncthreads();
-        PHASE(PH_CONTRACT);
-        const int ldt = F.ldt, R = M + 1, Rp = (R + 7) & ~7;
-        imma_slice(R, Rp, N, ldt, [&](int r, int h) { return r < M ? w[h] * s.phi[(size_t)r * LD + h] : e[h]; }, s.bslice, s.bscale);
-        __syncthreads();
-        int sc_of[2] = {-1, -1};
-        double sc_v[2] = {1.0, 1.0}, sc_i[2] = {1.0, 1.0};      // a lane emits for two candidates per tile: one division each
-        imma_pass(F.XT8f, F.XT8sqf, ldt, Kc, R, Rp, s.bslice, s.bscale, sV,
-            [&](int r, int c, double val, int half) {
-                if (r < M) {
-                    if (sc_of[half] != c) { sc_of[half] = c; sc_v[half] = scale[c]; sc_i[half] = 1.0 / sc_v[half]; }
-                    s.G[(size_t)s.grow[r] * Kc + c] = div_by(val, sc_v[half], sc_i[half]);
-                } else s.Q_in[c] = val;
-            },
-            [&](int c, double val) { s.S_in[c] = val; });
-    } else
-#endif
     contract_x<EPIS>(F, K, Kc, M, M,
         [&](int r) -> const double * { return s.phi + (size_t)r * LD; },
         [&](int r, bool &dv) -> double * { dv = true; return s.G + (size_t)s.grow[r] * Kc; },

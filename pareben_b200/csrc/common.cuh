@@ -41,8 +41,6 @@ struct FoldData {
     // to ldt (a multiple of 64).  Exactly one of the two is non-null (int8 when Xtr8 is).
     const int8_t *XT8;
     const double *XTd;
-    const int8_t *XT8f, *XT8sqf;   // binomial main-effect fits on genotype codes with |x| <= 11 (else null): XT8 and its element-wise
-                                   // squares in the fragment-major order of the int8 tensor-core contraction (imma_contract.cuh)
     int ldt;
     int ntr, nte;
     // Gaussian fits, "Gram" organisation (null otherwise): C[p][c] = x_c' phi_p / s_c for EVERY candidate p, i.e. the
@@ -89,9 +87,6 @@ struct Slab {
     double *mu, *alpha, *gamma, *tmp, *u, *colk;  // cap (+1) each
     int *used, *grow;                   // cap
     int *unused, *upos, *amap, *action, *block;   // Kc each
-    // binomial only (imma_contract.cuh): the right-hand sides of a score contraction as IM_SLICES int8 digit planes,
-    // [slice][column][position], and one power-of-two scale per column
-    int8_t *bslice; double *bscale;
 };
 
 // Each of the three cap x cap matrices is over-allocated to (cap + 32) x (cap + 8), rounded to a
@@ -110,20 +105,13 @@ __host__ __device__ inline size_t slab_doubles(int cap, int nmax, int Kc)
            (size_t)7 * (cap + 1);
 }
 __host__ __device__ inline size_t slab_ints(int cap, int Kc) { return (((size_t)2 * cap + (size_t)5 * Kc) + 3) & ~(size_t)3; }
-constexpr int IM_SLICES = 8;      // 7-bit signed digits per FP64 right-hand-side value (56 bits below the column maximum)
-__host__ __device__ inline int imma_cols(int cap) { return (cap + 2 + 7) & ~7; }          // active columns + e, + w; whole 8-column tiles
-__host__ __device__ inline int imma_ld(int nmax) { return (nmax + 63) & ~63; }            // == FoldData::ldt of the largest fold
-__host__ __device__ inline size_t slab_slice_bytes(int cap, int nmax, int binomial)
+__host__ __device__ inline size_t slab_bytes(int cap, int nmax, int Kc)
 {
-    return binomial ? (size_t)IM_SLICES * imma_cols(cap) * imma_ld(nmax) + (size_t)imma_cols(cap) * 8 : 0;
-}
-__host__ __device__ inline size_t slab_bytes(int cap, int nmax, int Kc, int binomial)
-{
-    size_t b = slab_doubles(cap, nmax, Kc) * 8 + slab_ints(cap, Kc) * 4 + slab_slice_bytes(cap, nmax, binomial);
+    size_t b = slab_doubles(cap, nmax, Kc) * 8 + slab_ints(cap, Kc) * 4;
     return (b + 255) & ~(size_t)255;
 }
 
-__device__ inline Slab carve_slab(char *base, int cap, int nmax, int Kc, int binomial)
+__device__ inline Slab carve_slab(char *base, int cap, int nmax, int Kc)
 {
     Slab s;
     double *d = reinterpret_cast<double *>(base);
@@ -142,12 +130,6 @@ __device__ inline Slab carve_slab(char *base, int cap, int nmax, int Kc, int bin
     int *i = reinterpret_cast<int *>(d);
     s.used = i; i += cap; s.grow = i; i += cap;
     s.unused = i; i += Kc; s.upos = i; i += Kc; s.amap = i; i += Kc; s.action = i; i += Kc; s.block = i; i += Kc;
-    s.bslice = nullptr; s.bscale = nullptr;
-    if (binomial) {
-        char *q = base + slab_doubles(cap, nmax, Kc) * 8 + slab_ints(cap, Kc) * 4;          // 16-byte aligned
-        s.bscale = reinterpret_cast<double *>(q);
-        s.bslice = reinterpret_cast<int8_t *>(q + (size_t)imma_cols(cap) * 8);
-    }
     return s;
 }
 

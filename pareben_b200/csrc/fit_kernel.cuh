@@ -117,11 +117,7 @@ eben_fit_kernel(Problem P, Variant v, const FitTask *__restrict__ tasks, int n_t
         const FitTask task = tasks[ti];
         const unsigned long long t_fit0 = sched_now();
         const FoldData F = P.folds[task.fold];
-        #ifdef PAREBEN_IMMA
-        Slab s = carve_slab(slabs + (size_t)blockIdx.x * slab_stride, P.cap, P.nmax, P.Kc, BINOMIAL ? 1 : 0);
-#else
-        Slab s = carve_slab(slabs + (size_t)blockIdx.x * slab_stride, P.cap, P.nmax, P.Kc, 0);
-#endif
+        Slab s = carve_slab(slabs + (size_t)blockIdx.x * slab_stride, P.cap, P.nmax, P.Kc);
 #ifdef PAREBEN_PHASE_TIMING
         if (threadIdx.x == 0 && task.out_index < FIT_TRACE_MAX) { g_fit_t0[task.out_index] = global_ns(); g_fit_block[task.out_index] = blockIdx.x; }
 #endif
@@ -152,7 +148,7 @@ fold_gram_kernel(Problem P, const int *__restrict__ fold_list, int n_fold_list, 
     const int K = P.K, Kc = P.Kc, T = blockDim.x;
     const int chunks = (Kc + GRAM_CHUNK - 1) / GRAM_CHUNK;
     const int n_items = chunks * n_fold_list;
-    Slab s = carve_slab(slabs + (size_t)blockIdx.x * slab_stride, P.cap, P.nmax, Kc, 0);
+    Slab s = carve_slab(slabs + (size_t)blockIdx.x * slab_stride, P.cap, P.nmax, Kc);
     const int rpb = min(GRAM_CHUNK, P.cap);            // right-hand sides per contraction: the slab's PHI holds `cap` columns
     for (;;) {
         __syncthreads();

@@ -153,29 +153,6 @@ __global__ void gather_vec_kernel(const double *__restrict__ y, const int *__res
     if (r < nrows) out[r] = y[rows[r]];
 }
 
-// The transposed int8 training matrix (and its element-wise squares; the caller has checked |x| <= 11) in the
-// fragment-major order of imma_contract.cuh: 16-byte piece ((mt * KP + kp) * 32 + lane) * 2 + half holds positions
-// 64 kp + 16 (lane % 4) .. + 15 of candidate 16 mt + 8 half + lane / 4 (zeros past the last candidate).
-__global__ void fragment_major_kernel(const int8_t *__restrict__ XT8, int K, int ldt, int8_t *__restrict__ out, int8_t *__restrict__ out_sq)
-{
-    const int KP = ldt >> 6;
-    const size_t n_piece = (size_t)((K + 15) >> 4) * KP * 64;
-    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_piece; i += (size_t)gridDim.x * blockDim.x) {
-        const int half = (int)(i & 1), lane = (int)((i >> 1) & 31);
-        const size_t t = i >> 6;
-        const int kp = (int)(t % KP), mt = (int)(t / KP);
-        const int c = mt * 16 + half * 8 + (lane >> 2);
-        int4 v = make_int4(0, 0, 0, 0), q = v;
-        if (c < K) {
-            v = *reinterpret_cast<const int4 *>(XT8 + (size_t)c * ldt + kp * 64 + (lane & 3) * 16);
-            auto sq = [](int w) { int o = 0; for (int b = 0; b < 4; b++) { const int x = (int)(int8_t)((unsigned)w >> (8 * b)); o |= ((x * x) & 0xff) << (8 * b); } return o; };
-            q = make_int4(sq(v.x), sq(v.y), sq(v.z), sq(v.w));
-        }
-        reinterpret_cast<int4 *>(out)[i] = v;
-        reinterpret_cast<int4 *>(out_sq)[i] = q;
-    }
-}
-
 __global__ void to_int8_kernel(const double *__restrict__ in, size_t n, int8_t *__restrict__ out)
 {
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x)
@@ -364,11 +341,7 @@ static void ensure_slabs(pareben_problem *p)
     if (p->cap < 2) p->cap = 2;
 
     // persistent grid: blocks per SM limited by memory for slabs
-    #ifdef PAREBEN_IMMA
-    p->slab_stride = slab_bytes(p->cap, p->nmax, p->kc, p->prior == PAREBEN_BINOMIAL ? 1 : 0);
-#else
-    p->slab_stride = slab_bytes(p->cap, p->nmax, p->kc, 0);
-#endif
+    p->slab_stride = slab_bytes(p->cap, p->nmax, p->kc);
     // resident blocks per SM of the kernel variant this problem will launch (asked once per variant:
     // the occupancy query, like cudaMemGetInfo below, costs up to tens of milliseconds)
     int per_sm = 1;
@@ -526,18 +499,11 @@ extern "C" int pareben_problem_create(pareben_problem **out, int device, const d
         // Genotype-coded designs (every entry an integer in [-127, 127], e.g. {-1, 0, 1}) also get an
         // int8 copy of the training matrices: the score contraction reads 1 byte instead of 8 per
         // element and widens in registers (exact).
-        bool small_int = getenv("PAREBEN_NO_INT8") == nullptr;
-        [[maybe_unused]] bool tiny_int = true;            // |x| <= 11: the squares fit in int8 too (binomial int8 contraction, experiment)
+        bool small_int = true;
         for (size_t i = 0, e = (size_t)n * k; small_int && i < e; i++) {
             const double v = basis[i];
             if (!(v >= -127.0 && v <= 127.0) || v != (double)(int)v) small_int = false;
-            if (!(v >= -11.0 && v <= 11.0)) tiny_int = false;
         }
-#ifdef PAREBEN_IMMA
-        const bool want_sq = small_int && tiny_int && prior == PAREBEN_BINOMIAL && !epis && getenv("PAREBEN_NO_IMMA") == nullptr;
-#else
-        const bool want_sq = false; (void)tiny_int;       // the int8 tensor-core contraction is an experiment (imma_contract.cuh), not built by default
-#endif
         lap("stream/events/h2d enqueue/scan");
         // row lists per fold: index 0 = all rows (only materialised when n_folds == 0)
         const int nf = n_folds;
@@ -577,7 +543,7 @@ extern "C" int pareben_problem_create(pareben_problem **out, int device, const d
                 else scales_kernel<false><<<(p->kc + 255) / 256, 256, 0, p->stream>>>(Xtr, F.ntr, k, p->kc, scale);
             }
             F.Xtr = Xtr; F.ytr = ytr; F.Xte = Xte; F.yte = yte; F.scale = scale; F.Xtr8 = nullptr;
-            F.XT8 = nullptr; F.XTd = nullptr; F.XT8f = nullptr; F.XT8sqf = nullptr; F.C = nullptr;
+            F.XT8 = nullptr; F.XTd = nullptr; F.C = nullptr;
             F.ldt = (F.ntr + 63) & ~63;      // whole stages of the contraction (KT = 64 rows)
             {
                 const dim3 tg((F.ldt + 31) / 32, (k + 31) / 32);
@@ -585,12 +551,6 @@ extern "C" int pareben_problem_create(pareben_problem **out, int device, const d
                     int8_t *t8 = p->dalloc<int8_t>((size_t)F.ldt * k + 16);
                     transpose_pad_kernel<int8_t><<<tg, blk, 0, p->stream>>>(Xtr, F.ntr, k, F.ldt, t8);
                     F.XT8 = t8;
-                    if (want_sq) {
-                        const size_t fb = (size_t)((k + 15) / 16) * 16 * F.ldt;
-                        int8_t *t8f = p->dalloc<int8_t>(fb), *t8sqf = p->dalloc<int8_t>(fb);
-                        fragment_major_kernel<<<(int)std::min<size_t>(1024, (fb / 16 + 255) / 256), 256, 0, p->stream>>>(t8, k, F.ldt, t8f, t8sqf);
-                        F.XT8f = t8f; F.XT8sqf = t8sqf;
-                    }
                 } else {
                     double *td = p->dalloc<double>((size_t)F.ldt * k + 4);
                     transpose_pad_kernel<double><<<tg, blk, 0, p->stream>>>(Xtr, F.ntr, k, F.ldt, td);
@@ -725,7 +685,7 @@ int run_fits_streaming(pareben_problem *p, int n_fits, const int *fold, const do
         CU(cudaMemsetAsync(p->d_flops, 0, 2 * sizeof(double), p->stream));
         CU(cudaMemsetAsync(d_nslots, 0, sizeof(int) * nvf, p->stream));
         StreamShared sh;
-        sh.folds = d_sf; sh.n_slots = d_nslots; sh.list_cap = list_cap; { const char *w = getenv("PAREBEN_STREAM_WIDE"); sh.wide = w ? atoi(w) : 0; } sh.warp_scratch = d_wscratch; sh.flops = p->d_flops;
+        sh.folds = d_sf; sh.n_slots = d_nslots; sh.list_cap = list_cap; sh.warp_scratch = d_wscratch; sh.flops = p->d_flops;
         FitOutputs out;
         out.fold_err = d_err; out.status = d_ints; out.n_selected = d_ints + n_fits; out.n_iter = d_ints + 2 * n_fits;
         out.m_out = nullptr; out.used_out = nullptr; out.beta_out = nullptr; out.var_out = nullptr; out.scalars_out = nullptr;
@@ -757,9 +717,9 @@ int run_fits_streaming(pareben_problem *p, int n_fits, const int *fold, const do
             if (scans > 0) { CU(cudaEventElapsedTime(&last_scan_ms, es0, es1)); scan_ms += last_scan_ms; }
             long long waiting = 0;
             double fl = 0;
-            long long waiting_a = 0;
-            for (int vf = 0; vf < nvf; vf++) { waiting += h_nslots[vf]; if (vf % STREAM_CLASSES == 0) waiting_a += h_nslots[vf]; fl += 2.0 * p->h_folds[vf / STREAM_CLASSES].ntr * (double)p->kc * h_nslots[vf]; }
-            if (timing) fprintf(stderr, "[pareben] stream round %d: %lld fits waiting (%lld with more than 7 active bases), last scan %.1f ms\n", rounds, waiting, waiting_a, last_scan_ms);
+            long long waiting_b = 0;
+            for (int vf = 0; vf < nvf; vf++) { waiting += h_nslots[vf]; if (vf % STREAM_CLASSES == 0) waiting_b += h_nslots[vf]; fl += 2.0 * p->h_folds[vf / STREAM_CLASSES].ntr * (double)p->kc * h_nslots[vf]; }
+            if (timing) fprintf(stderr, "[pareben] stream round %d: %lld fits waiting (%lld not on the initial basis), last scan %.1f ms\n", rounds, waiting, waiting_b, last_scan_ms);
             if (waiting == 0) break;
             scan_flops += fl;
             CU(cudaEventRecord(es0, p->stream));

@@ -111,23 +111,19 @@ __device__ inline double q2_threshold(double need, double sl, double l1, double 
     return lo * (1 - 1e-12);
 }
 
-// Right-hand-side classes.  A fit with a small active set brings its active columns along as extra right-hand sides,
-// so the contraction delivers g = PHI' x_c for every candidate and the epilogue computes S EXACTLY instead of
-// bounding it (the bound s_lb is loose as soon as one alpha is small, and a loose bound turns every candidate of a
-// small-lambda fit into a survivor):
+// Right-hand-side classes.  Every waiting fit brings its residual e' as one right-hand-side column:
 //   class 1 (A)   M = 1 and the basis is the initial one (candidate 1: the state of every fit of a large-lambda grid
 //                 point and of every fit's first pass, MainEff.c:1003-1090): its column phi_0 is the same vector for all
-//                 of them and rides ONCE per tile, in column 0; 63 fits per tile;
-//   class 2 (C4)  M <= 3: four columns per fit [e', phi_1..phi_3], 16 fits per tile;
-//   class 3 (C8)  M <= 7: eight columns per fit (one 8-wide DMMA tile), 8 fits per tile;
-//   class 0 (B)   larger active sets: one column per fit, the s_lb bound, survivors finished by a warp each.
-// The per-element test stays ONE comparison in every class: with u = beta_s g'SIGMA g in [0, 1), S = beta_s (1 - u), and
-// T[k] is the Q^2 threshold valid for u <= 2^-k (S >= max(s_lb, beta_s (1 - 2^-k))), k = 0..7.  Nearly every candidate of
-// a genotype design has u < 1/128 (k = 7), where the bound is within 1 % of its exact S.
+//                 of them and rides ONCE per tile, in column 0, so the contraction also delivers g = phi_0' x_c for every
+//                 candidate and the epilogue computes S EXACTLY instead of bounding it; 63 fits per tile;
+//   class 0 (B)   every other fit: one column per fit, the s_lb bound, survivors finished by a warp each.
+// The per-element test stays ONE comparison in both classes: with u = beta_s g'SIGMA g in [0, 1), S = beta_s (1 - u), and
+// T[k] is the Q^2 threshold valid for u <= 2^-k (S >= max(s_lb, beta_s (1 - 2^-k))), k = 0..7.  Class B, which has no g,
+// compares against T[0] (S >= s_lb); class A picks its bucket from u.  Nearly every candidate of a genotype design has
+// u < 1/128 (k = 7), where the bound is within 1 % of its exact S.
 struct ScanSlot { double bs, sig, l1, l2, s_lb, T[8]; };
-constexpr int STREAM_CLASSES = 4;
-__host__ __device__ inline int class_width(int cls) { return cls == 2 ? 4 : (cls == 3 ? 8 : 1); }
-__host__ __device__ inline int class_fits_per_tile(int cls) { return cls == 1 ? SN - 1 : SN / class_width(cls); }
+constexpr int STREAM_CLASSES = 2;
+__host__ __device__ inline int class_fits_per_tile(int cls) { return cls == 1 ? SN - 1 : SN; }
 
 __device__ inline void slot_thresholds(ScanSlot *sp, double need, double thr_basic, bool use_bound)
 {   // T[k] (in z^2 / ssq units) for `need`; only ever raised (atomicMax on the bit pattern: positive doubles are monotone)
@@ -159,7 +155,6 @@ struct StreamShared {
     StreamFold *folds;          // [STREAM_CLASSES * (n_folds + 1)]
     int *n_slots;               // [STREAM_CLASSES * (n_folds + 1)] fits waiting this round (advance kernel: atomicAdd; host: reset)
     int list_cap;
-    int wide;                   // classes C4 / C8 in use (PAREBEN_STREAM_WIDE=1; default 0 sends those fits to class B, measured faster on config-5 shapes)
     double *warp_scratch;       // [scan blocks][SCAN_WARPS][cap]
     double *flops;
 };

@@ -167,14 +167,13 @@ stream_advance_kernel(Problem P, Variant v, StreamFit *fits, int n_fits, StreamS
             if (!resume && !reuse) {
                 // request: publish e' and the screens, hand the fit to the scan kernel
                 (void)stream_residual(s, N, LD, s.M, s.d, s.e, sc);
-                // right-hand-side class (stream.cuh): small active sets bring their columns along
-                const int Mq = s.M;
-                const int cls = (Mq == 1 && s.used[0] == 1) ? 1 : (!sh.wide ? 0 : (Mq <= 3 ? 2 : (Mq <= 7 ? 3 : 0)));
+                // right-hand-side class (stream.cuh): a fit on the initial basis brings phi_0 along
+                const int cls = (s.M == 1 && s.used[0] == 1) ? 1 : 0;
                 const int vf = STREAM_CLASSES * s.fold + cls;
                 if (threadIdx.x == 0) s_slot = atomicAdd(sh.n_slots + vf, 1);
                 __syncthreads();
                 const int idx = s_slot, per = class_fits_per_tile(cls);
-                const int slot = (idx / per) * SN + (cls == 1 ? 1 + idx % per : (idx % per) * class_width(cls));
+                const int slot = (idx / per) * SN + (cls == 1 ? 1 + idx % per : idx % per);
                 const StreamFold SF = sh.folds[vf];
                 double *Et = SF.E + (size_t)(slot / SN) * e_tile_doubles(F.ldt);
                 double *E = Et + (size_t)(slot % SN) * SLD;
@@ -182,8 +181,6 @@ stream_advance_kernel(Problem P, Variant v, StreamFit *fits, int n_fits, StreamS
                     const size_t o = (size_t)(h / SK) * STAGE_D + (h % SK);
                     E[o] = h < N ? s.e[h] : 0.0;
                     if (cls == 1) Et[o] = h < N ? s.phi[h] : 0.0;          // every fit of the tile writes the same bytes
-                    if (cls >= 2)
-                        for (int j = 0; j < Mq; j++) E[(size_t)(1 + j) * SLD + o] = h < N ? s.phi[(size_t)j * LD + h] : 0.0;
                 }
                 if (threadIdx.x == 0) {
                     double thr_q2 = (2 * l1 + l2) * (1 - 1e-6) - 1e-10 * s.beta_s;       // Q^2 must exceed S + 2 l1 + l2 > this

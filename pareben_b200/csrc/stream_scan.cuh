@@ -157,7 +157,7 @@ __device__ inline void scan_survivor(const FoldData &F, int K, int c, double z_r
     }
 }
 
-// Cheap form of the per-element test of classes A / C: u (= beta_s g'SIGMA g, here from un-normalised products and a
+// Cheap form of the per-element test of class A: u (= beta_s g'SIGMA g, here from un-normalised products and a
 // reciprocal, inflated by 1e-6 so that it can only over-estimate) picks the bucket, one comparison decides.
 __device__ inline bool bucket_pass(const ScanSlot *sp, double z2, double ssq, double u)
 {
@@ -167,30 +167,19 @@ __device__ inline bool bucket_pass(const ScanSlot *sp, double z2, double ssq, do
     return z2 > sp->T[kb] * ssq;
 }
 
-// Classes A / C4 / C8: the contraction has delivered g_raw[j] = x_c' phi_j for the fit's M <= 7 active columns, so the
-// candidate's statistics are exact here (FullStat's formulas, NeFull2.c:1150-1185: bp = G'SIGMA, quad = bp'G), one lane.
+// Class A: the contraction has delivered g_raw = x_c' phi_0 for the fit's one active column, so the candidate's
+// statistics are exact here (FullStat's formulas, NeFull2.c:1150-1185: bp = G'SIGMA, quad = bp'G, with SIGMA = sp->sig), one lane.
 template <bool GAUSS_MAIN>
-__device__ inline void scan_exact_small(StreamFit *fit, ScanSlot *sp, int c, double z, double ssq, const double (&graw)[7], int M,
-                                        const double *__restrict__ sigma, int list_cap)
+__device__ inline void scan_exact_a(StreamFit *fit, ScanSlot *sp, int c, double z, double ssq, double g_raw, int list_cap)
 {
     const double scale = sqrt(ssq), bs = sp->bs;
-    double g[7];
-#pragma unroll
-    for (int j = 0; j < 7; j++) g[j] = j < M ? graw[j] / scale : 0.0;
-    double quad = 0;
-#pragma unroll
-    for (int j = 0; j < 7; j++)
-        if (j < M) {
-            double bp = 0;
-#pragma unroll
-            for (int p = 0; p < 7; p++) if (p < M) bp = fma(g[p], sigma[j * M + p], bp);
-            quad = fma(bp, g[j], quad);
-        }
+    const double g = g_raw / scale;
+    const double quad = fma(fma(g, sp->sig, 0.0), g, 0.0);
     const double u = bs * quad;
     int kb = 7;
     if (u >= 0.0078125) { kb = -ilogb(u) - 1; kb = kb < 0 ? 0 : (kb > 7 ? 7 : kb); }
     if (!(z * z > sp->T[kb] * ssq)) return;                     // S >= beta_s (1 - 2^-kb): its delta-ML cannot reach the cutoff
-    for (int j = 0; j < M; j++) if (fit->used[j] - 1 == c) return;
+    if (fit->used[0] - 1 == c) return;
     const double so = bs - bs * quad * bs, qo = bs * (z / scale);
     const double L = scan_decide<GAUSS_MAIN>(fit, c, so, qo, list_cap);
     if (!GAUSS_MAIN && L > 0) {
@@ -329,7 +318,7 @@ stream_scan_kernel(Problem P, StreamFit *fits, StreamShared sh)
         }
         const int n_wait = sh.n_slots[f];
         const int fits_here = min(class_fits_per_tile(cls), n_wait - rt * class_fits_per_tile(cls));
-        const int cols_live = cls == 1 ? 1 + fits_here : fits_here * class_width(cls);
+        const int cols_live = cls == 1 ? 1 + fits_here : fits_here;
         const int nt_live = (cols_live + 7) >> 3;                        // 8-column tiles that hold a waiting fit
         for (int st = 0; st < nstage; st++) {
             if (producer) produce_one();                                // stage g + 3 (its slot was released by everyone at g - 1)
@@ -372,8 +361,8 @@ stream_scan_kernel(Problem P, StreamFit *fits, StreamShared sh)
             for (int t = 0; t < 2; t++) {
                 const long long cl = cbase + 8 * t + gm;
                 const double ssq = t == 0 ? ssq0 : ssq1;
-                const double graw[7] = {t == 0 ? g0 : g1, 0, 0, 0, 0, 0, 0};
-                const double rho2 = ssq > 0 ? graw[0] * graw[0] * (1.0 / ssq) : 0.0;
+                const double graw = t == 0 ? g0 : g1;
+                const double rho2 = ssq > 0 ? graw * graw * (1.0 / ssq) : 0.0;
 #pragma unroll
                 for (int n = 0; n < 8; n++)
 #pragma unroll
@@ -383,81 +372,9 @@ stream_scan_kernel(Problem P, StreamFit *fits, StreamShared sh)
                             ScanSlot *sp = SF.par + rt * SN + col;
                             const double z = acc[t][n][i];
                             if (bucket_pass(sp, z * z, ssq, sp->bs * sp->sig * rho2))
-                                scan_exact_small<GAUSS_MAIN>(fits + SF.slot_fit[rt * SN + col], sp, (int)cl, z, ssq, graw, 1, &sp->sig, sh.list_cap);
+                                scan_exact_a<GAUSS_MAIN>(fits + SF.slot_fit[rt * SN + col], sp, (int)cl, z, ssq, graw, sh.list_cap);
                         }
                     }
-            }
-            continue;
-        }
-        if (cls == 2) {
-            // four columns per fit: (e', phi_1) in the even lane of a pair, (phi_2, phi_3) in the odd one
-#pragma unroll
-            for (int t = 0; t < 2; t++) {
-                const long long cl = cbase + 8 * t + gm;
-                const double ssq = t == 0 ? ssq0 : ssq1;
-#pragma unroll
-                for (int n = 0; n < 8; n++) {
-                    const double p0 = __shfl_xor_sync(0xffffffffu, acc[t][n][0], 1), p1 = __shfl_xor_sync(0xffffffffu, acc[t][n][1], 1);
-                    const int col = 8 * n + 2 * gk;                                   // first column of this lane pair's fit when gk is even
-                    if (!(gk & 1) && cl < Kc && col < cols_live) {
-                        ScanSlot *sp = SF.par + rt * SN + col;
-                        const double z = acc[t][n][0];
-                        if (z * z > sp->T[0] * ssq) {                                     // T[0] is the lowest threshold (S >= s_lb only)
-                            StreamFit *fit = fits + SF.slot_fit[rt * SN + col];
-                            const double graw[7] = {acc[t][n][1], p0, p1, 0, 0, 0, 0};
-                            const int M = fit->M;
-                            const double *sg = fit->sigma;
-                            double qr = 0;
-#pragma unroll
-                            for (int j = 0; j < 3; j++)
-                                if (j < M) {
-                                    double bp = 0;
-#pragma unroll
-                                    for (int p = 0; p < 3; p++) if (p < M) bp = fma(graw[p], sg[j * M + p], bp);
-                                    qr = fma(bp, graw[j], qr);
-                                }
-                            if (bucket_pass(sp, z * z, ssq, sp->bs * qr * (1.0 / ssq)))
-                                scan_exact_small<GAUSS_MAIN>(fit, sp, (int)cl, z, ssq, graw, M, sg, sh.list_cap);
-                        }
-                    }
-                }
-            }
-            continue;
-        }
-        if (cls == 3) {
-            // eight columns per fit = one n-tile: gather the quad's values into the lane with gk == 0
-#pragma unroll
-            for (int t = 0; t < 2; t++) {
-                const long long cl = cbase + 8 * t + gm;
-                const double ssq = t == 0 ? ssq0 : ssq1;
-#pragma unroll
-                for (int n = 0; n < 8; n++) {
-                    const double a0 = acc[t][n][0], a1 = acc[t][n][1];
-                    const double b0 = __shfl_xor_sync(0xffffffffu, a0, 1), b1 = __shfl_xor_sync(0xffffffffu, a1, 1);     // gk ^ 1
-                    const double c0 = __shfl_xor_sync(0xffffffffu, a0, 2), c1 = __shfl_xor_sync(0xffffffffu, a1, 2);     // gk ^ 2
-                    const double d0 = __shfl_xor_sync(0xffffffffu, b0, 2), d1 = __shfl_xor_sync(0xffffffffu, b1, 2);     // gk ^ 3
-                    const int col = 8 * n;
-                    if (gk == 0 && cl < Kc && col < cols_live) {
-                        ScanSlot *sp = SF.par + rt * SN + col;
-                        if (a0 * a0 > sp->T[0] * ssq) {
-                            StreamFit *fit = fits + SF.slot_fit[rt * SN + col];
-                            const double graw[7] = {a1, b0, b1, c0, c1, d0, d1};
-                            const int M = fit->M;
-                            const double *sg = fit->sigma;
-                            double qr = 0;
-#pragma unroll
-                            for (int j = 0; j < 7; j++)
-                                if (j < M) {
-                                    double bp = 0;
-#pragma unroll
-                                    for (int p = 0; p < 7; p++) if (p < M) bp = fma(graw[p], sg[j * M + p], bp);
-                                    qr = fma(bp, graw[j], qr);
-                                }
-                            if (bucket_pass(sp, a0 * a0, ssq, sp->bs * qr * (1.0 / ssq)))
-                                scan_exact_small<GAUSS_MAIN>(fit, sp, (int)cl, a0, ssq, graw, M, sg, sh.list_cap);
-                        }
-                    }
-                }
             }
             continue;
         }

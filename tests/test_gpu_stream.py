@@ -157,16 +157,3 @@ def test_stream_k2000_slice_against_reference_fixture(pb):
     rel = np.abs(err - want_e) / np.abs(want_e)
     assert rel.max() < 1e-8, rel
 
-
-def test_stream_wide_classes_give_the_same_table(pb, monkeypatch):
-    """PAREBEN_STREAM_WIDE=1 routes fits with up to 7 active bases through the 4- and 8-column right-hand-side classes
-    (their S is exact in the scan's epilogue); the table must not depend on that choice beyond rounding."""
-    rng = np.random.default_rng(7)
-    n, k = 200, 60
-    X = _genotypes(rng, n, k, block=10)
-    y = 50 + 2.5 * X[:, 3] - 2.0 * X[:, 40] + 3.0 * X[:, 7] * X[:, 22] - 2.5 * X[:, 31] * X[:, 55] + rng.normal(0, 2.0, n)
-    lam = np.array([1.5, 0.4, 0.1, 0.03]); alpha = np.array([1.0, 0.5, 0.1, 0.7])
-    err_n, _ = _stream_vs_oracle(pb, X, y, 3, lam, alpha, True)
-    monkeypatch.setenv("PAREBEN_STREAM_WIDE", "1")
-    err_w, _ = _stream_vs_oracle(pb, X, y, 3, lam, alpha, True)
-    assert np.max(np.abs(err_w - err_n) / np.abs(err_n)) < 1e-9
