@@ -157,6 +157,10 @@ int pareben_last_counters(pareben_problem *p, double *flops, double *kernel_ms, 
  * pareben_last_counters' model flops that the last call did not have to execute; build_ms: time the last call spent
  * building the matrices (0 once they exist; it is included in that call's kernel_ms). */
 int pareben_last_gram_info(pareben_problem *p, int *in_use, double *avoided_flops, double *build_ms);
+/* Score contraction of the binomial main-effect fits (FullStat, ElasticNetBinaryNEmainEff.c:1693-1735).  tensor_core: 1 when
+ * the problem computes it on the int8 tensor cores (every design entry an integer with |x| <= 11, exact to FP64 rounding),
+ * 0 when on the FP64 path; tc_contractions: how many contractions the last pareben_run_fits ran on the tensor cores. */
+int pareben_last_contraction_info(pareben_problem *p, int *tensor_core, double *tc_contractions);
 
 /* Solver organisation.  mode 0 (default) = automatic, 1 = cached kernel, 2 = streaming kernels.
  * The cached kernel keeps the reference's per-fit candidate cache (BASIS_PHI, one row of Kc doubles per active basis,

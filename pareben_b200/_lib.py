@@ -42,6 +42,7 @@ SIGNATURES = {
     "pareben_sl_filter": (ctypes.c_int, [_vp, ctypes.c_double, ctypes.c_double, ctypes.c_int, _ip, _dp, _ip]),
     "pareben_last_counters": (ctypes.c_int, [_vp, _dp, _dp, _ip]),
     "pareben_last_gram_info": (ctypes.c_int, [_vp, _ip, _dp, _dp]),
+    "pareben_last_contraction_info": (ctypes.c_int, [_vp, _ip, _dp]),
     "pareben_set_mode": (ctypes.c_int, [ctypes.c_int]),
     "pareben_is_streaming": (ctypes.c_int, [_vp]),
     "pareben_last_stream_counters": (ctypes.c_int, [_vp, _dp, _dp, _ip, _ip]),
@@ -215,6 +216,13 @@ class Problem:
         use = np.zeros(1, np.int32); av = np.zeros(1); ms = np.zeros(1)
         _check(load().pareben_last_gram_info(self._h, _i(use), _d(av), _d(ms)))
         return bool(use[0]), float(av[0]), float(ms[0])
+
+    def contraction_info(self):
+        """(binomial score contraction on the int8 tensor cores, contractions the last run_fits ran there)
+        (include/pareben.h, pareben_last_contraction_info)."""
+        tc = np.zeros(1, np.int32); n = np.zeros(1)
+        _check(load().pareben_last_contraction_info(self._h, _i(tc), _d(n)))
+        return bool(tc[0]), int(n[0])
 
 
 def cv_grid(BASIS, Target, fold_id, n_folds, alpha, lam, epis=False, prior="gaussian", device=None,

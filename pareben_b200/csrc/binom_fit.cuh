@@ -18,6 +18,7 @@
 #pragma once
 #include "common.cuh"
 #include "gauss_fit.cuh"
+#include "tc_contract.cuh"
 
 namespace pareben {
 
@@ -26,6 +27,7 @@ struct BinomState {
     int n_unused;
     int status;
     double flops;
+    double tc_calls;  // score contractions run on the int8 tensor cores
 };
 
 // z = sum_j phi_j[h] mu[j] and z2 = the same for row h2, j ascending: two rows per thread keep twice the loads of the
@@ -152,7 +154,7 @@ __device__ inline bool post_mode(Slab &s, BinomState &b, int N, const double *t,
     return current;                        // (IRLS work is not counted in the score-pass model)
 }
 
-template <bool EPIS>
+template <bool EPIS, bool TC>
 __device__ inline void binom_full_stat(const Problem &P, const FoldData &F, Slab &s, BinomState &b, double *sV,
                                        const Scratch &sc)
 {   // fEBCatFullStat* (NEmainEff.c:1633-1803, NeFull.c:848-993)
@@ -179,10 +181,11 @@ __device__ inline void binom_full_stat(const Problem &P, const FoldData &F, Slab
     //   bb = sum_h w[h] x_c[h]^2                        (BBsquare, :1728-1729)   -> S_in
     //   ze = sum_h x_c[h] e[h]                          (tempZE,  :1731-1732)    -> Q_in
     //   G[p][c] = sum_h x_c[h] phi_p[h] w[h] / s_c      (BPvector, :1693-1702)   -- kept as the action cache
-    contract_x<EPIS>(F, K, Kc, M, M,
-        [&](int r) -> const double * { return s.phi + (size_t)r * LD; },
-        [&](int r, bool &dv) -> double * { dv = true; return s.G + (size_t)s.grow[r] * Kc; },
-        sV, w, e, s.S_in, s.Q_in);
+    // on the int8 tensor cores where the fold carries their operand images (tc_contract.cuh), else in FP64 (DMMA)
+    auto phi_col = [&](int r) -> const double * { return s.phi + (size_t)r * LD; };
+    auto g_row = [&](int r, bool &dv) -> double * { dv = true; return s.G + (size_t)s.grow[r] * Kc; };
+    if constexpr (TC) { tc_contract(F, Kc, M, phi_col, g_row, w, e, s.S_in, s.Q_in, s.planes, sV, *sc.tc); b.tc_calls += 1; }
+    else contract_x<EPIS>(F, K, Kc, M, M, phi_col, g_row, sV, w, e, s.S_in, s.Q_in);
     quad_forms(s, s.sigma, s.sigma_new, M, Kc, nullptr, sc.sweep, [&](int c, double quad, double) {
         const double sc_c = scale[c];
         s.S_in[c] = s.S_in[c] / (sc_c * sc_c) - quad;
@@ -192,14 +195,15 @@ __device__ inline void binom_full_stat(const Problem &P, const FoldData &F, Slab
     refresh_out(s, M - 1, Kc);
 }
 
-template <bool EPIS>
+// TC: the score contraction runs on the int8 tensor cores (tc_contract.cuh; main effects, FoldData::Xtc present)
+template <bool EPIS, bool TC>
 __device__ void binom_fit(const Problem &P, const FoldData &F, const Variant &v, Slab &s, double lambda,
                           double alpha_en, const FitTask &task, const FitOutputs &out, double *sV, const Scratch &sc)
 {
     const int N = F.ntr, K = P.K, Kc = P.Kc, cap = P.cap, T = blockDim.x, LD = phi_ld(N);   // cap counts the intercept slot
     const int lane_ = threadIdx.x & 31, wid_ = threadIdx.x >> 5, nw_ = T >> 5;
     const double *X = F.Xtr, *t = F.ytr, *scale = F.scale;
-    BinomState b; b.M = 2; b.n_unused = 0; b.status = 0; b.flops = 0;
+    BinomState b; b.M = 2; b.n_unused = 0; b.status = 0; b.flops = 0; b.tc_calls = 0;
     for (int j = threadIdx.x; j < cap + 1; j += T) { if (j < cap) s.grow[j] = j; s.alpha[j] = 0; s.mu[j] = 0; }
     __syncthreads();
     double vk = 1e-30, vk0, err = 1000, loglik = 0;
@@ -260,7 +264,7 @@ __device__ void binom_fit(const Problem &P, const FoldData &F, const Variant &v,
         __syncthreads();
         b.n_unused = block_compact(Kc, [&](int c) { return s.amap[c] < 0; }, s.unused, s.upos, 1, sc);
         const int initial = s.used[0];
-        binom_full_stat<EPIS>(P, F, s, b, sV, sc);
+        binom_full_stat<EPIS, TC>(P, F, s, b, sV, sc);
         int selected = ACT_NONE, last = 0, n_update = 0, jj = -1, i_iter = 0;
         const int it_max = iter == 1 ? 10 : 100;
         loglik = 1e-30;
@@ -451,7 +455,7 @@ __device__ void binom_fit(const Problem &P, const FoldData &F, const Variant &v,
                     }
                     __syncthreads();
                     }
-                    if (iu == n_update - 1) binom_full_stat<EPIS>(P, F, s, b, sV, sc);          // after the last action of the block (:749-762)
+                    if (iu == n_update - 1) binom_full_stat<EPIS, TC>(P, F, s, b, sV, sc);          // after the last action of the block (:749-762)
                 }
             }
             if (selected == ACT_TERM && ini_removed) last = 1;
@@ -513,7 +517,7 @@ __device__ void binom_fit(const Problem &P, const FoldData &F, const Variant &v,
         if (out.status) out.status[o] = b.status;
         if (out.n_selected) out.n_selected[o] = nsel;
         if (out.n_iter) out.n_iter[o] = iter;
-        if (out.flops) atomicAdd(out.flops, b.flops);
+        if (out.flops) { atomicAdd(out.flops, b.flops); if (b.tc_calls > 0) atomicAdd(out.flops + 2, b.tc_calls); }
         if (out.m_out) {
             out.m_out[0] = M - 1;
             double wd = 0;

@@ -47,12 +47,17 @@ struct FoldData {
     // row the reference's CacheBP* (MainEff.c:1144-1201) would compute for basis p.  It depends on the fold only -- not
     // on alpha, lambda or the solver's state -- so it is built once per fold (fold_gram_kernel) and shared by all fits.
     double *C;
+    // Binomial main-effect fits on designs of integers with |x| <= 11 (null otherwise): the transposed training matrix and
+    // its elementwise square as int8 operand images of the tensor-core score contraction (tc_contract.cuh), zero-padded
+    // to whole 128-candidate tiles and 32-row stages.
+    const int8_t *Xtc, *Xtcsq;
 };
 
 struct Problem {
     int N, K, Kc, n_folds, epis, prior;
     int cap;                 // basis cap actually used (<= the reference's basisMax)
     int nmax;                // max ntr over folds
+    int tc;                  // 1 when the folds carry the int8 operand images (FoldData::Xtc): the slabs then hold digit planes
     const FoldData *folds;   // [n_folds + 1]; index 0 = all rows, f = rows with fold_id != f
 };
 
@@ -72,7 +77,8 @@ struct FitOutputs {
     int *status, *n_selected, *n_iter;
     // optional full-model dump for pareben_fit (batch of 1)
     int *m_out; int *used_out; double *beta_out; double *var_out; double *scalars_out; // wald, intercept0, intercept1, extra
-    double *flops;           // two accumulators (atomicAdd): [0] model flops (SURVEY 8d), [1] the part the Gram organisation avoided
+    double *flops;           // three accumulators (atomicAdd): [0] model flops (SURVEY 8d), [1] the part the Gram organisation avoided,
+                             // [2] score contractions run on the int8 tensor cores
 };
 
 // Per-block slab carved out of one big allocation.
@@ -87,6 +93,7 @@ struct Slab {
     double *mu, *alpha, *gamma, *tmp, *u, *colk;  // cap (+1) each
     int *used, *grow;                   // cap
     int *unused, *upos, *amap, *action, *block;   // Kc each
+    int8_t *planes;                     // digit planes of the tensor-core contraction (tc_planes_bytes), or null
 };
 
 // Each of the three cap x cap matrices is over-allocated to (cap + 32) x (cap + 8), rounded to a
@@ -105,13 +112,19 @@ __host__ __device__ inline size_t slab_doubles(int cap, int nmax, int Kc)
            (size_t)7 * (cap + 1);
 }
 __host__ __device__ inline size_t slab_ints(int cap, int Kc) { return (((size_t)2 * cap + (size_t)5 * Kc) + 3) & ~(size_t)3; }
-__host__ __device__ inline size_t slab_bytes(int cap, int nmax, int Kc)
+__host__ __device__ inline size_t slab_base_bytes(int cap, int nmax, int Kc)
 {
     size_t b = slab_doubles(cap, nmax, Kc) * 8 + slab_ints(cap, Kc) * 4;
     return (b + 255) & ~(size_t)255;
 }
+// right-hand-side digit planes of the tensor-core contraction: 8 planes x 30 columns x the training rows rounded up to 32
+__host__ __device__ inline size_t tc_planes_bytes(int nmax) { return (size_t)30 * 8 * (size_t)((nmax + 31) & ~31); }
+__host__ __device__ inline size_t slab_bytes(int cap, int nmax, int Kc, int tc)
+{
+    return slab_base_bytes(cap, nmax, Kc) + (tc ? (tc_planes_bytes(nmax) + 255) & ~(size_t)255 : 0);
+}
 
-__device__ inline Slab carve_slab(char *base, int cap, int nmax, int Kc)
+__device__ inline Slab carve_slab(char *base, int cap, int nmax, int Kc, int tc)
 {
     Slab s;
     double *d = reinterpret_cast<double *>(base);
@@ -130,6 +143,7 @@ __device__ inline Slab carve_slab(char *base, int cap, int nmax, int Kc)
     int *i = reinterpret_cast<int *>(d);
     s.used = i; i += cap; s.grow = i; i += cap;
     s.unused = i; i += Kc; s.upos = i; i += Kc; s.amap = i; i += Kc; s.action = i; i += Kc; s.block = i; i += Kc;
+    s.planes = tc ? reinterpret_cast<int8_t *>(base + slab_base_bytes(cap, nmax, Kc)) : nullptr;
     return s;
 }
 
@@ -154,8 +168,47 @@ __device__ inline unsigned long long global_ns() { unsigned long long t; asm vol
 #endif
 
 // ------------------------------------------------------------------------------------------
+// mbarrier and bulk-copy (TMA) helpers
+__device__ inline unsigned smem_u32(const void *p) { return (unsigned)__cvta_generic_to_shared(p); }
+
+__device__ inline void mbar_init(unsigned long long *bar, int count)
+{
+    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
+}
+__device__ inline void mbar_arrive(unsigned long long *bar)
+{
+    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
+}
+__device__ inline void mbar_expect_tx(unsigned long long *bar, unsigned bytes)
+{
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
+}
+__device__ inline void mbar_wait(unsigned long long *bar, unsigned parity)
+{
+    asm volatile(
+        "{\n"
+        ".reg .pred p;\n"
+        "WAIT_LOOP:\n"
+        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
+        "@p bra WAIT_DONE;\n"
+        "bra WAIT_LOOP;\n"
+        "WAIT_DONE:\n"
+        "}\n" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
+}
+// global -> shared bulk copy executed by the TMA unit (SASS: UBLKCP), completion counted in bytes on `bar`
+__device__ inline void bulk_load(void *dst_smem, const void *src_gmem, unsigned bytes, unsigned long long *bar)
+{
+    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+                 ::"r"(smem_u32(dst_smem)), "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar)) : "memory");
+}
+
+// ------------------------------------------------------------------------------------------
 // block-level primitives.  `red` is a shared scratch of >= 33 doubles, `redi` >= 33 ints.
-struct Scratch { double *red; int *redi; double *sweep; /* SWEEP_SMEM_M^2 + 2*SWEEP_SMEM_M doubles, or null */ };
+struct TcState;
+struct Scratch {
+    double *red; int *redi; double *sweep; /* SWEEP_SMEM_M^2 + 2*SWEEP_SMEM_M doubles, or null */
+    TcState *tc;                           // tensor-core contraction state (binomial main-effect kernel with Problem::tc), or null
+};
 
 __device__ inline double warp_sum(double v)
 {

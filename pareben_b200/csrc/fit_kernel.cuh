@@ -1,6 +1,7 @@
 // fit_kernel.cuh -- the persistent batched-fit kernel and its per-variant host launchers.
-// Each of the four (Epis, prior) variants is compiled in its own translation unit (fit_gm.cu,
-// fit_ge.cu, fit_bm.cu, fit_be.cu) so that the build runs four ptxas jobs in parallel; the host
+// Each of the four (Epis, prior) variants, and the binomial main-effect variant with the tensor-core score contraction,
+// is compiled in its own translation unit (fit_gm.cu, fit_ge.cu, fit_bm.cu, fit_be.cu, fit_bt.cu) so that the build runs
+// the ptxas jobs in parallel; the host
 // side (pareben.cu) reaches them through the plain functions declared in fit_launch.h.
 #pragma once
 #include "common.cuh"
@@ -21,6 +22,7 @@ constexpr int SWEEP_DOUBLES = SWEEP_SMEM_M * SWEEP_SMEM_M + 2 * SWEEP_SMEM_M;
 constexpr int QUAD_DOUBLES = cmax(2 * QT * LDS_V + 784, cmax(4096 + 1040, GRAM_PIPE_DOUBLES));
 constexpr int S_BUF_DOUBLES = cmax(cmax(cmax(SWEEP_DOUBLES, SWEEP_PANEL_DOUBLES), cmax(SV_DOUBLES, COL_MAX_ROWS)), cmax(GRAM_DOUBLES, QUAD_DOUBLES));
 constexpr size_t S_BUF_BYTES = (size_t)S_BUF_DOUBLES * sizeof(double);
+static_assert(TC_SMEM_BYTES <= S_BUF_BYTES, "the tensor-core contraction's ring must fit the shared buffer");
 
 __device__ inline unsigned long long sched_now()
 {
@@ -97,7 +99,9 @@ __device__ inline int next_task(const FitTask *__restrict__ tasks, int n_tasks, 
     }
 }
 
-template <bool EPIS, bool BINOMIAL>
+// TC (binomial main effects only): the score contraction on the int8 tensor cores, a separate instantiation so that the
+// kernels of every other design carry no tensor-memory allocation (it changes the occupancy query and the register allocation)
+template <bool EPIS, bool BINOMIAL, bool TC>
 __global__ void __launch_bounds__(FIT_THREADS, PAREBEN_MIN_BLOCKS)
 eben_fit_kernel(Problem P, Variant v, const FitTask *__restrict__ tasks, int n_tasks, Sched sched, char *slabs,
                 size_t slab_stride, FitOutputs out)
@@ -110,24 +114,28 @@ eben_fit_kernel(Problem P, Variant v, const FitTask *__restrict__ tasks, int n_t
     __shared__ double red[66];
     __shared__ int redi[66];
     __shared__ int s_task;
-    Scratch sc{red, redi, s_buf};
+    Scratch sc{red, redi, s_buf, nullptr};
+    static_assert(!TC || (BINOMIAL && !EPIS), "the tensor-core contraction serves binomial main-effect fits");
+    __shared__ TcState tcs;
+    if constexpr (TC) { tc_open(tcs); sc.tc = &tcs; }
     for (bool first = true;; first = false) {
         const int ti = next_task(tasks, n_tasks, sched, first, sc, &s_task);
         if (ti < 0) break;
         const FitTask task = tasks[ti];
         const unsigned long long t_fit0 = sched_now();
         const FoldData F = P.folds[task.fold];
-        Slab s = carve_slab(slabs + (size_t)blockIdx.x * slab_stride, P.cap, P.nmax, P.Kc);
+        Slab s = carve_slab(slabs + (size_t)blockIdx.x * slab_stride, P.cap, P.nmax, P.Kc, P.tc);
 #ifdef PAREBEN_PHASE_TIMING
         if (threadIdx.x == 0 && task.out_index < FIT_TRACE_MAX) { g_fit_t0[task.out_index] = global_ns(); g_fit_block[task.out_index] = blockIdx.x; }
 #endif
-        if (BINOMIAL) binom_fit<EPIS>(P, F, v, s, task.lambda, task.alpha, task, out, sV, sc);
+        if (BINOMIAL) binom_fit<EPIS, TC>(P, F, v, s, task.lambda, task.alpha, task, out, sV, sc);
         else gauss_fit<EPIS>(P, F, v, s, task.lambda, task.alpha, task, out, sV, sc);
         if (threadIdx.x == 0) atomicMax(sched.cost + task.group, sched_now() - t_fit0 + 1);
 #ifdef PAREBEN_PHASE_TIMING
         if (threadIdx.x == 0 && task.out_index < FIT_TRACE_MAX) g_fit_t1[task.out_index] = global_ns();
 #endif
     }
+    if constexpr (TC) tc_close(tcs);
 }
 
 
@@ -148,7 +156,7 @@ fold_gram_kernel(Problem P, const int *__restrict__ fold_list, int n_fold_list, 
     const int K = P.K, Kc = P.Kc, T = blockDim.x;
     const int chunks = (Kc + GRAM_CHUNK - 1) / GRAM_CHUNK;
     const int n_items = chunks * n_fold_list;
-    Slab s = carve_slab(slabs + (size_t)blockIdx.x * slab_stride, P.cap, P.nmax, Kc);
+    Slab s = carve_slab(slabs + (size_t)blockIdx.x * slab_stride, P.cap, P.nmax, Kc, P.tc);
     const int rpb = min(GRAM_CHUNK, P.cap);            // right-hand sides per contraction: the slab's PHI holds `cap` columns
     for (;;) {
         __syncthreads();
@@ -191,23 +199,23 @@ inline cudaError_t launch_gram_variant(int grid, int threads, cudaStream_t strea
     return cudaGetLastError();
 }
 
-template <bool EPIS, bool BINOMIAL>
+template <bool EPIS, bool BINOMIAL, bool TC>
 inline cudaError_t launch_fit_variant(int grid, int threads, cudaStream_t stream, const Problem &P, const Variant &v,
                                       const FitTask *tasks, int n_tasks, const Sched &sched, char *slabs, size_t slab_stride,
                                       const FitOutputs &out)
 {
-    cudaError_t e = cudaFuncSetAttribute(eben_fit_kernel<EPIS, BINOMIAL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S_BUF_BYTES);
+    cudaError_t e = cudaFuncSetAttribute(eben_fit_kernel<EPIS, BINOMIAL, TC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S_BUF_BYTES);
     if (e != cudaSuccess) return e;
-    eben_fit_kernel<EPIS, BINOMIAL><<<grid, threads, S_BUF_BYTES, stream>>>(P, v, tasks, n_tasks, sched, slabs, slab_stride, out);
+    eben_fit_kernel<EPIS, BINOMIAL, TC><<<grid, threads, S_BUF_BYTES, stream>>>(P, v, tasks, n_tasks, sched, slabs, slab_stride, out);
     return cudaGetLastError();
 }
 
-template <bool EPIS, bool BINOMIAL>
+template <bool EPIS, bool BINOMIAL, bool TC>
 inline cudaError_t occupancy_variant(int *blocks_per_sm, int threads)
 {
-    cudaError_t e = cudaFuncSetAttribute(eben_fit_kernel<EPIS, BINOMIAL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S_BUF_BYTES);
+    cudaError_t e = cudaFuncSetAttribute(eben_fit_kernel<EPIS, BINOMIAL, TC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S_BUF_BYTES);
     if (e != cudaSuccess) return e;
-    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, eben_fit_kernel<EPIS, BINOMIAL>, threads, S_BUF_BYTES);
+    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, eben_fit_kernel<EPIS, BINOMIAL, TC>, threads, S_BUF_BYTES);
 }
 
 // experiments only (timing build): copy out / reset this translation unit's phase counters and fit trace
@@ -230,13 +238,13 @@ inline void timing_variant(unsigned long long *cycles_calls, int reset, unsigned
 
 }  // namespace pareben
 
-#define PAREBEN_DEFINE_VARIANT(NAME, EPIS, BINOMIAL)                                                                      \
+#define PAREBEN_DEFINE_VARIANT(NAME, EPIS, BINOMIAL, TC)                                                                      \
     namespace pareben {                                                                                                   \
     cudaError_t launch_fit_##NAME(int grid, int threads, cudaStream_t stream, const Problem &P, const Variant &v,        \
                                   const FitTask *tasks, int n_tasks, const Sched &sched, char *slabs, size_t slab_stride,         \
                                   const FitOutputs &out)                                                                  \
-    { return launch_fit_variant<EPIS, BINOMIAL>(grid, threads, stream, P, v, tasks, n_tasks, sched, slabs, slab_stride, out); } \
-    cudaError_t occupancy_##NAME(int *blocks_per_sm, int threads) { return occupancy_variant<EPIS, BINOMIAL>(blocks_per_sm, threads); } \
+    { return launch_fit_variant<EPIS, BINOMIAL, TC>(grid, threads, stream, P, v, tasks, n_tasks, sched, slabs, slab_stride, out); } \
+    cudaError_t occupancy_##NAME(int *blocks_per_sm, int threads) { return occupancy_variant<EPIS, BINOMIAL, TC>(blocks_per_sm, threads); } \
     void timing_##NAME(unsigned long long *cc, int reset, unsigned long long *t0, unsigned long long *t1, int *block, int n) \
     { timing_variant(cc, reset, t0, t1, block, n); }                                                                      \
     }

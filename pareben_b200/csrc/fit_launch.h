@@ -1,4 +1,4 @@
-// fit_launch.h -- host-callable entry points of the four kernel translation units.
+// fit_launch.h -- host-callable entry points of the five kernel translation units.
 #pragma once
 #include "common.cuh"
 
@@ -17,6 +17,7 @@ PAREBEN_DECLARE_VARIANT(gm)   // Gaussian, main effects
 PAREBEN_DECLARE_VARIANT(ge)   // Gaussian, Epis
 PAREBEN_DECLARE_VARIANT(bm)   // binomial, main effects
 PAREBEN_DECLARE_VARIANT(be)   // binomial, Epis
+PAREBEN_DECLARE_VARIANT(bt)   // binomial, main effects, score contraction on the int8 tensor cores (Problem::tc)
 
 // Gaussian only: build FoldData::C for the listed folds (fold_gram_kernel, fit_kernel.cuh)
 cudaError_t launch_gram_gm(int grid, int threads, cudaStream_t stream, const Problem &P, const int *fold_list, int n_fold_list,

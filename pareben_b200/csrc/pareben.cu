@@ -5,6 +5,7 @@
 //  the hot loops use explicit fma()).
 #include "../../include/pareben.h"
 #include "common.cuh"
+#include "tc_contract.cuh"
 #include "fit_launch.h"
 #include "stream_launch.h"
 
@@ -159,6 +160,21 @@ __global__ void to_int8_kernel(const double *__restrict__ in, size_t n, int8_t *
         out[i] = (int8_t)in[i];
 }
 
+// The int8 operand images of the tensor-core contraction (tc_contract.cuh): X' and X o X' in the UMMA canonical K-major
+// layout, [128-candidate tile][32-row stage], zero-padded to whole tiles and stages.
+__global__ void tc_image_kernel(const double *__restrict__ X, int nrows, int K, int nst, int ntile, int8_t *__restrict__ img,
+                                int8_t *__restrict__ sq)
+{
+    const int cols = ntile * TC_TILE;
+    const size_t n = (size_t)cols * nst * TC_KS;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
+        const int c = (int)(i % cols), h = (int)(i / cols);
+        const int x = (c < K && h < nrows) ? (int)X[(size_t)h * K + c] : 0;
+        const size_t o = tc_image_offset(c, h, nst);
+        img[o] = (int8_t)x; sq[o] = (int8_t)(x * x);
+    }
+}
+
 // Transposed, row-padded copy of a row-major matrix: out[k*ldt + r] = X[r*K + k] (zero for r >= nrows), as int8 or f64.
 template <class T>
 __global__ void transpose_pad_kernel(const double *__restrict__ X, int nrows, int K, int ldt, T *__restrict__ out)
@@ -278,6 +294,7 @@ __global__ void sl_stat_kernel(const double *__restrict__ X, int N, int K, int c
 // ---------------------------------------------------------------------------------------------
 struct pareben_problem {
     int device = 0;
+    int tc = 0;                          // the folds carry the int8 operand images of the tensor-core contraction (FoldData::Xtc)
     int n = 0, k = 0, kc = 0, n_folds = 0, epis = 0, prior = 0, cap = 0, nmax = 0, min_ntr = 0;
     int sm_count = 0;
     std::vector<PoolEntry> allocs;       // every device buffer of this problem (returned to the pool on destroy)
@@ -295,6 +312,7 @@ struct pareben_problem {
     int gram_state = 0;                  // 0 = undecided, 1 = in use, -1 = refused (memory or too little work)
     double gram_ms = 0; int gram_launches = 0;      // time / launches spent building C in the last run_fits call
     double last_avoided = 0;             // model flops of the last call that the Gram organisation did not execute
+    double last_tc_calls = 0;            // score contractions the last call ran on the int8 tensor cores
     long long grid_fits_hint = 0;        // fits of the WHOLE grid a sharded call belongs to (0 = unknown): the work test must not
                                          // depend on how many ways the grid is split, or 1- and 8-GPU tables could differ in rounding
     double last_scan_ms = 0, last_scan_flops = 0; int last_scan_launches = 0, last_rounds = 0;
@@ -341,7 +359,7 @@ static void ensure_slabs(pareben_problem *p)
     if (p->cap < 2) p->cap = 2;
 
     // persistent grid: blocks per SM limited by memory for slabs
-    p->slab_stride = slab_bytes(p->cap, p->nmax, p->kc);
+    p->slab_stride = slab_bytes(p->cap, p->nmax, p->kc, p->tc);
     // resident blocks per SM of the kernel variant this problem will launch (asked once per variant:
     // the occupancy query, like cudaMemGetInfo below, costs up to tens of milliseconds)
     int per_sm = 1;
@@ -349,15 +367,19 @@ static void ensure_slabs(pareben_problem *p)
         // Block size: measured on B200 (config 2 / bundled Gaussian): 256 threads x 2 blocks per SM beats
         // 128 x 4 (-5 % / -43 %) and 64 x 8 (-40 % / -70 %) (measured with an earlier build that had a run-time block size).
         p->threads = FIT_THREADS_HOST;     // gram_tiled() maps 16 x 16 register blocks onto exactly 256 threads
-        static int occ_cache[4] = {0, 0, 0, 0};
-        int &occ = occ_cache[(p->prior == PAREBEN_BINOMIAL ? 2 : 0) + (p->epis ? 1 : 0)];
+        static int occ_cache[5] = {0, 0, 0, 0, 0};
+        int &occ = occ_cache[p->tc ? 4 : (p->prior == PAREBEN_BINOMIAL ? 2 : 0) + (p->epis ? 1 : 0)];
         if (!occ) {
             cudaError_t e;
             if (p->prior == PAREBEN_GAUSSIAN) e = p->epis ? occupancy_ge(&occ, p->threads) : occupancy_gm(&occ, p->threads);
-            else e = p->epis ? occupancy_be(&occ, p->threads) : occupancy_bm(&occ, p->threads);
+            else e = p->epis ? occupancy_be(&occ, p->threads) : p->tc ? occupancy_bt(&occ, p->threads) : occupancy_bm(&occ, p->threads);
             CU(e);
         }
         per_sm = std::max(1, occ);
+        // The occupancy calculator counts one block per SM for any kernel that contains a tensor-memory allocation.  Two blocks
+        // of the tensor-core variant fit its registers and shared memory and take 256 of the SM's 512 TMEM columns each
+        // (tc_contract.cuh); measured resident and running side by side on B200.
+        if (p->tc) per_sm = std::max(per_sm, 2);
     }
     const char *env_bps = getenv("PAREBEN_BLOCKS_PER_SM");
     if (env_bps) per_sm = std::max(1, std::min(per_sm, atoi(env_bps)));
@@ -437,7 +459,7 @@ static void ensure_gram(pareben_problem *p, int n_fits, const int *fold)
     CU(cudaMemcpyAsync(p->d_folds, p->h_folds.data(), sizeof(FoldData) * p->h_folds.size(), cudaMemcpyHostToDevice, p->stream));
     Problem P;
     P.N = p->n; P.K = p->k; P.Kc = p->kc; P.n_folds = p->n_folds; P.epis = p->epis; P.prior = p->prior;
-    P.cap = p->cap; P.nmax = p->nmax; P.folds = p->d_folds;
+    P.cap = p->cap; P.nmax = p->nmax; P.tc = p->tc; P.folds = p->d_folds;
     const int chunks = (p->kc + 31) / 32;
     const int grid = (int)std::min<long long>(p->n_slabs, (long long)chunks * (long long)need.size());
     CU(cudaEventRecord(p->ev0, p->stream));
@@ -500,10 +522,17 @@ extern "C" int pareben_problem_create(pareben_problem **out, int device, const d
         // int8 copy of the training matrices: the score contraction reads 1 byte instead of 8 per
         // element and widens in registers (exact).
         bool small_int = true;
+        double max_abs = 0;
         for (size_t i = 0, e = (size_t)n * k; small_int && i < e; i++) {
             const double v = basis[i];
             if (!(v >= -127.0 && v <= 127.0) || v != (double)(int)v) small_int = false;
+            max_abs = std::max(max_abs, std::fabs(v));
         }
+        // Binomial main-effect fits on such designs with |x| <= 11 (x^2 fits int8) run the score contraction on the int8
+        // tensor cores (tc_contract.cuh); every other design keeps the FP64 contraction.  The int32 sums of one digit plane
+        // are bounded by rows x max|x|^2 x 64, which must stay below 2^31 (about 277,000 training rows at |x| = 11).
+        p->tc = small_int && max_abs <= 11.0 && (double)n * max_abs * max_abs * 64.0 < 2147483648.0 && !epis &&
+                prior == PAREBEN_BINOMIAL && !p->streaming;
         lap("stream/events/h2d enqueue/scan");
         // row lists per fold: index 0 = all rows (only materialised when n_folds == 0)
         const int nf = n_folds;
@@ -543,7 +572,7 @@ extern "C" int pareben_problem_create(pareben_problem **out, int device, const d
                 else scales_kernel<false><<<(p->kc + 255) / 256, 256, 0, p->stream>>>(Xtr, F.ntr, k, p->kc, scale);
             }
             F.Xtr = Xtr; F.ytr = ytr; F.Xte = Xte; F.yte = yte; F.scale = scale; F.Xtr8 = nullptr;
-            F.XT8 = nullptr; F.XTd = nullptr; F.C = nullptr;
+            F.XT8 = nullptr; F.XTd = nullptr; F.C = nullptr; F.Xtc = nullptr; F.Xtcsq = nullptr;
             F.ldt = (F.ntr + 63) & ~63;      // whole stages of the contraction (KT = 64 rows)
             {
                 const dim3 tg((F.ldt + 31) / 32, (k + 31) / 32);
@@ -562,6 +591,13 @@ extern "C" int pareben_problem_create(pareben_problem **out, int device, const d
                 to_int8_kernel<<<std::min<size_t>(1024, ((size_t)F.ntr * k + 255) / 256), 256, 0, p->stream>>>(Xtr, (size_t)F.ntr * k, x8);
                 F.Xtr8 = x8;
             }
+            if (p->tc) {
+                const int nst = (F.ntr + TC_KS - 1) / TC_KS, ntile = (k + TC_TILE - 1) / TC_TILE;
+                const size_t bytes = (size_t)ntile * nst * TC_A_BYTES;
+                int8_t *img = p->dalloc<int8_t>(2 * bytes);
+                tc_image_kernel<<<(int)std::min<size_t>(1024, (bytes + 255) / 256), 256, 0, p->stream>>>(Xtr, F.ntr, k, nst, ntile, img, img + bytes);
+                F.Xtc = img; F.Xtcsq = img + bytes;
+            }
         }
         CU(cudaGetLastError());
         lap("per-fold layout (enqueue)");
@@ -569,7 +605,7 @@ extern "C" int pareben_problem_create(pareben_problem **out, int device, const d
         CU(cudaMemcpyAsync(p->d_folds, p->h_folds.data(), sizeof(FoldData) * (nf + 1), cudaMemcpyHostToDevice, p->stream));
 
         p->min_ntr = min_ntr;
-        p->d_flops = p->dalloc<double>(2);
+        p->d_flops = p->dalloc<double>(3);
         CU(cudaStreamSynchronize(p->stream));
         lap("final sync");
     } catch (std::pair<int, std::string> &e) {
@@ -699,7 +735,7 @@ int run_fits_streaming(pareben_problem *p, int n_fits, const int *fold, const do
         }
         Problem P;
         P.N = p->n; P.K = p->k; P.Kc = p->kc; P.n_folds = p->n_folds; P.epis = p->epis; P.prior = p->prior;
-        P.cap = cap; P.nmax = p->nmax; P.folds = p->d_folds;
+        P.cap = cap; P.nmax = p->nmax; P.tc = p->tc; P.folds = p->d_folds;
         const Variant v = make_variant(p->epis, p->prior);
         auto advance = [&] { CU((p->epis ? launch_stream_advance_ge : launch_stream_advance_gm)(n_fits, p->stream, P, v, d_fits, sh, out)); };
         auto scan = [&] { CU((p->epis ? launch_stream_scan_ge : launch_stream_scan_gm)(scan_grid, p->stream, P, d_fits, sh)); };
@@ -819,7 +855,7 @@ int run_fits_impl(pareben_problem *p, int n_fits, const int *fold, const double 
         sched.t_start = d_sched; sched.cost = d_sched + n_groups; sched.taken = reinterpret_cast<int *>(d_sched + 2 * (size_t)n_groups);
         CU(cudaMemcpyAsync(d_tasks, tasks.data(), sizeof(FitTask) * n_fits, cudaMemcpyHostToDevice, p->stream));
         CU(cudaMemsetAsync(d_sched, 0, sched_bytes, p->stream));
-        CU(cudaMemsetAsync(p->d_flops, 0, 2 * sizeof(double), p->stream));
+        CU(cudaMemsetAsync(p->d_flops, 0, 3 * sizeof(double), p->stream));
         FitOutputs out;
         out.fold_err = d_err; out.status = d_ints; out.n_selected = d_ints + n_fits; out.n_iter = d_ints + 2 * n_fits;
         out.m_out = nullptr; out.used_out = nullptr; out.beta_out = nullptr; out.var_out = nullptr; out.scalars_out = nullptr;
@@ -833,7 +869,7 @@ int run_fits_impl(pareben_problem *p, int n_fits, const int *fold, const double 
         }
         Problem P;
         P.N = p->n; P.K = p->k; P.Kc = p->kc; P.n_folds = p->n_folds; P.epis = p->epis; P.prior = p->prior;
-        P.cap = p->cap; P.nmax = p->nmax; P.folds = p->d_folds;
+        P.cap = p->cap; P.nmax = p->nmax; P.tc = p->tc; P.folds = p->d_folds;
         const Variant v = make_variant(p->epis, p->prior);
         int grid = std::min(p->n_slabs, n_fits);
         // A launch with few fits per SM (one shard of a grid split over 8 GPUs: 250 fits for 148 SMs): a binomial fit that has
@@ -847,17 +883,18 @@ int run_fits_impl(pareben_problem *p, int n_fits, const int *fold, const double 
         if (p->prior == PAREBEN_GAUSSIAN)
             CU((p->epis ? launch_fit_ge : launch_fit_gm)(grid, p->threads, p->stream, P, v, d_tasks, n_fits, sched, p->d_slabs, p->slab_stride, out));
         else
-            CU((p->epis ? launch_fit_be : launch_fit_bm)(grid, p->threads, p->stream, P, v, d_tasks, n_fits, sched, p->d_slabs, p->slab_stride, out));
+            CU((p->epis ? launch_fit_be : p->tc ? launch_fit_bt : launch_fit_bm)(grid, p->threads, p->stream, P, v, d_tasks, n_fits, sched, p->d_slabs, p->slab_stride, out));
         CU(cudaEventRecord(p->ev1, p->stream));
         std::vector<int> h_ints(3 * (size_t)n_fits);
         std::vector<double> h_err(n_fits);
         CU(cudaMemcpyAsync(h_err.data(), d_err, sizeof(double) * n_fits, cudaMemcpyDeviceToHost, p->stream));
         CU(cudaMemcpyAsync(h_ints.data(), d_ints, sizeof(int) * 3 * n_fits, cudaMemcpyDeviceToHost, p->stream));
-        double h_flops2[2] = {0, 0};
-        CU(cudaMemcpyAsync(h_flops2, p->d_flops, 2 * sizeof(double), cudaMemcpyDeviceToHost, p->stream));
+        double h_flops2[3] = {0, 0, 0};
+        CU(cudaMemcpyAsync(h_flops2, p->d_flops, 3 * sizeof(double), cudaMemcpyDeviceToHost, p->stream));
         CU(cudaStreamSynchronize(p->stream));
         const double h_flops = h_flops2[0];
         p->last_avoided = h_flops2[1];
+        p->last_tc_calls = h_flops2[2];
         float ms = 0;
         CU(cudaEventElapsedTime(&ms, p->ev0, p->ev1));
         p->last_ms = ms + p->gram_ms; p->last_flops = h_flops; p->last_launches = 1 + p->gram_launches;      // a call that had to build C pays for it
@@ -1224,13 +1261,13 @@ extern "C" int pareben_sl_filter(pareben_problem *p, double tau_main, double tau
 }
 
 // experiments only (timing build, -DPAREBEN_PHASE_TIMING; absent from the product library): cycles per phase summed over
-// blocks and over the four kernel variants.  out: PH_COUNT cycle totals then PH_COUNT call counts.
+// blocks and over the five kernel variants.  out: PH_COUNT cycle totals then PH_COUNT call counts.
 #ifdef PAREBEN_PHASE_TIMING
 extern "C" int pareben_phase_cycles(unsigned long long *out, int reset)
 {
     unsigned long long acc[2 * PH_COUNT] = {0}, one[2 * PH_COUNT];
-    void (*fn[4])(unsigned long long *, int, unsigned long long *, unsigned long long *, int *, int) = {timing_gm, timing_ge, timing_bm, timing_be};
-    for (int i = 0; i < 4; i++) {
+    void (*fn[5])(unsigned long long *, int, unsigned long long *, unsigned long long *, int *, int) = {timing_gm, timing_ge, timing_bm, timing_be, timing_bt};
+    for (int i = 0; i < 5; i++) {
         for (int j = 0; j < 2 * PH_COUNT; j++) one[j] = 0;
         fn[i](one, reset, nullptr, nullptr, nullptr, 0);
         for (int j = 0; j < 2 * PH_COUNT; j++) acc[j] += one[j];
@@ -1240,11 +1277,11 @@ extern "C" int pareben_phase_cycles(unsigned long long *out, int reset)
 }
 
 // experiments only: per-fit start/end (%globaltimer ns) and block id of the last launch of variant
-// `which` (0 gm, 1 ge, 2 bm, 3 be).
+// `which` (0 gm, 1 ge, 2 bm, 3 be, 4 bt).
 extern "C" int pareben_fit_trace(int which, unsigned long long *t0, unsigned long long *t1, int *block, int n)
 {
-    void (*fn[4])(unsigned long long *, int, unsigned long long *, unsigned long long *, int *, int) = {timing_gm, timing_ge, timing_bm, timing_be};
-    if (which < 0 || which > 3) return 0;
+    void (*fn[5])(unsigned long long *, int, unsigned long long *, unsigned long long *, int *, int) = {timing_gm, timing_ge, timing_bm, timing_be, timing_bt};
+    if (which < 0 || which > 4) return 0;
     fn[which](nullptr, 0, t0, t1, block, n);
     return n;
 }
@@ -1269,6 +1306,13 @@ extern "C" int pareben_last_stream_counters(pareben_problem *p, double *scan_ms,
     return PAREBEN_OK;
 }
 
+extern "C" int pareben_last_contraction_info(pareben_problem *p, int *tensor_core, double *tc_contractions)
+{
+    if (!p) return fail(PAREBEN_EINVAL, "null problem");
+    if (tensor_core) *tensor_core = p->tc;
+    if (tc_contractions) *tc_contractions = p->last_tc_calls;
+    return PAREBEN_OK;
+}
 extern "C" int pareben_last_gram_info(pareben_problem *p, int *in_use, double *avoided_flops, double *build_ms)
 {
     if (!p) return fail(PAREBEN_EINVAL, "null problem");

@@ -81,7 +81,7 @@ stream_advance_kernel(Problem P, Variant v, StreamFit *fits, int n_fits, StreamS
     __shared__ double red[66];
     __shared__ int redi[66];
     __shared__ int s_slot;
-    Scratch sc{red, redi, s_buf};
+    Scratch sc{red, redi, s_buf, nullptr};
     if ((int)blockIdx.x >= n_fits) return;
     StreamFit &G = fits[blockIdx.x];
     if (G.phase == SP_DONE) return;

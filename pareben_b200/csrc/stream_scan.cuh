@@ -28,39 +28,6 @@
 
 namespace pareben {
 
-__device__ inline unsigned smem_u32(const void *p) { return (unsigned)__cvta_generic_to_shared(p); }
-
-__device__ inline void mbar_init(unsigned long long *bar, int count)
-{
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ inline void mbar_arrive(unsigned long long *bar)
-{
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ inline void mbar_expect_tx(unsigned long long *bar, unsigned bytes)
-{
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ inline void mbar_wait(unsigned long long *bar, unsigned parity)
-{
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "WAIT_LOOP:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-        "@p bra WAIT_DONE;\n"
-        "bra WAIT_LOOP;\n"
-        "WAIT_DONE:\n"
-        "}\n" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
-}
-// global -> shared bulk copy executed by the TMA unit (SASS: UBLKCP), completion counted in bytes on `bar`
-__device__ inline void bulk_load(void *dst_smem, const void *src_gmem, unsigned bytes, unsigned long long *bar)
-{
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(smem_u32(dst_smem)), "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar)) : "memory");
-}
-
 // physical position of row h inside the transposed matrices (rows of every group of 16 permuted, see transpose_pad_kernel)
 __device__ inline int perm_row(int h) { return (h & ~15) | ((h & 3) << 2) | ((h >> 2) & 3); }
 

@@ -31,7 +31,8 @@ with pb.Problem(X, y, folds, nf, False, prior) as p:
     lib.pareben_fit_trace.restype = ctypes.c_int
     nf_ = fold.size
     t0 = np.zeros(nf_, np.uint64); t1 = np.zeros(nf_, np.uint64); blk = np.zeros(nf_, np.int32)
-    got = lib.pareben_fit_trace(2 if prior == 'binomial' else 0, t0.ctypes.data_as(ctypes.c_void_p), t1.ctypes.data_as(ctypes.c_void_p), blk.ctypes.data_as(ctypes.c_void_p), nf_)
+    which = 0 if prior != 'binomial' else (4 if p.contraction_info()[0] else 2)      # bt: the tensor-core variant
+    got = lib.pareben_fit_trace(which, t0.ctypes.data_as(ctypes.c_void_p), t1.ctypes.data_as(ctypes.c_void_p), blk.ctypes.data_as(ctypes.c_void_p), nf_)
     if got:
         start = t0.min(); dur = (t1 - t0).astype(float) * 1e-6; end = (t1.max() - start) * 1e-6
         busy = dur.sum() / (end * (blk.max() + 1))
