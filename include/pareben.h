@@ -61,6 +61,16 @@ int pareben_problem_create(pareben_problem **out, int device, const double *basi
                            const double *target, const int *fold_id, int n_folds, int epis, int prior);
 void pareben_problem_destroy(pareben_problem *p);
 
+/* Several responses, one design (QTL traits measured on the same genotypes, permuted copies of one response):
+ * pareben_problem_create with targets an n x n_targets column-major matrix, one response per column.  The design-side
+ * data (per-fold training matrices, column norms, Gram matrices, streaming buffers) exist once and serve every response;
+ * only the training and test vectors are kept per (response, fold).  Every fit of such a problem gives bitwise the result
+ * of the same fit on a problem created with that response alone.  pareben_problem_create is the n_targets = 1 case.
+ * pareben_fit, pareben_lambda_max, pareben_sl_filter and pareben_problem_cv_grid fail with PAREBEN_EINVAL on a problem
+ * with n_targets > 1 (use the _multi calls; the final model of a response is fitted on a single-response problem). */
+int pareben_problem_create_multi(pareben_problem **out, int device, const double *basis, int n, int k,
+                                 const double *targets, int n_targets, const int *fold_id, int n_folds, int epis, int prior);
+
 /* The library keeps one per-device work buffer alive between calls (allocating several GB per
  * CrossValidate would dominate small problems); this releases it. */
 void pareben_release_cache(void);
@@ -73,6 +83,12 @@ void pareben_release_cache(void);
  * n_selected (number of non-zero effects), n_iter (outer iterations). */
 int pareben_run_fits(pareben_problem *p, int n_fits, const int *fold, const double *alpha,
                      const double *lambda, double *fold_err, int *status, int *n_selected, int *n_iter);
+
+/* pareben_run_fits for a problem with several responses: fit i trains on response target[i] (0 .. n_targets - 1).
+ * Fits of every response share one launch (cached kernels) or the same lock-step rounds and scans (streaming mode); when
+ * the streaming states of all fits do not fit in device memory, whole responses run in successive waves. */
+int pareben_run_fits_multi(pareben_problem *p, int n_fits, const int *target, const int *fold, const double *alpha,
+                           const double *lambda, double *fold_err, int *status, int *n_selected, int *n_iter);
 
 /* One-shot grid call with host buffers: the replacement for the foreach loop of
  * R/CrossValidate.R:66-70 / 88-92.  Grid point g (alpha[g], lambda[g]) x fold f (1..n_folds)
@@ -98,6 +114,17 @@ int pareben_cv_grid(const double *basis, int n, int k, const double *target, con
  * grid and a LocalSearch refinement then share ONE upload and one set of per-fold layouts.  Same outputs, same shard rule. */
 int pareben_problem_cv_grid(pareben_problem *p, const double *alpha, const double *lambda, int n_grid, int shard,
                             int n_shards, double *fold_err, int *status, int *n_selected);
+
+/* pareben_cv_grid / pareben_problem_cv_grid for n_targets responses (targets n x n_targets column-major).  alpha and lambda
+ * are n_targets x n_grid, response-major (entry t * n_grid + g: each response has its own grid, from its own lambda_max);
+ * the tables are response-major, then grid, then fold: fit (t * n_grid + g) * n_folds + (f - 1).  That is the numbering of
+ * pareben_cv_grid on n_targets * n_grid grid points with the flattened lambda, and shards are dealt by pareben_shard_plan on
+ * exactly that (n_grid' = n_targets * n_grid).  One upload and one set of per-fold layouts per device serve all responses. */
+int pareben_cv_grid_multi(const double *basis, int n, int k, const double *targets, int n_targets, const int *fold_id,
+                          int n_folds, const double *alpha, const double *lambda, int n_grid, int epis, int prior,
+                          int n_devices, int device, int shard, int n_shards, double *fold_err, int *status, int *n_selected);
+int pareben_problem_cv_grid_multi(pareben_problem *p, const double *alpha, const double *lambda, int n_grid, int shard,
+                                  int n_shards, double *fold_err, int *status, int *n_selected);
 
 /* The shard assignment pareben_cv_grid uses, exposed for the host layer and tests (host-only
  * logic, needs no device): writes the ascending fit numbers of `shard` into fit_index
@@ -133,6 +160,9 @@ void ElasticNetBinaryNEfull(double *BASIS, double *Targets, double *a_Lambda, do
 /* lambda_max of R/BuildGrid.R:5-32 (before the x10), computed on the device for the problem's
  * full data; epis taken from the problem. */
 int pareben_lambda_max(pareben_problem *p, double *lambda_max);
+/* pareben_lambda_max of every response of the problem (lambda_max[n_targets]) in one pass over the candidates; each value
+ * is bitwise the one pareben_lambda_max gives on a problem holding that response alone. */
+int pareben_lambda_max_multi(pareben_problem *p, double *lambda_max);
 
 /* Single-locus prefilter of the published workflow, the step before CrossValidate
  * (paper_materials/Real Data Analysis/SL_filter.R:17-52): standardise the response and every candidate column with

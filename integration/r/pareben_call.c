@@ -6,6 +6,7 @@
  *
  * Entry points (all registered below):
  *   pareben_cv_grid_call     CrossValidate / LocalSearch: the whole (alpha, lambda) x fold table, nDevices GPUs
+ *   pareben_cv_grid_multi_call  the same for the T columns of a response matrix against one BASIS, in one call
  *   pareben_lambda_max_call  GetLambdaMax (R/BuildGrid.R:5-32), incl. the K^2/2 pair scan of Epis = "yes"
  *   pareben_fit_call         EBelasticNet.Gaussian / .Binomial: the `.C` outputs of one all-rows fit
  *   pareben_sl_filter_call   the single-locus prefilter of SL_filter.R
@@ -56,6 +57,36 @@ SEXP pareben_cv_grid_call(SEXP BASIS, SEXP Target, SEXP foldId, SEXP nFolds, SEX
     SEXP items[] = {err, st, ns};
     SEXP out = named_list(3, names, items);
     UNPROTECT(3);
+    return out;
+}
+
+/* .Call("pareben_cv_grid_multi_call", BASIS, Targets, foldId, nFolds, alpha, lambda, epis, prior, nDevices, device)
+ * Targets: n x T double matrix, one response per column (traits of one design, permuted copies of one response).
+ * alpha, lambda: nGrid x T matrices, column t = the grid of response t (its own BuildGrid / GetLambdaMax).
+ * returns list(fold_err = array[nFolds x nGrid x T], status, n_selected): slice [, , t] is what pareben_cv_grid_call
+ * returns for Targets[, t] alone, bitwise (pareben_cv_grid_multi's table order, fold fastest). */
+SEXP pareben_cv_grid_multi_call(SEXP BASIS, SEXP Targets, SEXP foldId, SEXP nFolds, SEXP alpha, SEXP lambda,
+                                SEXP epis, SEXP prior, SEXP nDevices, SEXP device)
+{
+    int n, k, nt, ng;
+    dims(BASIS, &n, &k);
+    dims(Targets, &nt, &ng);          /* rows, responses */
+    if (nt != n) error("Targets must have nrow(BASIS) rows");
+    const int T = ng, nf = asInteger(nFolds);
+    if (T < 1 || LENGTH(alpha) % T != 0) error("alpha must be an nGrid x ncol(Targets) matrix");
+    ng = LENGTH(alpha) / T;
+    if (ng < 1 || LENGTH(foldId) != n || LENGTH(lambda) != LENGTH(alpha)) error("argument lengths disagree");
+    SEXP dim = PROTECT(allocVector(INTSXP, 3));
+    INTEGER(dim)[0] = nf; INTEGER(dim)[1] = ng; INTEGER(dim)[2] = T;
+    SEXP err = PROTECT(allocArray(REALSXP, dim)), st = PROTECT(allocArray(INTSXP, dim)), ns = PROTECT(allocArray(INTSXP, dim));
+    const int rc = pareben_cv_grid_multi(REAL(BASIS), n, k, REAL(Targets), T, INTEGER(foldId), nf, REAL(alpha), REAL(lambda), ng,
+                                         asInteger(epis), asInteger(prior), asInteger(nDevices), asInteger(device), 0, 1,
+                                         REAL(err), INTEGER(st), INTEGER(ns));
+    if (rc != PAREBEN_OK) { UNPROTECT(4); error("pareben_cv_grid_multi failed (%d): %s", rc, pareben_last_error()); }
+    const char *names[] = {"fold_err", "status", "n_selected"};
+    SEXP items[] = {err, st, ns};
+    SEXP out = named_list(3, names, items);
+    UNPROTECT(4);
     return out;
 }
 
@@ -124,6 +155,7 @@ SEXP pareben_sl_filter_call(SEXP BASIS, SEXP Target, SEXP tauMain, SEXP tauPair,
 
 static const R_CallMethodDef call_methods[] = {
     {"pareben_cv_grid_call", (DL_FUNC)&pareben_cv_grid_call, 10},
+    {"pareben_cv_grid_multi_call", (DL_FUNC)&pareben_cv_grid_multi_call, 10},
     {"pareben_lambda_max_call", (DL_FUNC)&pareben_lambda_max_call, 4},
     {"pareben_fit_call", (DL_FUNC)&pareben_fit_call, 7},
     {"pareben_sl_filter_call", (DL_FUNC)&pareben_sl_filter_call, 6},

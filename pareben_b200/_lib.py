@@ -25,6 +25,8 @@ _vp = ctypes.c_void_p
 SIGNATURES = {
     "pareben_problem_create": (ctypes.c_int, [ctypes.POINTER(_vp), ctypes.c_int, _dp, ctypes.c_int, ctypes.c_int, _dp, _ip,
                                               ctypes.c_int, ctypes.c_int, ctypes.c_int]),
+    "pareben_problem_create_multi": (ctypes.c_int, [ctypes.POINTER(_vp), ctypes.c_int, _dp, ctypes.c_int, ctypes.c_int, _dp,
+                                                    ctypes.c_int, _ip, ctypes.c_int, ctypes.c_int, ctypes.c_int]),
     "pareben_problem_destroy": (None, [_vp]),
     "pareben_release_cache": (None, []),
     "pareben_run_fits": (ctypes.c_int, [_vp, ctypes.c_int, _ip, _dp, _dp, _dp, _ip, _ip, _ip]),
@@ -32,6 +34,11 @@ SIGNATURES = {
                                        ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, _dp, _ip,
                                        _ip]),
     "pareben_problem_cv_grid": (ctypes.c_int, [_vp, _dp, _dp, ctypes.c_int, ctypes.c_int, ctypes.c_int, _dp, _ip, _ip]),
+    "pareben_run_fits_multi": (ctypes.c_int, [_vp, ctypes.c_int, _ip, _ip, _dp, _dp, _dp, _ip, _ip, _ip]),
+    "pareben_cv_grid_multi": (ctypes.c_int, [_dp, ctypes.c_int, ctypes.c_int, _dp, ctypes.c_int, _ip, ctypes.c_int, _dp, _dp,
+                                             ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int,
+                                             ctypes.c_int, _dp, _ip, _ip]),
+    "pareben_problem_cv_grid_multi": (ctypes.c_int, [_vp, _dp, _dp, ctypes.c_int, ctypes.c_int, ctypes.c_int, _dp, _ip, _ip]),
     "elasticNetLinearNeMainEff": (None, [_dp, _dp, _dp, _dp, _dp, _dp, _dp, _ip, _ip, _ip, _dp]),
     "elasticNetLinearNeEpisEff": (None, [_dp, _dp, _dp, _dp, _dp, _dp, _dp, _ip, _ip, _ip, _dp]),
     "ElasticNetBinaryNEmainEff": (None, [_dp, _dp, _dp, _dp, _dp, _dp, _dp, _dp, _ip, _ip, _ip, _ip]),
@@ -39,6 +46,7 @@ SIGNATURES = {
     "pareben_shard_plan": (ctypes.c_int, [_dp, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, _ip, _ip]),
     "pareben_fit": (ctypes.c_int, [_vp, ctypes.c_double, ctypes.c_double, _dp, _dp, _dp, _dp, _ip]),
     "pareben_lambda_max": (ctypes.c_int, [_vp, _dp]),
+    "pareben_lambda_max_multi": (ctypes.c_int, [_vp, _dp]),
     "pareben_sl_filter": (ctypes.c_int, [_vp, ctypes.c_double, ctypes.c_double, ctypes.c_int, _ip, _dp, _ip]),
     "pareben_last_counters": (ctypes.c_int, [_vp, _dp, _dp, _ip]),
     "pareben_last_gram_info": (ctypes.c_int, [_vp, _ip, _dp, _dp]),
@@ -111,18 +119,35 @@ def default_device() -> int:
         return 0
 
 
+def _targets_matrix(Targets, n: int) -> np.ndarray:
+    """An n x T response matrix as the column-major doubles pareben_*_multi take; every shape is checked here."""
+    Y = np.asarray(Targets, dtype=np.float64)
+    if Y.ndim != 2 or Y.shape[0] != n:
+        raise ValueError(f"Targets must be an n x T matrix with n = nrow(BASIS) = {n}; got shape {Y.shape}")
+    if Y.shape[1] < 1:
+        raise ValueError("Targets must hold at least one response (T >= 1)")
+    return np.asfortranarray(Y)
+
+
 class Problem:
-    """One CrossValidate problem resident on a GPU (pareben_problem_create)."""
+    """One CrossValidate problem resident on a GPU (pareben_problem_create).  A 2-D Target of shape (n, T) makes a problem
+    with T responses sharing the design (pareben_problem_create_multi); a 1-D Target is the single-response problem."""
 
     def __init__(self, BASIS, Target, fold_id=None, n_folds: int = 0, epis: bool = False, prior: str = "gaussian",
                  device: int | None = None):
         lib = load()
         device = default_device() if device is None else int(device)
         self._X = np.asfortranarray(np.asarray(BASIS, dtype=np.float64))
-        self._y = np.ascontiguousarray(np.asarray(Target, dtype=np.float64).ravel())
         n, k = self._X.shape
-        if self._y.size != n:
-            raise ValueError("Target length must equal nrow(BASIS)")
+        multi = np.ndim(Target) == 2
+        if multi:
+            self._y = _targets_matrix(Target, n)
+            self.n_targets = self._y.shape[1]
+        else:
+            self._y = np.ascontiguousarray(np.asarray(Target, dtype=np.float64).ravel())
+            self.n_targets = 1
+            if self._y.size != n:
+                raise ValueError("Target length must equal nrow(BASIS)")
         self.n, self.k, self.n_folds, self.epis = n, k, int(n_folds), bool(epis)
         self.prior = GAUSSIAN if prior == "gaussian" else BINOMIAL
         fid = None
@@ -131,8 +156,12 @@ class Problem:
             if fid.size != n:
                 raise ValueError("fold_id length must equal nrow(BASIS)")
         self._h = _vp()
-        _check(lib.pareben_problem_create(ctypes.byref(self._h), device, _d(self._X), n, k, _d(self._y),
-                                          _i(fid) if fid is not None else None, self.n_folds, int(self.epis), self.prior))
+        if multi:
+            _check(lib.pareben_problem_create_multi(ctypes.byref(self._h), device, _d(self._X), n, k, _d(self._y), self.n_targets,
+                                                    _i(fid) if fid is not None else None, self.n_folds, int(self.epis), self.prior))
+        else:
+            _check(lib.pareben_problem_create(ctypes.byref(self._h), device, _d(self._X), n, k, _d(self._y),
+                                              _i(fid) if fid is not None else None, self.n_folds, int(self.epis), self.prior))
 
     def close(self):
         if getattr(self, "_h", None):
@@ -147,13 +176,22 @@ class Problem:
     def __exit__(self, *exc):
         self.close()
 
-    def run_fits(self, fold, alpha, lam):
+    def run_fits(self, fold, alpha, lam, target=None):
+        """(fold_err, status, n_selected, n_iter) of independent fits; target: response index of each fit (None: response 0)."""
         fold = np.ascontiguousarray(fold, dtype=np.int32)
         alpha = np.ascontiguousarray(alpha, dtype=np.float64)
         lam = np.ascontiguousarray(lam, dtype=np.float64)
         m = fold.size
+        if alpha.size != m or lam.size != m:
+            raise ValueError("fold, alpha and lambda must have equal length")
         err = np.empty(m); st = np.empty(m, np.int32); ns = np.empty(m, np.int32); it = np.empty(m, np.int32)
-        _check(load().pareben_run_fits(self._h, m, _i(fold), _d(alpha), _d(lam), _d(err), _i(st), _i(ns), _i(it)))
+        if target is None:
+            _check(load().pareben_run_fits(self._h, m, _i(fold), _d(alpha), _d(lam), _d(err), _i(st), _i(ns), _i(it)))
+        else:
+            target = np.ascontiguousarray(target, dtype=np.int32)
+            if target.size != m:
+                raise ValueError("target must have one entry per fit")
+            _check(load().pareben_run_fits_multi(self._h, m, _i(target), _i(fold), _d(alpha), _d(lam), _d(err), _i(st), _i(ns), _i(it)))
         return err, st, ns, it
 
     def cv_grid(self, alpha, lam, shard: int = 0, n_shards: int = 1):
@@ -167,6 +205,20 @@ class Problem:
         err = np.zeros(total); st = np.zeros(total, np.int32); ns = np.zeros(total, np.int32)
         _check(load().pareben_problem_cv_grid(self._h, _d(alpha), _d(lam), alpha.size, int(shard), int(n_shards), _d(err), _i(st), _i(ns)))
         return err.reshape(alpha.size, nf), st.reshape(alpha.size, nf), ns.reshape(alpha.size, nf)
+
+    def cv_grid_multi(self, alpha, lam, shard: int = 0, n_shards: int = 1):
+        """pareben_problem_cv_grid_multi: alpha and lam are (T, n_grid), one grid per response; returns three
+        (T, n_grid, n_folds) tables.  Entries of other shards stay 0."""
+        alpha = np.ascontiguousarray(alpha, dtype=np.float64)
+        lam = np.ascontiguousarray(lam, dtype=np.float64)
+        T = self.n_targets
+        if alpha.shape != lam.shape or alpha.ndim != 2 or alpha.shape[0] != T or alpha.shape[1] < 1 or self.n_folds < 1:
+            raise ValueError(f"alpha and lambda must both be ({T}, n_grid) arrays and the problem must have folds")
+        n_grid, nf = alpha.shape[1], self.n_folds
+        total = T * n_grid * nf
+        err = np.zeros(total); st = np.zeros(total, np.int32); ns = np.zeros(total, np.int32)
+        _check(load().pareben_problem_cv_grid_multi(self._h, _d(alpha), _d(lam), n_grid, int(shard), int(n_shards), _d(err), _i(st), _i(ns)))
+        return err.reshape(T, n_grid, nf), st.reshape(T, n_grid, nf), ns.reshape(T, n_grid, nf)
 
     def fit(self, alpha: float, lam: float):
         """Batch-of-1 final model: returns (beta_table, wald, intercept, extra, status)."""
@@ -184,6 +236,12 @@ class Problem:
         out = np.zeros(1)
         _check(load().pareben_lambda_max(self._h, _d(out)))
         return float(out[0])
+
+    def lambda_max_multi(self) -> np.ndarray:
+        """pareben_lambda_max_multi: lambda_max of every response (length T), one pass over the candidates."""
+        out = np.zeros(self.n_targets)
+        _check(load().pareben_lambda_max_multi(self._h, _d(out)))
+        return out
 
     def sl_filter(self, tau_main: float, tau_pair: float):
         """pareben_sl_filter: (candidate ids ascending, statistics) of the single-locus prefilter."""
@@ -255,6 +313,36 @@ def cv_grid(BASIS, Target, fold_id, n_folds, alpha, lam, epis=False, prior="gaus
                                   GAUSSIAN if prior == "gaussian" else BINOMIAL, int(n_devices), device, shard, n_shards,
                                   _d(err), _i(st), _i(ns)))
     return err.reshape(alpha.size, n_folds), st.reshape(alpha.size, n_folds), ns.reshape(alpha.size, n_folds)
+
+
+def cv_grid_multi(BASIS, Targets, fold_id, n_folds, alpha, lam, epis=False, prior="gaussian", device=None,
+                  shard=0, n_shards=1, n_devices=1):
+    """pareben_cv_grid_multi: T responses (Targets n x T) against one design in one call.  alpha and lam are (T, n_grid),
+    each response's own grid; returns three (T, n_grid, n_folds) tables.  Entries owned by other shards are left 0."""
+    X = np.asfortranarray(np.asarray(BASIS, dtype=np.float64))
+    if X.ndim != 2:
+        raise ValueError("BASIS must be a matrix")
+    n, k = X.shape
+    Y = _targets_matrix(Targets, n)
+    T = Y.shape[1]
+    fid = np.ascontiguousarray(np.asarray(fold_id, dtype=np.int32).ravel())
+    alpha = np.ascontiguousarray(alpha, dtype=np.float64)
+    lam = np.ascontiguousarray(lam, dtype=np.float64)
+    n_folds = int(n_folds)
+    if fid.size != n:
+        raise ValueError("fold_id length must equal nrow(BASIS)")
+    if alpha.shape != lam.shape or alpha.ndim != 2 or alpha.shape[0] != T or alpha.shape[1] < 1:
+        raise ValueError(f"alpha and lambda must both be ({T}, n_grid) arrays")
+    if n_folds < 1:
+        raise ValueError("n_folds must be >= 1")
+    device = default_device() if device is None else int(device)
+    n_grid = alpha.shape[1]
+    total = T * n_grid * n_folds
+    err = np.zeros(total); st = np.zeros(total, np.int32); ns = np.zeros(total, np.int32)
+    _check(load().pareben_cv_grid_multi(_d(X), n, k, _d(Y), T, _i(fid), n_folds, _d(alpha), _d(lam), n_grid, int(bool(epis)),
+                                        GAUSSIAN if prior == "gaussian" else BINOMIAL, int(n_devices), device, shard, n_shards,
+                                        _d(err), _i(st), _i(ns)))
+    return err.reshape(T, n_grid, n_folds), st.reshape(T, n_grid, n_folds), ns.reshape(T, n_grid, n_folds)
 
 
 def shard_plan(lam, n_folds: int, shard: int, n_shards: int) -> np.ndarray:

@@ -6,6 +6,8 @@ image, so this Python layer stands where R/CrossValidate.R etc. would call `.Cal
   BuildGrid       /root/reference/R/BuildGrid.R:34-52     GetLambdaMax  :5-32
   AssignToFolds   /root/reference/R/AssignToFolds.R:6-19
   LocalSearch     /root/reference/R/LocalSearch.R:6-130
+  CrossValidateMulti  (no reference counterpart: the reference loops CrossValidate) T responses against one design in
+                  one upload and one batched fit call, each result equal to CrossValidate on that response
   EBelasticNet_Gaussian / EBelasticNet_Binomial  (final model after CV, README.md:89-94;
                   /root/reference/EBEN_orig/R/EBelasticNet.Gaussian.R, .Binomial.R)
 The foreach/%dopar% fan-out (CrossValidate.R:66-70, 88-92; LocalSearch.R:67-104) is replaced
@@ -155,6 +157,11 @@ def CrossValidate(BASIS, Target, nFolds, foldId=0, Epis="no", prior="gaussian", 
     # TestModel ignores the caller's foldId and recomputes folds with set.seed(1) (TestModel.R:9)
     folds = AssignToFolds(X, nFolds, sample_kind=sample_kind)
     grid, err, status, nsel = _grid_and_errors(X, y, folds, nFolds, Epis, prior_key, device, n_devices)
+    return _global_result(grid, err, status, nsel, folds, nFolds, prior_key)
+
+
+def _global_result(grid, err, status, nsel, folds, nFolds, prior_key):
+    """CrossValidate's return value (CrossValidate.R:72-117) from the grid and its n_grid x n_folds tables."""
     n_grid = grid["alpha"].size
     value = "MSE" if prior_key == "gaussian" else "logL"
     detail = {"foldId": np.tile(np.arange(1, nFolds + 1), n_grid), "alpha": np.repeat(grid["alpha"], nFolds),
@@ -179,6 +186,11 @@ def LocalSearch(BASIS, Target, nFolds, Epis="no", foldId=0, prior="gaussian", de
     prior_key = "gaussian" if prior == "gaussian" else "binomial"
     folds = AssignToFolds(X, nFolds, foldId, sample_kind, rng)
     grid, err, status, nsel = _grid_and_errors(X, y, folds, nFolds, Epis, prior_key, device, n_devices)
+    return _local_result(grid, err, status, folds, nFolds, prior_key)
+
+
+def _local_result(grid, err, status, folds, nFolds, prior_key):
+    """LocalSearch's early-stopping walk (LocalSearch.R:56-122) replayed over a complete n_grid x n_folds table."""
     if prior_key == "binomial":
         err = -err                       # walk on Likelihood = -logL (documented deviation)
     Alpha, Lambda = grid["alpha"][:20], grid["lambda"][::20]
@@ -204,6 +216,61 @@ def LocalSearch(BASIS, Target, nFolds, Epis="no", foldId=0, prior="gaussian", de
     idx = _which_min(each[:, 2], status, "per-alpha minimum")
     return {"CrossValidation": each, "alpha.optimal": float(each[idx, 0]), "lambda.optimal": float(each[idx, 1]),
             "fullCV": full, "status": status, "foldId": folds}
+
+
+def _targets(X, Targets):
+    Y = np.asarray(Targets, dtype=np.float64)
+    if Y.ndim != 2 or Y.shape[0] != X.shape[0] or Y.shape[1] < 1:
+        raise ValueError(f"Targets must be an n x T matrix (T >= 1) with n = nrow(BASIS) = {X.shape[0]}; got shape {Y.shape}")
+    bad = np.nonzero(~np.isfinite(Y).all(axis=0))[0]
+    if bad.size:
+        raise ValueError(f"Targets column {int(bad[0])} holds non-finite values (NA/NaN/Inf): per-response missing rows are not "
+                         "supported; drop the rows for every response, or run CrossValidate on that response alone")
+    return Y
+
+
+def _grids_and_errors_multi(X, Y, fold_id, n_folds, Epis, prior, device, n_devices=1):
+    """_grid_and_errors for the T columns of Y: each response's BuildGrid grid from its own lambda_max (one pass over the
+    candidates for all of them) and all T x n_grid x n_folds hold-out errors from one fit call.  Sharding and merging as in
+    _grid_and_errors."""
+    dist = _dist()
+    rank, world = (dist.get_rank(), dist.get_world_size()) if dist is not None else (0, 1)
+    epis = Epis == "yes"
+
+    def grids_of(p):
+        grids = [_grid_from_lambda_max(float(v)) for v in p.lambda_max_multi()]
+        return grids, np.stack([g["alpha"] for g in grids]), np.stack([g["lambda"] for g in grids])
+
+    if n_devices != 1:
+        with _lib.Problem(X, Y, None, 0, epis, "gaussian", device) as p:
+            grids, A, L = grids_of(p)
+        err, st, ns = _lib.cv_grid_multi(X, Y, fold_id, n_folds, A, L, epis, prior, device, rank, world, n_devices)
+    else:
+        with _lib.Problem(X, Y, fold_id, n_folds, epis, prior, device) as p:
+            grids, A, L = grids_of(p)
+            err, st, ns = p.cv_grid_multi(A, L, rank, world)
+    err, st, ns = _merge_shards(err, st, ns, device)
+    return grids, err, st, ns
+
+
+def CrossValidateMulti(BASIS, Targets, nFolds, foldId=0, Epis="no", prior="gaussian", search="global",
+                       device: int | None = None, sample_kind: str = "Rejection", n_devices: int = 1):
+    """CrossValidate for each column of Targets (n x T) against the same BASIS, in one problem upload and one fit call.
+    Returns a list of T dicts; entry t equals CrossValidate(BASIS, Targets[:, t], nFolds, foldId, Epis, prior, search, ...)
+    entry for entry: the folds are the same for every response (AssignToFolds does not look at the response), each
+    response gets its own grid from its own lambda_max, and every fit is bitwise the single-response fit.  search="local"
+    replays LocalSearch's walk per response over the shared table.  Every response must be observed on every row."""
+    X = _as_matrix(BASIS)
+    Y = _targets(X, Targets)
+    prior_key = "gaussian" if prior == "gaussian" else "binomial"
+    if search != "global":
+        folds = AssignToFolds(X, nFolds, foldId, sample_kind)
+    else:
+        folds = AssignToFolds(X, nFolds, sample_kind=sample_kind)
+    grids, err, status, nsel = _grids_and_errors_multi(X, Y, folds, nFolds, Epis, prior_key, device, n_devices)
+    if search != "global":
+        return [_local_result(grids[t], err[t], status[t], folds, nFolds, prior_key) for t in range(Y.shape[1])]
+    return [_global_result(grids[t], err[t], status[t], nsel[t], folds, nFolds, prior_key) for t in range(Y.shape[1])]
 
 
 def _weight_table(table, keep, epis, n):

@@ -58,10 +58,14 @@ struct Problem {
     int cap;                 // basis cap actually used (<= the reference's basisMax)
     int nmax;                // max ntr over folds
     int tc;                  // 1 when the folds carry the int8 operand images (FoldData::Xtc): the slabs then hold digit planes
-    const FoldData *folds;   // [n_folds + 1]; index 0 = all rows, f = rows with fold_id != f
+    // [n_targets][n_folds + 1]; fold index 0 = all rows, f = rows with fold_id != f.  The records of one fold differ
+    // only in ytr / yte (one response each) and share every design-side buffer, so whatever depends on the design alone
+    // (the Gram build, the streaming scan) indexes folds[f], the records of response 0.
+    const FoldData *folds;
 };
 
-struct FitTask { int fold; double alpha, lambda; int out_index; int group; };
+// target: the response the fit trains on; its data are P.folds[target * (n_folds + 1) + fold] (see Problem::folds)
+struct FitTask { int fold, target; double alpha, lambda; int out_index; int group; };
 
 // Device-side scheduler state of one launch (see next_task() in fit_kernel.cuh).  Fits that differ only in the
 // fold (same alpha, lambda: one row of the reference's ParameterGrid, R/CrossValidate.R:66) form a group and

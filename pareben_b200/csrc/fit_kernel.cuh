@@ -123,7 +123,7 @@ eben_fit_kernel(Problem P, Variant v, const FitTask *__restrict__ tasks, int n_t
         if (ti < 0) break;
         const FitTask task = tasks[ti];
         const unsigned long long t_fit0 = sched_now();
-        const FoldData F = P.folds[task.fold];
+        const FoldData F = P.folds[task.target * (P.n_folds + 1) + task.fold];
         Slab s = carve_slab(slabs + (size_t)blockIdx.x * slab_stride, P.cap, P.nmax, P.Kc, P.tc);
 #ifdef PAREBEN_PHASE_TIMING
         if (threadIdx.x == 0 && task.out_index < FIT_TRACE_MAX) { g_fit_t0[task.out_index] = global_ns(); g_fit_block[task.out_index] = blockIdx.x; }

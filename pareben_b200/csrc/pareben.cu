@@ -11,6 +11,7 @@
 
 #include <algorithm>
 #include <map>
+#include <tuple>
 #include <thread>
 #include <chrono>
 #include <mutex>
@@ -147,11 +148,12 @@ __global__ void gather_rows_kernel(const double *__restrict__ Xcol, int N, int K
     }
 }
 
-__global__ void gather_vec_kernel(const double *__restrict__ y, const int *__restrict__ rows, int nrows,
-                                  double *__restrict__ out)
+// out[t * ld_out + r] = y[t * n + rows[r]] for response t = blockIdx.y (columns of an n x n_targets matrix)
+__global__ void gather_vec_kernel(const double *__restrict__ y, int n, const int *__restrict__ rows, int nrows,
+                                  double *__restrict__ out, size_t ld_out)
 {
     const int r = blockIdx.x * blockDim.x + threadIdx.x;
-    if (r < nrows) out[r] = y[rows[r]];
+    if (r < nrows) out[blockIdx.y * ld_out + r] = y[(size_t)blockIdx.y * n + rows[r]];
 }
 
 __global__ void to_int8_kernel(const double *__restrict__ in, size_t n, int8_t *__restrict__ out)
@@ -207,27 +209,60 @@ __global__ void scales_kernel(const double *__restrict__ X, int N, int K, int Kc
     scale[c] = sqrt(z);
 }
 
-// lambda_max pieces (R/BuildGrid.R:5-32): max over candidates of x_c' r / ||x_c||
-template <bool EPIS>
-__global__ void lambda_max_kernel(const double *__restrict__ X, int N, int K, int c_begin, int c_end,
-                                  const double *__restrict__ resp, double *__restrict__ block_max)
+// lambda_max pieces (R/BuildGrid.R:5-32) for T responses in one pass over the candidates: lmax[t] = max(lmax[t], max over
+// candidates c of x_c' r_t / ||x_c||), r_t = resp + t * N.  A thread owns a candidate and holds TT accumulators, one per
+// response of the current tile; the tile's responses are staged in shared memory LM_ROWS rows at a time and read as
+// broadcasts, so each value x of the candidate column feeds TT FMAs.  For every (candidate, response) the FMA chain is
+// z = fma(x_h, r_h, z) over h = 0..N-1 from z = 0, and ||x_c||^2 = fma(x_h, x_h, nn) once per candidate: a response's
+// value does not depend on T or on which tile it falls in.  Only positive maxima matter to the caller (it starts from
+// log(1.1)), and a positive double's bit pattern orders like its value, so the block maxima meet in lmax with atomicMax.
+constexpr int LM_THREADS = 256, LM_ROWS = 64;
+template <bool EPIS, int TT>
+__global__ void __launch_bounds__(LM_THREADS) lambda_max_multi_kernel(const double *__restrict__ X, int N, int K, int c_begin,
+                                                                      int c_end, const double *__restrict__ resp, int T,
+                                                                      double *__restrict__ lmax)
 {
-    __shared__ double red[32];
-    const int c = c_begin + blockIdx.x * blockDim.x + threadIdx.x;
-    double v = -1e300;
-    if (c < c_end) {
-        Cand<EPIS> cd(c, K);
-        double z = 0, nn = 0;
-        for (int h = 0; h < N; h++) { const double x = cd.at(X + (size_t)h * K); z = fma(x, resp[h], z); nn = fma(x, x, nn); }
-        if (nn > 0) v = z / sqrt(nn);
-    }
-    for (int o = 16; o > 0; o >>= 1) v = fmax(v, __shfl_xor_sync(0xffffffffu, v, o));
-    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = v;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        double m = red[0];
-        for (int w = 1; w < (int)(blockDim.x >> 5); w++) m = fmax(m, red[w]);
-        block_max[blockIdx.x] = m;
+    __shared__ __align__(16) double s_r[LM_ROWS][TT];
+    __shared__ double red[LM_THREADS / 32][TT];
+    const int c = c_begin + blockIdx.x * LM_THREADS + threadIdx.x;
+    const bool live = c < c_end;
+    const Cand<EPIS> cd(live ? c : c_begin, K);
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    double nn = 0;
+    for (int t0 = 0; t0 < T; t0 += TT) {
+        double z[TT];
+#pragma unroll
+        for (int j = 0; j < TT; j++) z[j] = 0;
+        for (int h0 = 0; h0 < N; h0 += LM_ROWS) {
+            const int nh = min(LM_ROWS, N - h0);
+            __syncthreads();
+            for (int i = threadIdx.x; i < LM_ROWS * TT; i += LM_THREADS) {
+                const int hh = i / TT, j = i % TT;
+                s_r[hh][j] = (t0 + j < T && hh < nh) ? resp[(size_t)(t0 + j) * N + h0 + hh] : 0.0;
+            }
+            __syncthreads();
+            if (live) {
+                for (int hh = 0; hh < nh; hh++) {
+                    const double x = cd.at(X + (size_t)(h0 + hh) * K);
+#pragma unroll
+                    for (int j = 0; j < TT; j++) z[j] = fma(x, s_r[hh][j], z[j]);
+                    if (t0 == 0) nn = fma(x, x, nn);
+                }
+            }
+        }
+        const double rn = live && nn > 0 ? sqrt(nn) : 0.0;
+#pragma unroll
+        for (int j = 0; j < TT; j++) {
+            double v = rn > 0 ? z[j] / rn : -1e300;
+            for (int o = 16; o > 0; o >>= 1) v = fmax(v, __shfl_xor_sync(0xffffffffu, v, o));
+            if (lane == 0) red[wid][j] = v;
+        }
+        __syncthreads();
+        if (threadIdx.x < TT && t0 + (int)threadIdx.x < T) {
+            double m = red[0][threadIdx.x];
+            for (int w = 1; w < LM_THREADS / 32; w++) m = fmax(m, red[w][threadIdx.x]);
+            if (m > 0) atomicMax(reinterpret_cast<unsigned long long *>(lmax + t0 + threadIdx.x), (unsigned long long)__double_as_longlong(m));
+        }
     }
 }
 
@@ -296,11 +331,14 @@ struct pareben_problem {
     int device = 0;
     int tc = 0;                          // the folds carry the int8 operand images of the tensor-core contraction (FoldData::Xtc)
     int n = 0, k = 0, kc = 0, n_folds = 0, epis = 0, prior = 0, cap = 0, nmax = 0, min_ntr = 0;
+    int n_targets = 1;                   // responses sharing the design (pareben_problem_create_multi)
     int sm_count = 0;
     std::vector<PoolEntry> allocs;       // every device buffer of this problem (returned to the pool on destroy)
     FoldData *d_folds = nullptr;
+    // [n_targets][n_folds + 1] (Problem::folds): h_folds[f] are response 0's records, whose design-side pointers every
+    // response shares; whatever changes a design-side field changes it in all n_targets records of the fold
     std::vector<FoldData> h_folds;
-    double *d_Xcol = nullptr, *d_y = nullptr;     // full data, column-major (kept for lambda_max)
+    double *d_Xcol = nullptr, *d_y = nullptr;     // full data, column-major: X n x k, y n x n_targets (kept for lambda_max)
     char *d_slabs = nullptr; size_t slab_stride = 0, slab_total = 0; int n_slabs = 0;
     double *d_flops = nullptr;
     cudaStream_t stream = nullptr;
@@ -451,7 +489,11 @@ static void ensure_gram(pareben_problem *p, int n_fits, const int *fold)
         if (all_folds > free_b / 2) { p->gram_state = -1; return; }
         p->gram_state = 1;
     }
-    for (int f : need) p->h_folds[f].C = p->dalloc<double>(bytes_per_fold / sizeof(double));
+    const int nf1 = p->n_folds + 1;
+    for (int f : need) {
+        double *C = p->dalloc<double>(bytes_per_fold / sizeof(double));
+        for (int t = 0; t < p->n_targets; t++) p->h_folds[(size_t)t * nf1 + f].C = C;
+    }
     int *d_list = p->dalloc<int>(need.size() + 1);           // fold list + the work counter (small, kept with the problem)
     std::vector<int> h_list(need);
     h_list.push_back(0);
@@ -481,10 +523,11 @@ extern "C" int pareben_device_count(void)
 extern "C" const char *pareben_last_error(void) { return g_err.c_str(); }
 extern "C" int pareben_version(void) { return PAREBEN_VERSION; }
 
-extern "C" int pareben_problem_create(pareben_problem **out, int device, const double *basis, int n, int k,
-                                      const double *target, const int *fold_id, int n_folds, int epis, int prior)
+extern "C" int pareben_problem_create_multi(pareben_problem **out, int device, const double *basis, int n, int k,
+                                            const double *targets, int n_targets, const int *fold_id, int n_folds, int epis,
+                                            int prior)
 {
-    if (!out || !basis || !target || n < 2 || k < 1 || n_folds < 0 || (n_folds > 0 && !fold_id))
+    if (!out || !basis || !targets || n < 2 || k < 1 || n_targets < 1 || n_folds < 0 || (n_folds > 0 && !fold_id))
         return fail(PAREBEN_EINVAL, "pareben_problem_create: bad argument");
     if (prior != PAREBEN_GAUSSIAN && prior != PAREBEN_BINOMIAL) return fail(PAREBEN_EINVAL, "prior must be 0 or 1");
     if (epis && (long long)k * (k + 1) / 2 > 0x7fffffffLL) return fail(PAREBEN_EINVAL, "k(k+1)/2 exceeds int32");
@@ -506,7 +549,7 @@ extern "C" int pareben_problem_create(pareben_problem **out, int device, const d
             fprintf(stderr, "[pareben]   create: %-28s %.2f ms\n", what, std::chrono::duration<double, std::milli>(t - tc0).count());
             tc0 = t;
         };
-        p->n = n; p->k = k; p->epis = epis; p->prior = prior; p->n_folds = n_folds;
+        p->n = n; p->k = k; p->epis = epis; p->prior = prior; p->n_folds = n_folds; p->n_targets = n_targets;
         p->kc = epis ? (int)((long long)k * (k + 1) / 2) : k;
         p->streaming = want_streaming(p->kc, prior);
         if (p->streaming && n_folds + 1 > STREAM_MAX_FOLDS) throw std::make_pair((int)PAREBEN_EINVAL, std::string("streaming mode supports at most 255 folds"));
@@ -514,9 +557,9 @@ extern "C" int pareben_problem_create(pareben_problem **out, int device, const d
         CU(cudaEventCreate(&p->ev0)); CU(cudaEventCreate(&p->ev1));
 
         p->d_Xcol = p->dalloc<double>((size_t)n * k);
-        p->d_y = p->dalloc<double>(n);
+        p->d_y = p->dalloc<double>((size_t)n * n_targets);
         CU(cudaMemcpyAsync(p->d_Xcol, basis, sizeof(double) * n * k, cudaMemcpyHostToDevice, p->stream));
-        CU(cudaMemcpyAsync(p->d_y, target, sizeof(double) * n, cudaMemcpyHostToDevice, p->stream));
+        CU(cudaMemcpyAsync(p->d_y, targets, sizeof(double) * n * n_targets, cudaMemcpyHostToDevice, p->stream));
 
         // Genotype-coded designs (every entry an integer in [-127, 127], e.g. {-1, 0, 1}) also get an
         // int8 copy of the training matrices: the score contraction reads 1 byte instead of 8 per
@@ -536,7 +579,8 @@ extern "C" int pareben_problem_create(pareben_problem **out, int device, const d
         lap("stream/events/h2d enqueue/scan");
         // row lists per fold: index 0 = all rows (only materialised when n_folds == 0)
         const int nf = n_folds;
-        p->h_folds.assign(nf + 1, FoldData{});
+        p->h_folds.assign((size_t)n_targets * (nf + 1), FoldData{});
+        std::vector<size_t> ld_y(2 * (nf + 1), 0);      // per fold: stride of the responses' training / test vectors
         int min_ntr = n;
         for (int f = (nf == 0 ? 0 : 1); f <= nf; f++) {
             std::vector<int> tr, te;
@@ -557,16 +601,23 @@ extern "C" int pareben_problem_create(pareben_problem **out, int device, const d
             if (!te.empty())
                 CU(cudaMemcpyAsync(d_rows + tr.size(), te.data(), sizeof(int) * te.size(), cudaMemcpyHostToDevice, p->stream));
             CU(cudaStreamSynchronize(p->stream));      // tr/te go out of scope
-            double *Xtr = p->dalloc<double>((size_t)F.ntr * k), *ytr = p->dalloc<double>(F.ntr);
-            double *Xte = p->dalloc<double>((size_t)F.nte * k), *yte = p->dalloc<double>(F.nte);
+            // responses of the fold: one vector per response, each starting on a 256-byte boundary like its own allocation would
+            ld_y[2 * f] = ((size_t)F.ntr + 31) & ~(size_t)31; ld_y[2 * f + 1] = ((size_t)F.nte + 31) & ~(size_t)31;
+            double *Xtr = p->dalloc<double>((size_t)F.ntr * k), *ytr = p->dalloc<double>(ld_y[2 * f] * n_targets);
+            double *Xte = p->dalloc<double>((size_t)F.nte * k), *yte = p->dalloc<double>(ld_y[2 * f + 1] * n_targets);
             double *scale = p->streaming ? nullptr : p->dalloc<double>(p->kc);     // streaming: norms are computed on the fly
             dim3 blk(32, 8);
             gather_rows_kernel<<<dim3((F.ntr + 31) / 32, (k + 31) / 32), blk, 0, p->stream>>>(p->d_Xcol, n, k, d_rows, F.ntr, Xtr);
-            gather_vec_kernel<<<(F.ntr + 255) / 256, 256, 0, p->stream>>>(p->d_y, d_rows, F.ntr, ytr);
-            if (F.nte > 0) {
-                gather_rows_kernel<<<dim3((F.nte + 31) / 32, (k + 31) / 32), blk, 0, p->stream>>>(p->d_Xcol, n, k, d_rows + F.ntr, F.nte, Xte);
-                gather_vec_kernel<<<(F.nte + 255) / 256, 256, 0, p->stream>>>(p->d_y, d_rows + F.ntr, F.nte, yte);
+            for (int t0 = 0; t0 < n_targets; t0 += 65535) {          // grid.y: one response each
+                const unsigned nt = (unsigned)std::min(65535, n_targets - t0);
+                gather_vec_kernel<<<dim3((F.ntr + 255) / 256, nt), 256, 0, p->stream>>>(p->d_y + (size_t)t0 * n, n, d_rows, F.ntr,
+                                                                                         ytr + t0 * ld_y[2 * f], ld_y[2 * f]);
+                if (F.nte > 0)
+                    gather_vec_kernel<<<dim3((F.nte + 255) / 256, nt), 256, 0, p->stream>>>(p->d_y + (size_t)t0 * n, n, d_rows + F.ntr, F.nte,
+                                                                                             yte + t0 * ld_y[2 * f + 1], ld_y[2 * f + 1]);
             }
+            if (F.nte > 0)
+                gather_rows_kernel<<<dim3((F.nte + 31) / 32, (k + 31) / 32), blk, 0, p->stream>>>(p->d_Xcol, n, k, d_rows + F.ntr, F.nte, Xte);
             if (scale) {
                 if (epis) scales_kernel<true><<<(p->kc + 255) / 256, 256, 0, p->stream>>>(Xtr, F.ntr, k, p->kc, scale);
                 else scales_kernel<false><<<(p->kc + 255) / 256, 256, 0, p->stream>>>(Xtr, F.ntr, k, p->kc, scale);
@@ -600,9 +651,16 @@ extern "C" int pareben_problem_create(pareben_problem **out, int device, const d
             }
         }
         CU(cudaGetLastError());
+        // the other responses' records: response 0's design side, their own ytr / yte
+        for (int t = 1; t < n_targets; t++)
+            for (int f = 0; f <= nf; f++) {
+                FoldData &R = p->h_folds[(size_t)t * (nf + 1) + f];
+                R = p->h_folds[f];
+                if (R.ytr) { R.ytr += t * ld_y[2 * f]; R.yte += t * ld_y[2 * f + 1]; }
+            }
         lap("per-fold layout (enqueue)");
-        p->d_folds = p->dalloc<FoldData>(nf + 1);
-        CU(cudaMemcpyAsync(p->d_folds, p->h_folds.data(), sizeof(FoldData) * (nf + 1), cudaMemcpyHostToDevice, p->stream));
+        p->d_folds = p->dalloc<FoldData>(p->h_folds.size());
+        CU(cudaMemcpyAsync(p->d_folds, p->h_folds.data(), sizeof(FoldData) * p->h_folds.size(), cudaMemcpyHostToDevice, p->stream));
 
         p->min_ntr = min_ntr;
         p->d_flops = p->dalloc<double>(3);
@@ -614,6 +672,12 @@ extern "C" int pareben_problem_create(pareben_problem **out, int device, const d
     }
     *out = p;
     return PAREBEN_OK;
+}
+
+extern "C" int pareben_problem_create(pareben_problem **out, int device, const double *basis, int n, int k,
+                                      const double *target, const int *fold_id, int n_folds, int epis, int prior)
+{
+    return pareben_problem_create_multi(out, device, basis, n, k, target, 1, fold_id, n_folds, epis, prior);
 }
 
 extern "C" void pareben_problem_destroy(pareben_problem *p) { delete p; }
@@ -637,8 +701,31 @@ struct DumpBuffers { int *m = nullptr, *used = nullptr; double *beta = nullptr, 
 // Streaming mode (stream.cuh): every fit keeps only its active set; all fits advance in lock-step rounds of
 //   stream_advance_kernel (one block per fit)  ->  stream_scan_kernel (one dense contraction per fold for all waiting fits)
 // until no fit is waiting for a scan.  One 4-byte-per-fold read-back per round tells the host when to stop.
-int run_fits_streaming(pareben_problem *p, int n_fits, const int *fold, const double *alpha, const double *lambda,
-                       double *fold_err, int *status, int *n_selected, int *n_iter, DumpBuffers *dump)
+constexpr int STREAM_LIST_CAP = 4096;
+
+// device bytes of one streaming fit's state at basis cap c (the layout run_fits_streaming carves)
+size_t stream_fit_bytes(const pareben_problem *p, int c)
+{
+    const size_t LD = phi_ld(p->nmax), lc = STREAM_LIST_CAP;
+    const size_t dbl = (size_t)4 * c * c + LD * c + (size_t)12 * (c + 1) + (size_t)4 * p->nmax + 2 * lc + 16;
+    const size_t ints = (size_t)2 * c + (size_t)4 * (c + lc) + lc + 16;
+    return ((dbl * 8 + ints * 4) + 255) & ~(size_t)255;
+}
+
+// basis cap of a streaming call whose largest response has fits_per_target fits: the reference's basisMax, bounded by
+// PAREBEN_BASIS_CAP and by what that many active sets may occupy.  It depends on the fits of one response, never on the
+// number of responses, so each response's fits end as they would in a single-response call.
+int stream_cap(const pareben_problem *p, long long fits_per_target, size_t free_b)
+{
+    int cap = reference_basis_max(p->min_ntr, p->k, p->kc, p->epis, p->prior);
+    const char *env_cap = getenv("PAREBEN_BASIS_CAP");
+    cap = std::max(2, std::min(cap, env_cap ? atoi(env_cap) : 1024));
+    while (cap > 16 && stream_fit_bytes(p, cap) * (size_t)fits_per_target > free_b / 2) cap = cap * 3 / 4;
+    return cap;
+}
+
+int run_fits_streaming(pareben_problem *p, int n_fits, const int *target, const int *fold, const double *alpha, const double *lambda,
+                       double *fold_err, int *status, int *n_selected, int *n_iter, DumpBuffers *dump, int cap)
 {
     std::vector<std::pair<void *, size_t>> scratch;
     cudaEvent_t es0 = nullptr, es1 = nullptr;
@@ -650,23 +737,10 @@ int run_fits_streaming(pareben_problem *p, int n_fits, const int *fold, const do
             void *q = pool_take(p->device, bytes, false, nullptr);
             if (!q) CU(malloc_retry(p->device, &q, bytes));
             scratch.emplace_back(q, bytes); return q; };
-        // basis cap: the reference's basisMax, bounded by PAREBEN_BASIS_CAP and by what n_fits active sets may occupy
-        int cap = reference_basis_max(p->min_ntr, p->k, p->kc, p->epis, p->prior);
-        const char *env_cap = getenv("PAREBEN_BASIS_CAP");
-        cap = std::max(2, std::min(cap, env_cap ? atoi(env_cap) : 1024));
-        const int list_cap = 4096;
+        const int list_cap = STREAM_LIST_CAP;
         const int LD = phi_ld(p->nmax);
-        auto fit_doubles = [&](int c) { return (size_t)4 * c * c + (size_t)LD * c + (size_t)12 * (c + 1) + (size_t)4 * p->nmax + (size_t)2 * list_cap + 16; };
-        auto fit_ints = [&](int c) { return (size_t)2 * c + (size_t)4 * (c + list_cap) + list_cap + 16; };
-        auto fit_bytes = [&](int c) { return ((fit_doubles(c) * 8 + fit_ints(c) * 4) + 255) & ~(size_t)255; };
-        {
-            size_t free_b = 0, total_b = 0;
-            CU(cudaMemGetInfo(&free_b, &total_b));
-            free_b += pool_parked(p->device);
-            while (cap > 16 && fit_bytes(cap) * (size_t)n_fits > free_b / 2) cap = cap * 3 / 4;
-        }
         p->cap = cap;
-        const size_t stride = fit_bytes(cap);
+        const size_t stride = stream_fit_bytes(p, cap);
         char *d_state = (char *)tmp_alloc(stride * (size_t)n_fits);
         StreamFit *d_fits = (StreamFit *)tmp_alloc(sizeof(StreamFit) * (size_t)n_fits);
         std::vector<StreamFit> h_fits(n_fits);
@@ -677,7 +751,7 @@ int run_fits_streaming(pareben_problem *p, int n_fits, const int *fold, const do
             per_fold[fold[i]]++;
             StreamFit f;
             memset(&f, 0, sizeof f);
-            f.fold = fold[i]; f.out_index = i; f.lambda = lambda[i]; f.alpha_en = alpha[i]; f.phase = SP_START;
+            f.fold = fold[i]; f.target = target[i]; f.out_index = i; f.lambda = lambda[i]; f.alpha_en = alpha[i]; f.phase = SP_START;
             double *d = reinterpret_cast<double *>(d_state + stride * (size_t)i);
             const size_t cc = (size_t)cap * cap;
             f.sigma = d; d += cc; f.sigma_new = d; d += cc; f.H = d; d += cc; f.ptp = d; d += cc;
@@ -802,12 +876,64 @@ int run_fits_streaming(pareben_problem *p, int n_fits, const int *fold, const do
     return PAREBEN_OK;
 }
 
-int run_fits_impl(pareben_problem *p, int n_fits, const int *fold, const double *alpha, const double *lambda,
+// Streaming call: the basis cap comes from the largest share of the fits that one response has (stream_cap).  When the
+// states of all fits do not fit in device memory at that cap, the responses run in waves of whole responses.
+int run_fits_streaming_waves(pareben_problem *p, int n_fits, const int *target, const int *fold, const double *alpha,
+                             const double *lambda, double *fold_err, int *status, int *n_selected, int *n_iter, DumpBuffers *dump)
+{
+    std::vector<long long> per_t(p->n_targets, 0);
+    for (int i = 0; i < n_fits; i++) per_t[target[i]]++;
+    size_t free_b = 0, total_b = 0;
+    cudaError_t e = cudaSetDevice(p->device);
+    if (e == cudaSuccess) e = cudaMemGetInfo(&free_b, &total_b);
+    if (e != cudaSuccess) return fail(PAREBEN_ECUDA, std::string("cudaMemGetInfo failed: ") + cudaGetErrorString(e));
+    free_b += pool_parked(p->device);
+    const int cap = stream_cap(p, *std::max_element(per_t.begin(), per_t.end()), free_b);
+    const long long budget = std::max<long long>(1, (long long)(free_b / 2 / stream_fit_bytes(p, cap)));
+    if (n_fits <= budget)
+        return run_fits_streaming(p, n_fits, target, fold, alpha, lambda, fold_err, status, n_selected, n_iter, dump, cap);
+    double ms = 0, flops = 0, scan_ms = 0, scan_flops = 0;
+    int launches = 0, scans = 0, rounds = 0;
+    for (int t0 = 0; t0 < p->n_targets;) {
+        long long cnt = per_t[t0];
+        int t1 = t0 + 1;
+        while (t1 < p->n_targets && cnt + per_t[t1] <= budget) cnt += per_t[t1++];
+        std::vector<int> idx;
+        for (int i = 0; i < n_fits; i++) if (target[i] >= t0 && target[i] < t1) idx.push_back(i);
+        t0 = t1;
+        if (idx.empty()) continue;
+        const int m = (int)idx.size();
+        std::vector<int> tg(m), fd(m), st(m), ns(m), it(m);
+        std::vector<double> a(m), l(m), err(m);
+        for (int j = 0; j < m; j++) { tg[j] = target[idx[j]]; fd[j] = fold[idx[j]]; a[j] = alpha[idx[j]]; l[j] = lambda[idx[j]]; }
+        const int rc = run_fits_streaming(p, m, tg.data(), fd.data(), a.data(), l.data(), err.data(), st.data(), ns.data(), it.data(),
+                                          nullptr, cap);
+        if (rc != PAREBEN_OK) return rc;
+        for (int j = 0; j < m; j++) {
+            if (fold_err) fold_err[idx[j]] = err[j];
+            if (status) status[idx[j]] = st[j];
+            if (n_selected) n_selected[idx[j]] = ns[j];
+            if (n_iter) n_iter[idx[j]] = it[j];
+        }
+        ms += p->last_ms; flops += p->last_flops; launches += p->last_launches;
+        scan_ms += p->last_scan_ms; scan_flops += p->last_scan_flops; scans += p->last_scan_launches; rounds += p->last_rounds;
+    }
+    p->last_ms = ms; p->last_flops = flops; p->last_launches = launches;
+    p->last_scan_ms = scan_ms; p->last_scan_flops = scan_flops; p->last_scan_launches = scans; p->last_rounds = rounds;
+    return PAREBEN_OK;
+}
+
+// target: response of each fit (0 .. n_targets - 1); null = response 0 for every fit
+int run_fits_impl(pareben_problem *p, int n_fits, const int *target, const int *fold, const double *alpha, const double *lambda,
                   double *fold_err, int *status, int *n_selected, int *n_iter, DumpBuffers *dump)
 {
     if (!p || n_fits < 0 || (n_fits > 0 && (!fold || !alpha || !lambda))) return fail(PAREBEN_EINVAL, "pareben_run_fits: bad argument");
     if (n_fits == 0) return PAREBEN_OK;
-    if (p->streaming) return run_fits_streaming(p, n_fits, fold, alpha, lambda, fold_err, status, n_selected, n_iter, dump);
+    std::vector<int> target0;
+    if (!target) { target0.assign(n_fits, 0); target = target0.data(); }
+    for (int i = 0; i < n_fits; i++)
+        if (target[i] < 0 || target[i] >= p->n_targets) return fail(PAREBEN_EINVAL, "pareben_run_fits: target index out of range");
+    if (p->streaming) return run_fits_streaming_waves(p, n_fits, target, fold, alpha, lambda, fold_err, status, n_selected, n_iter, dump);
     void *scratch[8] = {nullptr};
     size_t scratch_bytes[8] = {0};
     int ns = 0;
@@ -819,16 +945,17 @@ int run_fits_impl(pareben_problem *p, int n_fits, const int *fold, const double 
                 return fail(PAREBEN_EINVAL, "pareben_run_fits: fold label not available in this problem");
         ensure_gram(p, n_fits, fold);
         std::vector<FitTask> tasks(n_fits);
-        // groups: fits that share (alpha, lambda) -- one row of the reference's ParameterGrid -- differ only in the fold
-        // and cost about the same; the device scheduler prices a group by its first finished fit (fit_kernel.cuh)
-        std::map<std::pair<double, double>, int> group_of;
+        // groups: fits of one response that share (alpha, lambda) -- one row of the reference's ParameterGrid -- differ
+        // only in the fold and cost about the same; the device scheduler prices a group by its first finished fit
+        // (fit_kernel.cuh).  Another response's fits at the same point can cost quite differently, so they form their own group.
+        std::map<std::tuple<int, double, double>, int> group_of;
         for (int i = 0; i < n_fits; i++) {
             if (fold[i] < 0 || fold[i] > p->n_folds || (p->n_folds > 0 && fold[i] == 0) || !p->h_folds[fold[i]].Xtr)
                 return fail(PAREBEN_EINVAL, "pareben_run_fits: fold label not available in this problem");
-            const auto key = std::make_pair(alpha[i], lambda[i]);
+            const auto key = std::make_tuple(target[i], alpha[i], lambda[i]);
             auto it = group_of.find(key);
             if (it == group_of.end()) it = group_of.emplace(key, (int)group_of.size()).first;
-            tasks[i] = FitTask{fold[i], alpha[i], lambda[i], i, it->second};
+            tasks[i] = FitTask{fold[i], target[i], alpha[i], lambda[i], i, it->second};
         }
         const int n_groups = (int)group_of.size();
         // host order: rising lambda (larger active sets first) is the prior; one pilot per group goes to the front
@@ -924,7 +1051,14 @@ int run_fits_impl(pareben_problem *p, int n_fits, const int *fold, const double 
 extern "C" int pareben_run_fits(pareben_problem *p, int n_fits, const int *fold, const double *alpha,
                                 const double *lambda, double *fold_err, int *status, int *n_selected, int *n_iter)
 {
-    return run_fits_impl(p, n_fits, fold, alpha, lambda, fold_err, status, n_selected, n_iter, nullptr);
+    return run_fits_impl(p, n_fits, nullptr, fold, alpha, lambda, fold_err, status, n_selected, n_iter, nullptr);
+}
+
+extern "C" int pareben_run_fits_multi(pareben_problem *p, int n_fits, const int *target, const int *fold, const double *alpha,
+                                      const double *lambda, double *fold_err, int *status, int *n_selected, int *n_iter)
+{
+    if (n_fits > 0 && !target) return fail(PAREBEN_EINVAL, "pareben_run_fits_multi: bad argument");
+    return run_fits_impl(p, n_fits, target, fold, alpha, lambda, fold_err, status, n_selected, n_iter, nullptr);
 }
 
 // Cost-aware interleaving (SURVEY.md 8e): order fits by falling expected cost (rising lambda,
@@ -949,30 +1083,31 @@ extern "C" int pareben_shard_plan(const double *lambda, int n_grid, int n_folds,
 
 namespace {
 
-// One sub-shard of a grid call on one device: upload, lay out, run, scatter into the caller's tables.
-int cv_grid_on_device(const double *basis, int n, int k, const double *target, const int *fold_id, int n_folds,
+// One sub-shard of a grid call on one device: upload, lay out, run, scatter into the caller's tables.  Responses, grid
+// points and folds are numbered as in pareben_cv_grid_multi.
+int cv_grid_on_device(const double *basis, int n, int k, const double *targets, int n_targets, const int *fold_id, int n_folds,
                       const double *alpha, const double *lambda, int n_grid, int epis, int prior, int device,
                       int shard, int n_shards, double *fold_err, int *status, int *n_selected)
 {
-    const int total = n_grid * n_folds;
+    const int rows = n_targets * n_grid, total = rows * n_folds;
     std::vector<int> mine(total);
     int m = 0;
-    pareben_shard_plan(lambda, n_grid, n_folds, shard, n_shards, mine.data(), &m);
+    pareben_shard_plan(lambda, rows, n_folds, shard, n_shards, mine.data(), &m);
     if (m == 0) return PAREBEN_OK;
     pareben_problem *p = nullptr;
     const bool timing = getenv("PAREBEN_TIMING") != nullptr;
     auto t0 = std::chrono::steady_clock::now();
-    int rc = pareben_problem_create(&p, device, basis, n, k, target, fold_id, n_folds, epis, prior);
+    int rc = pareben_problem_create_multi(&p, device, basis, n, k, targets, n_targets, fold_id, n_folds, epis, prior);
     if (rc != PAREBEN_OK) return rc;
     auto t1 = std::chrono::steady_clock::now();
-    std::vector<int> fold(m), st(m), ns(m);
+    std::vector<int> tg(m), fold(m), st(m), ns(m);
     std::vector<double> a(m), l(m), err(m);
     for (int i = 0; i < m; i++) {
-        const int fit = mine[i];
-        fold[i] = fit % n_folds + 1; a[i] = alpha[fit / n_folds]; l[i] = lambda[fit / n_folds];
+        const int fit = mine[i], row = fit / n_folds;
+        tg[i] = row / n_grid; fold[i] = fit % n_folds + 1; a[i] = alpha[row]; l[i] = lambda[row];
     }
     p->grid_fits_hint = total;
-    rc = pareben_run_fits(p, m, fold.data(), a.data(), l.data(), err.data(), st.data(), ns.data(), nullptr);
+    rc = run_fits_impl(p, m, tg.data(), fold.data(), a.data(), l.data(), err.data(), st.data(), ns.data(), nullptr, nullptr);
     auto t2 = std::chrono::steady_clock::now();
     const double kernel_ms = p->last_ms;
     pareben_problem_destroy(p);
@@ -997,26 +1132,27 @@ int cv_grid_on_device(const double *basis, int n, int k, const double *target, c
 // over the box's GPUs from ONE call on ONE host thread of the caller.  Each device is driven by its own worker thread
 // (upload, layout kernels, one fit launch, read-back); the workers write disjoint entries of the caller's tables, so
 // the "gather" is the join.  No R API is touched from the workers.
-extern "C" int pareben_cv_grid(const double *basis, int n, int k, const double *target, const int *fold_id,
-                               int n_folds, const double *alpha, const double *lambda, int n_grid, int epis,
-                               int prior, int n_devices, int device, int shard, int n_shards, double *fold_err,
-                               int *status, int *n_selected)
+extern "C" int pareben_cv_grid_multi(const double *basis, int n, int k, const double *targets, int n_targets, const int *fold_id,
+                                     int n_folds, const double *alpha, const double *lambda, int n_grid, int epis,
+                                     int prior, int n_devices, int device, int shard, int n_shards, double *fold_err,
+                                     int *status, int *n_selected)
 {
-    if (n_folds < 1 || n_grid < 1 || !alpha || !lambda || !fold_err) return fail(PAREBEN_EINVAL, "pareben_cv_grid: bad argument");
+    if (n_folds < 1 || n_grid < 1 || n_targets < 1 || !alpha || !lambda || !fold_err) return fail(PAREBEN_EINVAL, "pareben_cv_grid: bad argument");
+    if ((long long)n_targets * n_grid * n_folds > 0x7fffffffLL) return fail(PAREBEN_EINVAL, "pareben_cv_grid: more than 2^31 - 1 fits");
     if (n_shards < 1 || shard < 0 || shard >= n_shards) return fail(PAREBEN_EINVAL, "pareben_cv_grid: bad shard");
     const int visible = pareben_device_count();
     if (visible < 1) return fail(PAREBEN_ENODEVICE, "no usable CUDA device");
     if (n_devices == 0) n_devices = visible - device;                 // 0 = every device from `device` on
     if (device < 0 || n_devices < 1 || device + n_devices > visible) return fail(PAREBEN_ENODEVICE, "pareben_cv_grid: device range not available");
     if (n_devices == 1)
-        return cv_grid_on_device(basis, n, k, target, fold_id, n_folds, alpha, lambda, n_grid, epis, prior, device,
+        return cv_grid_on_device(basis, n, k, targets, n_targets, fold_id, n_folds, alpha, lambda, n_grid, epis, prior, device,
                                  shard, n_shards, fold_err, status, n_selected);
     std::vector<int> rcs(n_devices, PAREBEN_OK);
     std::vector<std::string> msgs(n_devices);
     std::vector<std::thread> workers;
     for (int d = 0; d < n_devices; d++)
         workers.emplace_back([&, d] {
-            rcs[d] = cv_grid_on_device(basis, n, k, target, fold_id, n_folds, alpha, lambda, n_grid, epis, prior, device + d,
+            rcs[d] = cv_grid_on_device(basis, n, k, targets, n_targets, fold_id, n_folds, alpha, lambda, n_grid, epis, prior, device + d,
                                        shard * n_devices + d, n_shards * n_devices, fold_err, status, n_selected);
             if (rcs[d] != PAREBEN_OK) msgs[d] = g_err;                // g_err is thread-local: carry the text back
         });
@@ -1026,15 +1162,25 @@ extern "C" int pareben_cv_grid(const double *basis, int n, int k, const double *
     return PAREBEN_OK;
 }
 
+extern "C" int pareben_cv_grid(const double *basis, int n, int k, const double *target, const int *fold_id,
+                               int n_folds, const double *alpha, const double *lambda, int n_grid, int epis,
+                               int prior, int n_devices, int device, int shard, int n_shards, double *fold_err,
+                               int *status, int *n_selected)
+{
+    return pareben_cv_grid_multi(basis, n, k, target, 1, fold_id, n_folds, alpha, lambda, n_grid, epis, prior, n_devices, device,
+                                 shard, n_shards, fold_err, status, n_selected);
+}
+
 extern "C" int pareben_fit(pareben_problem *p, double alpha, double lambda, double *beta_table, double *wald,
                            double *intercept, double *extra, int *status)
 {
     if (!p || !beta_table) return fail(PAREBEN_EINVAL, "pareben_fit: bad argument");
     if (p->n_folds != 0) return fail(PAREBEN_EINVAL, "pareben_fit needs a problem created with n_folds == 0");
+    if (p->n_targets != 1) return fail(PAREBEN_EINVAL, "pareben_fit needs a problem with one response");
     DumpBuffers dump;
     int fold = 0, st = 0;
     double err = 0;
-    int rc = run_fits_impl(p, 1, &fold, &alpha, &lambda, &err, &st, nullptr, nullptr, &dump);
+    int rc = run_fits_impl(p, 1, nullptr, &fold, &alpha, &lambda, &err, &st, nullptr, nullptr, &dump);
     if (rc != PAREBEN_OK) return rc;
     const int k = p->k, kc = p->kc;
     const int M = dump.m[0];
@@ -1076,23 +1222,27 @@ extern "C" int pareben_fit(pareben_problem *p, double alpha, double lambda, doub
 }
 
 // The grid call on a problem that is already resident (one upload serves BuildGrid's lambda_max, the grid and any
-// LocalSearch refinement): same table layout and shard assignment as pareben_cv_grid.
-extern "C" int pareben_problem_cv_grid(pareben_problem *p, const double *alpha, const double *lambda, int n_grid, int shard,
-                                       int n_shards, double *fold_err, int *status, int *n_selected)
+// LocalSearch refinement): same table layout and shard assignment as pareben_cv_grid_multi.
+extern "C" int pareben_problem_cv_grid_multi(pareben_problem *p, const double *alpha, const double *lambda, int n_grid, int shard,
+                                             int n_shards, double *fold_err, int *status, int *n_selected)
 {
     if (!p || !alpha || !lambda || !fold_err || n_grid < 1) return fail(PAREBEN_EINVAL, "pareben_problem_cv_grid: bad argument");
     if (p->n_folds < 1) return fail(PAREBEN_EINVAL, "pareben_problem_cv_grid needs a problem created with folds");
     if (n_shards < 1 || shard < 0 || shard >= n_shards) return fail(PAREBEN_EINVAL, "pareben_problem_cv_grid: bad shard");
-    const int nf = p->n_folds, total = n_grid * nf;
+    if ((long long)p->n_targets * n_grid * p->n_folds > 0x7fffffffLL) return fail(PAREBEN_EINVAL, "pareben_problem_cv_grid: more than 2^31 - 1 fits");
+    const int nf = p->n_folds, rows = p->n_targets * n_grid, total = rows * nf;
     std::vector<int> mine(total);
     int m = 0;
-    int rc = pareben_shard_plan(lambda, n_grid, nf, shard, n_shards, mine.data(), &m);
+    int rc = pareben_shard_plan(lambda, rows, nf, shard, n_shards, mine.data(), &m);
     if (rc != PAREBEN_OK || m == 0) return rc;
-    std::vector<int> fold(m), st(m), ns(m);
+    std::vector<int> tg(m), fold(m), st(m), ns(m);
     std::vector<double> a(m), l(m), err(m);
-    for (int i = 0; i < m; i++) { fold[i] = mine[i] % nf + 1; a[i] = alpha[mine[i] / nf]; l[i] = lambda[mine[i] / nf]; }
+    for (int i = 0; i < m; i++) {
+        const int row = mine[i] / nf;
+        tg[i] = row / n_grid; fold[i] = mine[i] % nf + 1; a[i] = alpha[row]; l[i] = lambda[row];
+    }
     p->grid_fits_hint = total;
-    rc = pareben_run_fits(p, m, fold.data(), a.data(), l.data(), err.data(), st.data(), ns.data(), nullptr);
+    rc = run_fits_impl(p, m, tg.data(), fold.data(), a.data(), l.data(), err.data(), st.data(), ns.data(), nullptr, nullptr);
     p->grid_fits_hint = 0;
     if (rc != PAREBEN_OK) return rc;
     for (int i = 0; i < m; i++) {
@@ -1101,6 +1251,13 @@ extern "C" int pareben_problem_cv_grid(pareben_problem *p, const double *alpha, 
         if (n_selected) n_selected[mine[i]] = ns[i];
     }
     return PAREBEN_OK;
+}
+
+extern "C" int pareben_problem_cv_grid(pareben_problem *p, const double *alpha, const double *lambda, int n_grid, int shard,
+                                       int n_shards, double *fold_err, int *status, int *n_selected)
+{
+    if (p && p->n_targets != 1) return fail(PAREBEN_EINVAL, "pareben_problem_cv_grid: the problem holds several responses (use pareben_problem_cv_grid_multi)");
+    return pareben_problem_cv_grid_multi(p, alpha, lambda, n_grid, shard, n_shards, fold_err, status, n_selected);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1161,56 +1318,77 @@ extern "C" void ElasticNetBinaryNEfull(double *BASIS, double *Targets, double *a
               logLIKELIHOOD, 2 * *kdim, 4);
 }
 
-extern "C" int pareben_lambda_max(pareben_problem *p, double *lambda_max)
+namespace {
+template <bool EPIS>
+void launch_lambda_max(int T, int nb, cudaStream_t s, const double *X, int n, int k, int c0, int c1, const double *resp, double *out)
+{   // response tile: 1 (a single response keeps the FMA pipe for itself), else the smallest of 4 / 8 / 16 that covers T
+    if (T == 1) lambda_max_multi_kernel<EPIS, 1><<<nb, LM_THREADS, 0, s>>>(X, n, k, c0, c1, resp, T, out);
+    else if (T <= 4) lambda_max_multi_kernel<EPIS, 4><<<nb, LM_THREADS, 0, s>>>(X, n, k, c0, c1, resp, T, out);
+    else if (T <= 8) lambda_max_multi_kernel<EPIS, 8><<<nb, LM_THREADS, 0, s>>>(X, n, k, c0, c1, resp, T, out);
+    else lambda_max_multi_kernel<EPIS, 16><<<nb, LM_THREADS, 0, s>>>(X, n, k, c0, c1, resp, T, out);
+}
+}  // namespace
+
+extern "C" int pareben_lambda_max_multi(pareben_problem *p, double *lambda_max)
 {
     if (!p || !lambda_max) return fail(PAREBEN_EINVAL, "pareben_lambda_max: bad argument");
     try {
         CU(cudaSetDevice(p->device));
         // GetLambdaMax works on ALL rows (R/BuildGrid.R:5-32): build a row-major copy once.
-        const int n = p->n, k = p->k;
-        std::vector<double> y(n);
-        CU(cudaMemcpy(y.data(), p->d_y, sizeof(double) * n, cudaMemcpyDeviceToHost));
-        long double s = 0; for (double v : y) s += v;
-        long double mean = s / n, t = 0; for (double v : y) t += (v - mean);
-        mean += t / n;
-        std::vector<double> centred(n), resp(n);
-        long double ss = 0;
-        for (int i = 0; i < n; i++) { centred[i] = (double)(y[i] - (double)mean); ss += (long double)centred[i] * centred[i]; }
-        const double nrm = std::sqrt((double)ss);
-        for (int i = 0; i < n; i++) resp[i] = centred[i] / nrm;
+        const int n = p->n, k = p->k, T = p->n_targets;
+        std::vector<double> y((size_t)n * T), centred((size_t)n * T), resp((size_t)n * T);
+        CU(cudaMemcpy(y.data(), p->d_y, sizeof(double) * n * T, cudaMemcpyDeviceToHost));
+        for (int r = 0; r < T; r++) {
+            const double *yr = y.data() + (size_t)r * n;
+            double *cr = centred.data() + (size_t)r * n, *rr = resp.data() + (size_t)r * n;
+            long double s = 0; for (int i = 0; i < n; i++) s += yr[i];
+            long double mean = s / n, t = 0; for (int i = 0; i < n; i++) t += (yr[i] - mean);
+            mean += t / n;
+            long double ss = 0;
+            for (int i = 0; i < n; i++) { cr[i] = (double)(yr[i] - (double)mean); ss += (long double)cr[i] * cr[i]; }
+            const double nrm = std::sqrt((double)ss);
+            for (int i = 0; i < n; i++) rr[i] = cr[i] / nrm;
+        }
         // scratch comes from the problem's pooled allocations (returned to the pool with the problem; nothing to leak on error)
-        double *d_rows_x = p->dalloc<double>((size_t)n * k), *d_resp = p->dalloc<double>(n);
+        double *d_rows_x = p->dalloc<double>((size_t)n * k), *d_resp = p->dalloc<double>((size_t)n * T);
+        double *d_max = p->dalloc<double>(T);
         int *d_rows = p->dalloc<int>(n);
         std::vector<int> rows(n); for (int i = 0; i < n; i++) rows[i] = i;
         CU(cudaMemcpy(d_rows, rows.data(), sizeof(int) * n, cudaMemcpyHostToDevice));
+        CU(cudaMemsetAsync(d_max, 0, sizeof(double) * T, p->stream));
         gather_rows_kernel<<<dim3((n + 31) / 32, (k + 31) / 32), dim3(32, 8), 0, p->stream>>>(p->d_Xcol, n, k, d_rows, n, d_rows_x);
-        double best = std::log(1.1);
         auto pass = [&](int c0, int c1, const std::vector<double> &r, bool epis) {
-            const int nb = (c1 - c0 + 255) / 256;
+            const int nb = (c1 - c0 + LM_THREADS - 1) / LM_THREADS;
             if (nb <= 0) return;
-            CU(cudaMemcpyAsync(d_resp, r.data(), sizeof(double) * n, cudaMemcpyHostToDevice, p->stream));
-            double *d_max = p->dalloc<double>(nb);
-            if (epis) lambda_max_kernel<true><<<nb, 256, 0, p->stream>>>(d_rows_x, n, k, c0, c1, d_resp, d_max);
-            else lambda_max_kernel<false><<<nb, 256, 0, p->stream>>>(d_rows_x, n, k, c0, c1, d_resp, d_max);
+            CU(cudaMemcpyAsync(d_resp, r.data(), sizeof(double) * n * T, cudaMemcpyHostToDevice, p->stream));
+            (epis ? launch_lambda_max<true> : launch_lambda_max<false>)(T, nb, p->stream, d_rows_x, n, k, c0, c1, d_resp, d_max);
             CU(cudaGetLastError());
-            std::vector<double> hm(nb);
-            CU(cudaMemcpyAsync(hm.data(), d_max, sizeof(double) * nb, cudaMemcpyDeviceToHost, p->stream));
-            CU(cudaStreamSynchronize(p->stream));
-            for (double v : hm) if (v > best) best = v;
+            CU(cudaStreamSynchronize(p->stream));      // r may be the next pass's source
         };
         pass(0, k, resp, false);                       // main effects against the normalised response (:14-19)
         if (p->epis) pass(k, p->kc, centred, true);    // pairs against the UN-normalised centred response (:24-27)
-        *lambda_max = best;
+        std::vector<double> hm(T);
+        CU(cudaMemcpyAsync(hm.data(), d_max, sizeof(double) * T, cudaMemcpyDeviceToHost, p->stream));
+        CU(cudaStreamSynchronize(p->stream));
+        const double floor_ = std::log(1.1);
+        for (int r = 0; r < T; r++) lambda_max[r] = hm[r] > floor_ ? hm[r] : floor_;
     } catch (std::pair<int, std::string> &e) {
         return fail(e.first, e.second);
     }
     return PAREBEN_OK;
 }
 
+extern "C" int pareben_lambda_max(pareben_problem *p, double *lambda_max)
+{
+    if (p && p->n_targets != 1) return fail(PAREBEN_EINVAL, "pareben_lambda_max: the problem holds several responses (use pareben_lambda_max_multi)");
+    return pareben_lambda_max_multi(p, lambda_max);
+}
+
 extern "C" int pareben_sl_filter(pareben_problem *p, double tau_main, double tau_pair, int capacity, int *cand, double *stat,
                                  int *n_kept)
 {
     if (!p || !n_kept || capacity < 0) return fail(PAREBEN_EINVAL, "pareben_sl_filter: bad argument");
+    if (p->n_targets != 1) return fail(PAREBEN_EINVAL, "pareben_sl_filter needs a problem with one response");
     try {
         CU(cudaSetDevice(p->device));
         const int n = p->n, k = p->k;

@@ -56,7 +56,7 @@ constexpr int ADV_THREADS = 256;
 
 struct StreamFit {
     // task
-    int fold, out_index;
+    int fold, target, out_index;           // target: response index, as FitTask::target
     double lambda, alpha_en;
     // control state of the solver between two rounds (the loop-carried scalars of gauss_fit())
     int phase;

@@ -86,7 +86,7 @@ stream_advance_kernel(Problem P, Variant v, StreamFit *fits, int n_fits, StreamS
     StreamFit &G = fits[blockIdx.x];
     if (G.phase == SP_DONE) return;
     StreamFit s = G;                                          // local copy: pointers and scalars (written back at the end)
-    const FoldData F = P.folds[s.fold];
+    const FoldData F = P.folds[s.target * (P.n_folds + 1) + s.fold];
     const int N = F.ntr, K = P.K, cap = P.cap, T = blockDim.x, LD = phi_ld(N);
     const int lane_ = threadIdx.x & 31, wid_ = threadIdx.x >> 5, nw_ = T >> 5;
     const double *y = F.ytr;

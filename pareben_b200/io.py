@@ -7,7 +7,8 @@
   * .rda / .RDS (R's XDR serialisation; the package's bundled BASIS.rda, y.rda, ...), via pareben_b200.rdata;
   * .npy / .npz for convenience.
 `load_problem` applies the row selection of the published workflow (rows of the genotype table whose sample id occurs
-in the phenotype table, in phenotype order: SL_filter.R:14 `genotype[pheno[,1],]`)."""
+in the phenotype table, in phenotype order: SL_filter.R:14 `genotype[pheno[,1],]`); `load_problem_multi` does the same
+for several phenotype files of one design."""
 from __future__ import annotations
 
 import io as _io
@@ -89,20 +90,65 @@ def read_matrix(path: str, name: str | None = None):
     return M
 
 
+def _text_like(p: str) -> bool:
+    return os.path.splitext(p)[1].lower() in (".txt", ".tsv", ".zip", ".tab", "")
+
+
+def _genotype_rows(basis_path: str, pid):
+    """Rows of the genotype text in the order of the phenotype ids `pid` (None: as stored)."""
+    ids, _names, X = read_genotype_text(basis_path)
+    if pid is not None:
+        pos = {s: i for i, s in enumerate(ids)}
+        missing = [s for s in pid if s not in pos]
+        if missing:
+            raise ValueError(f"{len(missing)} phenotype ids are absent from the genotype table (first: {missing[0]})")
+        X = X[[pos[s] for s in pid]]
+    return X
+
+
+def read_targets(paths, name: str | None = None):
+    """-> (sample_ids [n] or None, Targets [n, T]) from several response files, one response each (phenotype text or a
+    vector file), or from ONE .npy / .npz holding an n x T matrix.  Phenotype texts are joined on the sample id in the
+    order of the first file and must all list the same ids; files without ids are taken row for row."""
+    paths = list(paths)
+    if not paths:
+        raise ValueError("no response file given")
+    if len(paths) == 1 and os.path.splitext(paths[0])[1].lower() in (".npy", ".npz"):
+        Y = np.asarray(read_matrix(paths[0], name), dtype=np.float64)
+        return None, Y.reshape(-1, 1) if Y.ndim == 1 else Y
+    first_ids, cols = None, []
+    for j, p in enumerate(paths):
+        ids, v = read_phenotype_text(p) if _text_like(p) else (None, np.asarray(read_matrix(p, name), dtype=np.float64).ravel())
+        if j == 0:
+            first_ids = ids
+        elif (ids is None) != (first_ids is None):
+            raise ValueError(f"{p}: either every response file lists sample ids or none does ({paths[0]} differs)")
+        elif ids is not None:
+            pos = {s: i for i, s in enumerate(ids)}
+            if len(pos) != ids.size or ids.size != first_ids.size or set(pos) != set(first_ids.tolist()):
+                raise ValueError(f"{p}: sample ids differ from those of {paths[0]}")
+            v = v[[pos[s] for s in first_ids]]
+        elif v.size != cols[0].size:
+            raise ValueError(f"{p}: {v.size} values, {paths[0]} has {cols[0].size}")
+        cols.append(np.asarray(v, dtype=np.float64))
+    return first_ids, np.column_stack(cols)
+
+
+def load_problem_multi(basis_path: str, target_paths, basis_name: str | None = None, target_name: str | None = None):
+    """(BASIS [n, k], Targets [n, T]) for several responses of one design (read_targets).  With genotype text and
+    phenotype texts the genotype rows follow the ids of the first phenotype file, as in load_problem."""
+    pid, Y = read_targets(target_paths, target_name)
+    X = _genotype_rows(basis_path, pid) if _text_like(basis_path) and pid is not None else read_matrix(basis_path, basis_name)
+    return X, Y
+
+
 def load_problem(basis_path: str, target_path: str, basis_name: str | None = None, target_name: str | None = None):
     """(BASIS [n, k], Target [n]) from a pair of files.  Genotype text + two-column phenotype text are joined on the
     sample id (rows in phenotype order, SL_filter.R:14); everything else is taken row for row."""
-    text_like = lambda p: os.path.splitext(p)[1].lower() in (".txt", ".tsv", ".zip", ".tab", "")  # noqa: E731
+    text_like = _text_like
     if text_like(basis_path) and text_like(target_path):
         pid, y = read_phenotype_text(target_path)
-        ids, _names, X = read_genotype_text(basis_path)
-        if pid is not None:
-            pos = {s: i for i, s in enumerate(ids)}
-            missing = [s for s in pid if s not in pos]
-            if missing:
-                raise ValueError(f"{len(missing)} phenotype ids are absent from the genotype table (first: {missing[0]})")
-            X = X[[pos[s] for s in pid]]
-        return X, y
+        return _genotype_rows(basis_path, pid), y
     X = read_matrix(basis_path, basis_name)
     y = read_matrix(target_path, target_name) if not text_like(target_path) else read_phenotype_text(target_path)[1]
     return X, np.asarray(y, dtype=np.float64).ravel()
