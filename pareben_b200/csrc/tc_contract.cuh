@@ -137,7 +137,10 @@ __device__ inline void tc_digits(int j0, int ncols, int N, int nst, Val val, int
         (void)frexp(mx, &ex);                                   // mx = m 2^ex, m in [1/2, 1)
         const bool live = !bad && mx > 1e-290;                  // an all-zero (or denormal) column contributes zeros
         const double down = live ? scalbn(1.0, 55 - ex) : 0.0;  // |val * down| < 2^55, exact
-        if (lane == 0) bscale[jl] = bad ? __longlong_as_double(0x7ff8000000000000LL) : (live ? scalbn(1.0, ex + 1) : 0.0);
+        // the column's scale 2^(ex+1) is stored as 2^(ex-1), and Horner's last step multiplies by 2^-5 instead of 2^-7:
+        // 2^(ex+1) itself overflows for a column maximum >= 2^1022 (ex = 1023, 1024).  Horner's sum is never subnormal,
+        // so both forms are one exact power-of-two scaling (rounded only on overflow) and agree bit for bit below 2^1022.
+        if (lane == 0) bscale[jl] = bad ? __longlong_as_double(0x7ff8000000000000LL) : (live ? scalbn(1.0, ex - 1) : 0.0);
         int8_t *colp = planes + (size_t)jl * TC_COL_BYTES;
         for (int p4 = 4 * lane; p4 < nst * TC_KS; p4 += 128) {
             unsigned wout[TC_PLANES];
@@ -251,7 +254,7 @@ __device__ inline void tc_contract(const FoldData &F, int Kc, int R, Col col, De
                     if (jj < je && live) {
                         double v = 0.0;
 #pragma unroll
-                        for (int s = TC_PLANES - 1; s >= 0; s--) v = (v + (double)acc[8 * u + s]) * 0.0078125;   // Horner, 128^-1 exact
+                        for (int s = TC_PLANES - 1; s >= 0; s--) v = (v + (double)acc[8 * u + s]) * (s ? 0.0078125 : 0.03125);   // Horner, 128^-1 exact
                         v *= bscale[jj];
                         const int j = j0 + jj;
                         if (j < R) { bool dv = false; double *row = dest(j, dv); row[c] = dv ? div_by(v, sc, isc) : v; }
@@ -265,7 +268,7 @@ __device__ inline void tc_contract(const FoldData &F, int Kc, int R, Col col, De
                 if (live) {
                     double v = 0.0;
 #pragma unroll
-                    for (int s = TC_PLANES - 1; s >= 0; s--) v = (v + (double)acc[s]) * 0.0078125;
+                    for (int s = TC_PLANES - 1; s >= 0; s--) v = (v + (double)acc[s]) * (s ? 0.0078125 : 0.03125);
                     bb_out[c] = v * bscale[0];
                 }
             }
