@@ -67,7 +67,7 @@ void pareben_problem_destroy(pareben_problem *p);
  * only the training and test vectors are kept per (response, fold).  Every fit of such a problem gives bitwise the result
  * of the same fit on a problem created with that response alone.  pareben_problem_create is the n_targets = 1 case.
  * pareben_fit, pareben_lambda_max, pareben_sl_filter and pareben_problem_cv_grid fail with PAREBEN_EINVAL on a problem
- * with n_targets > 1 (use the _multi calls; the final model of a response is fitted on a single-response problem). */
+ * with n_targets > 1 (use the _multi calls; the final models of several responses come from pareben_fit_batch). */
 int pareben_problem_create_multi(pareben_problem **out, int device, const double *basis, int n, int k,
                                  const double *targets, int n_targets, const int *fold_id, int n_folds, int epis, int prior);
 
@@ -140,6 +140,27 @@ int pareben_shard_plan(const double *lambda, int n_grid, int n_folds, int shard,
  *   MainEff.c:227) or log-likelihood (binomial, NEmainEff.c:805). */
 int pareben_fit(pareben_problem *p, double alpha, double lambda, double *beta_table, double *wald,
                 double *intercept, double *extra, int *status);
+
+/* Upper bound on the effects one fit of this problem can report (the basis cap, without the binomial intercept slot). */
+int pareben_max_effects(pareben_problem *p, int *max_effects);
+
+/* pareben_fit for n_fits fits in one launch: fit i trains response target[i] on fold[i]
+ * (0 = all rows, problem created with n_folds == 0; f >= 1 = the training rows of fold f, i.e. fold f's CV model)
+ * at (alpha[i], lambda[i]).  Compact records, row-major with stride max_effects (>= pareben_max_effects, else EINVAL):
+ *   n_effects[i], cand[i*max_effects + j] = 1-based candidate id in Used order (the reference's Used / Beta[,5]; main
+ *   effects first, then pairs row-major in i < j), beta[..] = mu/scale, var[..] = sigma_jj/scale^2 (entries j >=
+ *   n_effects[i] are 0), scalars[4*i + 0..3] = wald, intercept[0], intercept[1] (binomial; 0 for Gaussian), residual
+ *   variance | log-likelihood, status[i] (PAREBEN_FIT_* bits), fold_err[i] (hold-out score of a fold fit, the value
+ *   pareben_run_fits gives; 0 for fold 0).  Any output may be NULL except n_effects/cand/beta when max_effects > 0.
+ * Each record is bitwise the model pareben_fit returns for that fit alone, with two limits: the Gram organisation of the
+ * Gaussian cached kernels is chosen by the fits of the call (pin it with PAREBEN_GRAM to compare calls), and in streaming
+ * mode the basis cap is sized by the largest number of fits one response has in the call, so a path of many fits on one
+ * response can get a lower cap than a lone fit (one fit per response gets the cap of pareben_fit).  Record memory is
+ * n_fits x ((1 + cap) ints + (2 cap + 4) doubles) on the device; PAREBEN_ENOMEM if it does not fit.  Nothing is written
+ * to the outputs unless the whole call succeeds; n_fits == 0 is a no-op. */
+int pareben_fit_batch(pareben_problem *p, int n_fits, const int *target, const int *fold, const double *alpha,
+                      const double *lambda, int max_effects, int *n_effects, int *cand, double *beta, double *var,
+                      double *scalars, int *status, double *fold_err);
 
 /* EBEN's own four `.C` entry points, same names, argument lists and output layouts, as wrappers over
  * pareben_problem_create + pareben_fit: an R session that loads this library in place of EBEN's (useDynLib / PACKAGE

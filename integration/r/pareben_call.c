@@ -9,6 +9,7 @@
  *   pareben_cv_grid_multi_call  the same for the T columns of a response matrix against one BASIS, in one call
  *   pareben_lambda_max_call  GetLambdaMax (R/BuildGrid.R:5-32), incl. the K^2/2 pair scan of Epis = "yes"
  *   pareben_fit_call         EBelasticNet.Gaussian / .Binomial: the `.C` outputs of one all-rows fit
+ *   pareben_fit_batch_call   the final models of the T columns of a response matrix against one BASIS, in one call
  *   pareben_sl_filter_call   the single-locus prefilter of SL_filter.R
  * EBEN's own `.C` symbols (elasticNetLinearNeMainEff, ...) are exported by libpareben.so itself under their original
  * names: EBEN's R wrappers need no shim at all, only `useDynLib(pareben)`. */
@@ -131,6 +132,42 @@ SEXP pareben_fit_call(SEXP BASIS, SEXP Target, SEXP lambda, SEXP alpha, SEXP epi
     return out;
 }
 
+/* .Call("pareben_fit_batch_call", BASIS, Targets, lambda, alpha, epis, prior, device)
+ * Targets: n x T double matrix, one response per column; lambda, alpha: length T (response t at (lambda[t], alpha[t])).
+ * One problem (no folds, T responses) and one pareben_fit_batch launch.  Returns the compact records:
+ * list(n_effects = integer[T], cand = integer matrix[maxEffects x T] (1-based candidate ids in Used order: main effects
+ * 1..k, then pairs i < j row-major), beta, var = matrices[maxEffects x T] (mu/scale, sigma_jj/scale^2), scalars =
+ * matrix[4 x T] (WaldScore, Intercept[1], Intercept[2] (binomial), residual variance | logLikelihood), status = integer[T]).
+ * Column t holds what pareben_fit_call's Beta has for Targets[, t] alone, bitwise; rows past n_effects[t] are 0. */
+SEXP pareben_fit_batch_call(SEXP BASIS, SEXP Targets, SEXP lambda, SEXP alpha, SEXP epis, SEXP prior, SEXP device)
+{
+    int n, k, nt, T;
+    dims(BASIS, &n, &k);
+    dims(Targets, &nt, &T);
+    if (nt != n) error("Targets must have nrow(BASIS) rows");
+    if (T < 1 || LENGTH(lambda) != T || LENGTH(alpha) != T) error("lambda and alpha must have one entry per column of Targets");
+    pareben_problem *p = NULL;
+    int rc = pareben_problem_create_multi(&p, asInteger(device), REAL(BASIS), n, k, REAL(Targets), T, NULL, 0, asInteger(epis),
+                                          asInteger(prior));
+    int me = 0;
+    if (rc == PAREBEN_OK) rc = pareben_max_effects(p, &me);
+    if (rc != PAREBEN_OK) { if (p) pareben_problem_destroy(p); error("pareben_fit_batch failed (%d): %s", rc, pareben_last_error()); }
+    SEXP ne = PROTECT(allocVector(INTSXP, T)), cand = PROTECT(allocMatrix(INTSXP, me, T));
+    SEXP beta = PROTECT(allocMatrix(REALSXP, me, T)), var = PROTECT(allocMatrix(REALSXP, me, T));
+    SEXP sc = PROTECT(allocMatrix(REALSXP, 4, T)), st = PROTECT(allocVector(INTSXP, T));
+    SEXP target = PROTECT(allocVector(INTSXP, T)), fold = PROTECT(allocVector(INTSXP, T));
+    for (int t = 0; t < T; t++) { INTEGER(target)[t] = t; INTEGER(fold)[t] = 0; }
+    rc = pareben_fit_batch(p, T, INTEGER(target), INTEGER(fold), REAL(alpha), REAL(lambda), me, INTEGER(ne), INTEGER(cand),
+                           REAL(beta), REAL(var), REAL(sc), INTEGER(st), NULL);
+    pareben_problem_destroy(p);
+    if (rc != PAREBEN_OK) { UNPROTECT(8); error("pareben_fit_batch failed (%d): %s", rc, pareben_last_error()); }
+    const char *names[] = {"n_effects", "cand", "beta", "var", "scalars", "status"};
+    SEXP items[] = {ne, cand, beta, var, sc, st};
+    SEXP out = named_list(6, names, items);
+    UNPROTECT(8);
+    return out;
+}
+
 /* .Call("pareben_sl_filter_call", BASIS, Target, tauMain, tauPair, epis, device)
  * -> list(cand = 0-based candidate ids ascending (0..k-1 main effects, then pairs i < j row-major), stat) */
 SEXP pareben_sl_filter_call(SEXP BASIS, SEXP Target, SEXP tauMain, SEXP tauPair, SEXP epis, SEXP device)
@@ -158,6 +195,7 @@ static const R_CallMethodDef call_methods[] = {
     {"pareben_cv_grid_multi_call", (DL_FUNC)&pareben_cv_grid_multi_call, 10},
     {"pareben_lambda_max_call", (DL_FUNC)&pareben_lambda_max_call, 4},
     {"pareben_fit_call", (DL_FUNC)&pareben_fit_call, 7},
+    {"pareben_fit_batch_call", (DL_FUNC)&pareben_fit_batch_call, 7},
     {"pareben_sl_filter_call", (DL_FUNC)&pareben_sl_filter_call, 6},
     {NULL, NULL, 0}
 };

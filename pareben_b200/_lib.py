@@ -45,6 +45,8 @@ SIGNATURES = {
     "ElasticNetBinaryNEfull": (None, [_dp, _dp, _dp, _dp, _dp, _dp, _dp, _dp, _ip, _ip, _ip, _ip]),
     "pareben_shard_plan": (ctypes.c_int, [_dp, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, _ip, _ip]),
     "pareben_fit": (ctypes.c_int, [_vp, ctypes.c_double, ctypes.c_double, _dp, _dp, _dp, _dp, _ip]),
+    "pareben_max_effects": (ctypes.c_int, [_vp, _ip]),
+    "pareben_fit_batch": (ctypes.c_int, [_vp, ctypes.c_int, _ip, _ip, _dp, _dp, ctypes.c_int, _ip, _ip, _dp, _dp, _dp, _ip, _dp]),
     "pareben_lambda_max": (ctypes.c_int, [_vp, _dp]),
     "pareben_lambda_max_multi": (ctypes.c_int, [_vp, _dp]),
     "pareben_sl_filter": (ctypes.c_int, [_vp, ctypes.c_double, ctypes.c_double, ctypes.c_int, _ip, _dp, _ip]),
@@ -231,6 +233,32 @@ class Problem:
         wald = np.zeros(1); icpt = np.zeros(2); extra = np.zeros(1); st = np.zeros(1, np.int32)
         _check(load().pareben_fit(self._h, float(alpha), float(lam), _d(beta), _d(wald), _d(icpt), _d(extra), _i(st)))
         return beta.reshape((rows, cols), order="F"), float(wald[0]), icpt, float(extra[0]), int(st[0])
+
+    def max_effects(self) -> int:
+        """pareben_max_effects: the most effects one fit of this problem can report."""
+        out = ctypes.c_int(0)
+        _check(load().pareben_max_effects(self._h, ctypes.byref(out)))
+        return out.value
+
+    def fit_batch(self, target, fold, alpha, lam):
+        """pareben_fit_batch: the final models of len(target) fits in one launch (fit i: response target[i], fold[i]: 0 =
+        all rows, f >= 1 = fold f's training rows, at (alpha[i], lam[i])).  Returns a dict of compact records:
+        n_effects (m,), cand (m, max_effects) 1-based candidate ids in Used order, beta and var (m, max_effects),
+        scalars (m, 4) = wald, intercept[0], intercept[1], residual variance | log-likelihood, status (m,), fold_err (m,)."""
+        target = np.ascontiguousarray(target, dtype=np.int32).ravel()
+        fold = np.ascontiguousarray(fold, dtype=np.int32).ravel()
+        alpha = np.ascontiguousarray(alpha, dtype=np.float64).ravel()
+        lam = np.ascontiguousarray(lam, dtype=np.float64).ravel()
+        m = target.size
+        if fold.size != m or alpha.size != m or lam.size != m:
+            raise ValueError("target, fold, alpha and lambda must have equal length")
+        me = self.max_effects()
+        out = {"n_effects": np.zeros(m, np.int32), "cand": np.zeros((m, me), np.int32), "beta": np.zeros((m, me)),
+               "var": np.zeros((m, me)), "scalars": np.zeros((m, 4)), "status": np.zeros(m, np.int32), "fold_err": np.zeros(m)}
+        _check(load().pareben_fit_batch(self._h, m, _i(target), _i(fold), _d(alpha), _d(lam), me, _i(out["n_effects"]),
+                                        _i(out["cand"]), _d(out["beta"]), _d(out["var"]), _d(out["scalars"]), _i(out["status"]),
+                                        _d(out["fold_err"])))
+        return out
 
     def lambda_max(self) -> float:
         out = np.zeros(1)

@@ -10,6 +10,8 @@ image, so this Python layer stands where R/CrossValidate.R etc. would call `.Cal
                   one upload and one batched fit call, each result equal to CrossValidate on that response
   EBelasticNet_Gaussian / EBelasticNet_Binomial  (final model after CV, README.md:89-94;
                   /root/reference/EBEN_orig/R/EBelasticNet.Gaussian.R, .Binomial.R)
+  EBelasticNetMulti  (no reference counterpart) the final models of T responses of one design in one fit call, each
+                  equal to EBelasticNet_Gaussian / _Binomial on that response
 The foreach/%dopar% fan-out (CrossValidate.R:66-70, 88-92; LocalSearch.R:67-104) is replaced
 by ONE batched launch per GPU; with torch.distributed initialised (one process per GPU) the
 fits are sharded by cost-aware interleaving and merged with one tiny all-reduce.
@@ -273,6 +275,19 @@ def CrossValidateMulti(BASIS, Targets, nFolds, foldId=0, Epis="no", prior="gauss
     return [_global_result(grids[t], err[t], status[t], nsel[t], folds, nFolds, prior_key) for t in range(Y.shape[1])]
 
 
+def candidate_loci(cand, k: int):
+    """1-based loci (i, j) of 0-based candidate ids, the numbering of the whole library: main effect c < k is (c+1, c+1),
+    pair c = k + i*(2k-i-1)/2 + (j-i-1) with i < j (the enumeration of elasticNetLinearNeFull2.c:115-134) is (i+1, j+1)."""
+    c = np.asarray(cand, dtype=np.int64)
+    pc = np.maximum(c - k, 0)
+    i = np.floor(((2 * k - 1) - np.sqrt((2 * k - 1) ** 2 - 8.0 * pc)) / 2).astype(np.int64)
+    i = np.where(i * (2 * k - i - 1) // 2 > pc, i - 1, i)
+    i = np.where((i + 1) * (2 * k - i - 2) // 2 <= pc, i + 1, i)
+    j = pc - i * (2 * k - i - 1) // 2 + i + 1
+    main = c < k
+    return np.where(main, c, i) + 1, np.where(main, c, j) + 1
+
+
 def _weight_table(table, keep, epis, n):
     ncol = table.shape[1]
     blup = table[keep] if keep.size else np.zeros((1, ncol))
@@ -309,6 +324,54 @@ def EBelasticNet_Binomial(BASIS, Target, lam, alpha, Epis="no", verbose=0, devic
             "Intercept": icpt.copy(), "lambda": lam, "alpha": alpha, "status": status}
 
 
+def _record_weight(n_eff, cand, beta, var, epis, gaussian, k, n):
+    """The `weight` table of EBelasticNet_Gaussian / _Binomial from one compact pareben_fit_batch record (cand 1-based, in
+    Used order), through _weight_table on the record's own rows: the rows and their order are those the reference-layout
+    table of pareben_fit gives.  Gaussian main and binomial main: effects with beta != 0 in candidate order; Gaussian Epis:
+    every used candidate in candidate order; binomial Epis: Used order, beta != 0; Epis then sorts main before pairs."""
+    m = int(n_eff)
+    c = np.asarray(cand[:m], dtype=np.int64) - 1
+    b, v = np.asarray(beta[:m], dtype=np.float64), np.asarray(var[:m], dtype=np.float64)
+    if gaussian or not epis:
+        order = np.argsort(c, kind="stable")                  # candidate order, as the tables indexed by candidate id
+        c, b, v = c[order], b[order], v[order]
+    li, lj = candidate_loci(c, k)
+    table = np.column_stack([li.astype(np.float64), lj.astype(np.float64), b, v])
+    keep = np.arange(m) if (gaussian and epis) else np.nonzero(b != 0)[0]
+    return _weight_table(table, keep, epis, n)
+
+
+def EBelasticNetMulti(BASIS, Targets, lam, alpha, Epis="no", prior="gaussian", device: int | None = None):
+    """The final model of each column of Targets (n x T) against the same BASIS, from one problem upload and one
+    pareben_fit_batch launch.  lam and alpha have length T, or are scalars applied to every response.  Returns a list of
+    T dicts; entry t equals EBelasticNet_Gaussian / _Binomial(BASIS, Targets[:, t], lam[t], alpha[t], Epis) key for key.
+    Every response must be observed on every row."""
+    X = _as_matrix(BASIS)
+    Y = _targets(X, Targets)
+    T = Y.shape[1]
+    lam_t = np.broadcast_to(np.asarray(lam, dtype=np.float64), (T,)) if np.ndim(lam) == 0 else np.asarray(lam, dtype=np.float64)
+    alpha_t = np.broadcast_to(np.asarray(alpha, dtype=np.float64), (T,)) if np.ndim(alpha) == 0 else np.asarray(alpha, dtype=np.float64)
+    if lam_t.shape != (T,) or alpha_t.shape != (T,):
+        raise ValueError(f"lam and alpha must be scalars or have one entry per response ({T})")
+    epis, gaussian = Epis == "yes", prior == "gaussian"
+    with _lib.Problem(X, Y, None, 0, epis, "gaussian" if gaussian else "binomial", device) as p:
+        r = p.fit_batch(np.arange(T), np.zeros(T, np.int32), alpha_t, lam_t)
+    n, k = X.shape
+    out = []
+    for t in range(T):
+        w = _record_weight(r["n_effects"][t], r["cand"][t], r["beta"][t], r["var"][t], epis, gaussian, k, n)
+        wald, i0, i1, extra = (float(v) for v in r["scalars"][t])
+        lt = lam[t] if np.ndim(lam) else lam
+        at = alpha[t] if np.ndim(alpha) else alpha
+        if gaussian:
+            out.append({"weight": w, "WaldScore": wald, "Intercept": i0, "residVar": extra, "lambda": lt, "alpha": at,
+                        "status": int(r["status"][t])})
+        else:
+            out.append({"weight": w, "logLikelihood": extra, "WaldScore": wald, "Intercept": np.array([i0, i1]), "lambda": lt,
+                        "alpha": at, "status": int(r["status"][t])})
+    return out
+
+
 def SLFilter(BASIS, Target, tau_main: float = 0.02, tau_pair: float = 0.05, Epis: str = "yes", device: int | None = None):
     """The single-locus prefilter that precedes CrossValidate in the published workflow
     (paper_materials/Real Data Analysis/SL_filter.R:17-52): standardised-correlation screening of the main-effect
@@ -319,10 +382,5 @@ def SLFilter(BASIS, Target, tau_main: float = 0.02, tau_pair: float = 0.05, Epis
     with _lib.Problem(X, Target, None, 0, Epis == "yes", "gaussian", device=device) as p:
         cand, stat = p.sl_filter(tau_main, tau_pair)
     main = cand < k
-    pc = cand[~main].astype(np.int64) - k
-    # invert c = i*(2k-i-1)/2 + (j-i-1) for i < j (the enumeration of elasticNetLinearNeFull2.c:115-134)
-    i = np.floor(((2 * k - 1) - np.sqrt((2 * k - 1) ** 2 - 8.0 * pc)) / 2).astype(np.int64)
-    i = np.where(i * (2 * k - i - 1) // 2 > pc, i - 1, i)
-    i = np.where((i + 1) * (2 * k - i - 2) // 2 <= pc, i + 1, i)
-    j = pc - i * (2 * k - i - 1) // 2 + i + 1
-    return {"main": cand[main] + 1, "pairs": np.stack([i + 1, j + 1], axis=1), "stat_main": stat[main], "stat_pairs": stat[~main]}
+    return {"main": cand[main] + 1, "pairs": np.stack(candidate_loci(cand[~main], k), axis=1), "stat_main": stat[main],
+            "stat_pairs": stat[~main]}

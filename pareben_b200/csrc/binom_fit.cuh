@@ -518,21 +518,23 @@ __device__ void binom_fit(const Problem &P, const FoldData &F, const Variant &v,
         if (out.n_selected) out.n_selected[o] = nsel;
         if (out.n_iter) out.n_iter[o] = iter;
         if (out.flops) { atomicAdd(out.flops, b.flops); if (b.tc_calls > 0) atomicAdd(out.flops + 2, b.tc_calls); }
-        if (out.m_out) {
-            out.m_out[0] = M - 1;
+        if (out.m_out) {          // full-model record of fit o (pareben_fit_batch); slot 0 is the intercept
+            out.m_out[o] = M - 1;
             double wd = 0;
             for (int i = 0; i < M; i++) {
                 double z = 0;
                 for (int j = 0; j < M; j++) z += s.mu[j] * s.H[i * M + j];
                 wd += z * s.mu[i];
             }
+            const size_t r = (size_t)o * out.dump_ld;
             for (int i = 1; i < M; i++) {
                 const int c = s.used[i - 1] - 1;
-                out.used_out[i - 1] = s.used[i - 1];
-                out.beta_out[i - 1] = s.mu[i] / scale[c];
-                out.var_out[i - 1] = s.sigma[i * M + i] / (scale[c] * scale[c]);
+                out.used_out[r + i - 1] = s.used[i - 1];
+                out.beta_out[r + i - 1] = s.mu[i] / scale[c];
+                out.var_out[r + i - 1] = s.sigma[i * M + i] / (scale[c] * scale[c]);
             }
-            out.scalars_out[0] = wd; out.scalars_out[1] = s.mu[0]; out.scalars_out[2] = s.sigma[0]; out.scalars_out[3] = loglik;
+            out.scalars_out[4 * (size_t)o + 0] = wd; out.scalars_out[4 * (size_t)o + 1] = s.mu[0];
+            out.scalars_out[4 * (size_t)o + 2] = s.sigma[0]; out.scalars_out[4 * (size_t)o + 3] = loglik;
         }
     }
     __syncthreads();

@@ -79,8 +79,10 @@ struct Sched {
 struct FitOutputs {
     double *fold_err;        // [n] indexed by out_index
     int *status, *n_selected, *n_iter;
-    // optional full-model dump for pareben_fit (batch of 1)
-    int *m_out; int *used_out; double *beta_out; double *var_out; double *scalars_out; // wald, intercept0, intercept1, extra
+    // optional full-model records (pareben_fit_batch; null in a CV launch): fit o writes m_out[o], used_out / beta_out /
+    // var_out[o * dump_ld + i] (i < m_out[o]) and scalars_out[4 o + 0..3] = wald, intercept0, intercept1, extra
+    int *m_out; int *used_out; double *beta_out; double *var_out; double *scalars_out;
+    int dump_ld;             // record stride: the basis cap of the launch
     double *flops;           // three accumulators (atomicAdd): [0] model flops (SURVEY 8d), [1] the part the Gram organisation avoided,
                              // [2] score contractions run on the int8 tensor cores
 };

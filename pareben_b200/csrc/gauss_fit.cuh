@@ -1829,22 +1829,24 @@ __device__ void gauss_fit(const Problem &P, const FoldData &F, const Variant &v,
         if (out.n_selected) out.n_selected[o] = nsel;
         if (out.n_iter) out.n_iter[o] = iter;
         if (out.flops) { atomicAdd(out.flops, g.flops); if (g.avoided > 0) atomicAdd(out.flops + 1, g.avoided); }
-        if (out.m_out) {          // full-model dump (pareben_fit)
-            out.m_out[0] = M;
+        if (out.m_out) {          // full-model record of fit o (pareben_fit_batch)
+            out.m_out[o] = M;
             double wd = 0;        // Wald score mu'H mu with H read at leading dimension M (:206-215)
             for (int i = 0; i < M; i++) {
                 double z = 0;
                 for (int j = 0; j < M; j++) z += s.mu[j] * s.H[i * M + j];
                 wd += z * s.mu[i];
             }
+            const size_t r = (size_t)o * out.dump_ld;
             for (int i = 0; i < M; i++) {
                 const int c = s.used[i] - 1;
-                out.used_out[i] = s.used[i];
-                out.beta_out[i] = s.mu[i] / scale[c];
-                out.var_out[i] = s.sigma[i * M + i] / (scale[c] * scale[c]);
+                out.used_out[r + i] = s.used[i];
+                out.beta_out[r + i] = s.mu[i] / scale[c];
+                out.var_out[r + i] = s.sigma[i * M + i] / (scale[c] * scale[c]);
             }
-            out.scalars_out[0] = wd; out.scalars_out[1] = b; out.scalars_out[2] = 0;
-            out.scalars_out[3] = 1 / (g.beta + 1e-10);
+            out.scalars_out[4 * (size_t)o + 0] = wd; out.scalars_out[4 * (size_t)o + 1] = b;
+            out.scalars_out[4 * (size_t)o + 2] = 0;
+            out.scalars_out[4 * (size_t)o + 3] = 1 / (g.beta + 1e-10);
         }
     }
     __syncthreads();

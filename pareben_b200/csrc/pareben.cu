@@ -12,6 +12,7 @@
 
 #include <algorithm>
 #include <map>
+#include <new>
 #include <tuple>
 #include <thread>
 #include <chrono>
@@ -329,20 +330,25 @@ static int reference_basis_max(int n_train, int k, int kc, int epis, int prior)
     return n_train > k ? 2 * k : (n_train < 200 ? 4 * k : k);                      // NeFull2.c:67-80
 }
 
+// basis cap of the cached kernels: the reference's basisMax, bounded (PAREBEN_BASIS_CAP, default 1024) so that the
+// per-block slab stays reasonable
+static int cached_cap(const pareben_problem *p)
+{
+    int cap = reference_basis_max(p->min_ntr, p->k, p->kc, p->epis, p->prior);
+    const char *env_cap = getenv("PAREBEN_BASIS_CAP");
+    int hard = env_cap ? atoi(env_cap) : 1024;
+    if (hard < 2) hard = 2;
+    if (p->prior == PAREBEN_BINOMIAL) cap += 1;       // slot 0 is the intercept
+    return std::max(2, std::min(cap, hard));
+}
+
 // The per-block work slabs are only needed by the fit kernel: they are sized and allocated at the first
 // pareben_run_fits / pareben_fit of a problem (lambda_max and the single-locus prefilter never touch them, and an
 // Epis problem's candidate cache can be far larger than those two need).  Throws like the CU() macro.
 static void ensure_slabs(pareben_problem *p)
 {
     if (p->d_slabs) return;
-    // basis cap: the reference's basisMax, bounded so that the per-block slab stays reasonable.
-    int cap = reference_basis_max(p->min_ntr, p->k, p->kc, p->epis, p->prior);
-    const char *env_cap = getenv("PAREBEN_BASIS_CAP");
-    int hard = env_cap ? atoi(env_cap) : 1024;
-    if (hard < 2) hard = 2;
-    if (p->prior == PAREBEN_BINOMIAL) cap += 1;       // slot 0 is the intercept
-    p->cap = std::min(cap, hard);
-    if (p->cap < 2) p->cap = 2;
+    p->cap = cached_cap(p);
 
     // persistent grid: blocks per SM limited by memory for slabs
     p->slab_stride = slab_bytes(p->cap, p->nmax, p->kc, p->tc);
@@ -644,7 +650,38 @@ extern "C" void pareben_release_cache(void)
 
 namespace {
 
-struct DumpBuffers { int *m = nullptr, *used = nullptr; double *beta = nullptr, *var = nullptr, *scalars = nullptr; };
+// Full-model records of a launch's fits (FitOutputs::m_out ..): fit o has m(o) effects, used(o)[i] / beta(o)[i] / var(o)[i]
+// for i < m(o), and scalars(o)[0..3].  The device buffer is one allocation of bytes(n, ld), doubles first, and comes back
+// into `host` with one copy.
+struct DumpBuffers {
+    int n = 0, ld = 0;                   // records, record stride (the basis cap of the launch)
+    std::vector<char> host;
+    static size_t bytes(size_t n, int ld) { return n * ((2 * (size_t)ld + 4) * sizeof(double) + (1 + (size_t)ld) * sizeof(int)); }
+    // point out's record arrays into a buffer of bytes(n, ld) bytes
+    static void carve(char *base, size_t n, int ld, FitOutputs &out)
+    {
+        out.beta_out = reinterpret_cast<double *>(base); out.var_out = out.beta_out + n * ld; out.scalars_out = out.var_out + n * ld;
+        out.m_out = reinterpret_cast<int *>(out.scalars_out + 4 * n); out.used_out = out.m_out + n; out.dump_ld = ld;
+    }
+    // size the host side for n records of stride ld (throws std::bad_alloc like any host allocation)
+    void resize(int n_, int ld_) { n = n_; ld = ld_; host.assign(bytes(n, ld), 0); }
+    FitOutputs view() { FitOutputs o; carve(host.data(), n, ld, o); return o; }
+    int m(int o) { return view().m_out[o]; }
+    const int *used(int o) { return view().used_out + (size_t)o * ld; }
+    const double *beta(int o) { return view().beta_out + (size_t)o * ld; }
+    const double *var(int o) { return view().var_out + (size_t)o * ld; }
+    const double *scalars(int o) { return view().scalars_out + 4 * (size_t)o; }
+    // record j of src into record i of this (same stride)
+    void copy_from(int i, DumpBuffers &src, int j)
+    {
+        FitOutputs d = view(), s = src.view();
+        d.m_out[i] = s.m_out[j];
+        memcpy(d.used_out + (size_t)i * ld, s.used_out + (size_t)j * ld, sizeof(int) * ld);
+        memcpy(d.beta_out + (size_t)i * ld, s.beta_out + (size_t)j * ld, sizeof(double) * ld);
+        memcpy(d.var_out + (size_t)i * ld, s.var_out + (size_t)j * ld, sizeof(double) * ld);
+        memcpy(d.scalars_out + 4 * (size_t)i, s.scalars_out + 4 * (size_t)j, sizeof(double) * 4);
+    }
+};
 
 // Streaming mode (stream.cuh): every fit keeps only its active set; all fits advance in lock-step rounds of
 //   stream_advance_kernel (one block per fit)  ->  stream_scan_kernel (one dense contraction per fold for all waiting fits)
@@ -660,14 +697,20 @@ size_t stream_fit_bytes(const pareben_problem *p, int c)
     return ((dbl * 8 + ints * 4) + 255) & ~(size_t)255;
 }
 
-// basis cap of a streaming call whose largest response has fits_per_target fits: the reference's basisMax, bounded by
-// PAREBEN_BASIS_CAP and by what that many active sets may occupy.  It depends on the fits of one response, never on the
-// number of responses, so each response's fits end as they would in a single-response call.
+// the largest basis cap a streaming call can get: the reference's basisMax, bounded by PAREBEN_BASIS_CAP
+int stream_cap_bound(const pareben_problem *p)
+{
+    const int cap = reference_basis_max(p->min_ntr, p->k, p->kc, p->epis, p->prior);
+    const char *env_cap = getenv("PAREBEN_BASIS_CAP");
+    return std::max(2, std::min(cap, env_cap ? atoi(env_cap) : 1024));
+}
+
+// basis cap of a streaming call whose largest response has fits_per_target fits: stream_cap_bound, lowered to what that
+// many active sets may occupy.  It depends on the fits of one response, never on the number of responses, so each
+// response's fits end as they would in a single-response call.
 int stream_cap(const pareben_problem *p, long long fits_per_target, size_t free_b)
 {
-    int cap = reference_basis_max(p->min_ntr, p->k, p->kc, p->epis, p->prior);
-    const char *env_cap = getenv("PAREBEN_BASIS_CAP");
-    cap = std::max(2, std::min(cap, env_cap ? atoi(env_cap) : 1024));
+    int cap = stream_cap_bound(p);
     while (cap > 16 && stream_fit_bytes(p, cap) * (size_t)fits_per_target > free_b / 2) cap = cap * 3 / 4;
     return cap;
 }
@@ -747,13 +790,13 @@ int run_fits_streaming(pareben_problem *p, int n_fits, const int *target, const 
         FitOutputs out;
         out.fold_err = d_err; out.status = d_ints; out.n_selected = d_ints + n_fits; out.n_iter = d_ints + 2 * n_fits;
         out.m_out = nullptr; out.used_out = nullptr; out.beta_out = nullptr; out.var_out = nullptr; out.scalars_out = nullptr;
+        out.dump_ld = 0;
         out.flops = p->d_flops;
+        char *d_dump = nullptr;
         if (dump) {
-            dump->m = (int *)tmp_alloc(sizeof(int) * (1 + cap));
-            dump->used = dump->m + 1;
-            dump->beta = (double *)tmp_alloc(sizeof(double) * (2 * cap + 4));
-            dump->var = dump->beta + cap; dump->scalars = dump->var + cap;
-            out.m_out = dump->m; out.used_out = dump->used; out.beta_out = dump->beta; out.var_out = dump->var; out.scalars_out = dump->scalars;
+            dump->resize(n_fits, cap);
+            d_dump = (char *)tmp_alloc(DumpBuffers::bytes(n_fits, cap));
+            DumpBuffers::carve(d_dump, n_fits, cap, out);
         }
         Problem P;
         P.N = p->n; P.K = p->k; P.Kc = p->kc; P.n_folds = p->n_folds; P.epis = p->epis; P.prior = p->prior;
@@ -795,6 +838,7 @@ int run_fits_streaming(pareben_problem *p, int n_fits, const int *target, const 
         CU(cudaMemcpyAsync(h_ints.data(), d_ints, sizeof(int) * 3 * n_fits, cudaMemcpyDeviceToHost, p->stream));
         double h_flops = 0;
         CU(cudaMemcpyAsync(&h_flops, p->d_flops, sizeof(double), cudaMemcpyDeviceToHost, p->stream));
+        if (dump) CU(cudaMemcpyAsync(dump->host.data(), d_dump, dump->host.size(), cudaMemcpyDeviceToHost, p->stream));
         CU(cudaStreamSynchronize(p->stream));
         float ms = 0;
         CU(cudaEventElapsedTime(&ms, p->ev0, p->ev1));
@@ -806,13 +850,6 @@ int run_fits_streaming(pareben_problem *p, int n_fits, const int *target, const 
             if (n_selected) n_selected[i] = h_ints[n_fits + i];
             if (n_iter) n_iter[i] = h_ints[2 * (size_t)n_fits + i];
         }
-        if (dump) {
-            int *hm = (int *)malloc(sizeof(int) * (1 + cap));
-            double *hb = (double *)malloc(sizeof(double) * (2 * cap + 4));
-            CU(cudaMemcpy(hm, dump->m, sizeof(int) * (1 + cap), cudaMemcpyDeviceToHost));
-            CU(cudaMemcpy(hb, dump->beta, sizeof(double) * (2 * cap + 4), cudaMemcpyDeviceToHost));
-            dump->m = hm; dump->used = hm + 1; dump->beta = hb; dump->var = hb + cap; dump->scalars = hb + 2 * cap;
-        }
         cudaEventDestroy(es0); cudaEventDestroy(es1);
         for (auto &q : scratch) pool_give(p->device, q.first, q.second);
     } catch (std::pair<int, std::string> &e) {
@@ -820,6 +857,11 @@ int run_fits_streaming(pareben_problem *p, int n_fits, const int *target, const 
         if (es1) cudaEventDestroy(es1);
         for (auto &q : scratch) pool_give(p->device, q.first, q.second);
         return fail(e.first, e.second);
+    } catch (std::bad_alloc &) {
+        if (es0) cudaEventDestroy(es0);
+        if (es1) cudaEventDestroy(es1);
+        for (auto &q : scratch) pool_give(p->device, q.first, q.second);
+        return fail(PAREBEN_ENOMEM, "host allocation of the fit records failed");
     }
     return PAREBEN_OK;
 }
@@ -840,6 +882,10 @@ int run_fits_streaming_waves(pareben_problem *p, int n_fits, const int *target, 
     const long long budget = std::max<long long>(1, (long long)(free_b / 2 / stream_fit_bytes(p, cap)));
     if (n_fits <= budget)
         return run_fits_streaming(p, n_fits, target, fold, alpha, lambda, fold_err, status, n_selected, n_iter, dump, cap);
+    if (dump) {
+        try { dump->resize(n_fits, cap); } catch (std::bad_alloc &) { return fail(PAREBEN_ENOMEM, "host allocation of the fit records failed"); }
+    }
+    DumpBuffers wave_dump;                 // each wave's records, moved into `dump` at the wave's fit numbers
     double ms = 0, flops = 0, scan_ms = 0, scan_flops = 0;
     int launches = 0, scans = 0, rounds = 0;
     for (int t0 = 0; t0 < p->n_targets;) {
@@ -855,9 +901,10 @@ int run_fits_streaming_waves(pareben_problem *p, int n_fits, const int *target, 
         std::vector<double> a(m), l(m), err(m);
         for (int j = 0; j < m; j++) { tg[j] = target[idx[j]]; fd[j] = fold[idx[j]]; a[j] = alpha[idx[j]]; l[j] = lambda[idx[j]]; }
         const int rc = run_fits_streaming(p, m, tg.data(), fd.data(), a.data(), l.data(), err.data(), st.data(), ns.data(), it.data(),
-                                          nullptr, cap);
+                                          dump ? &wave_dump : nullptr, cap);
         if (rc != PAREBEN_OK) return rc;
         for (int j = 0; j < m; j++) {
+            if (dump) dump->copy_from(idx[j], wave_dump, j);
             if (fold_err) fold_err[idx[j]] = err[j];
             if (status) status[idx[j]] = st[j];
             if (n_selected) n_selected[idx[j]] = ns[j];
@@ -934,13 +981,13 @@ int run_fits_impl(pareben_problem *p, int n_fits, const int *target, const int *
         FitOutputs out;
         out.fold_err = d_err; out.status = d_ints; out.n_selected = d_ints + n_fits; out.n_iter = d_ints + 2 * n_fits;
         out.m_out = nullptr; out.used_out = nullptr; out.beta_out = nullptr; out.var_out = nullptr; out.scalars_out = nullptr;
+        out.dump_ld = 0;
         out.flops = p->d_flops;
+        char *d_dump = nullptr;
         if (dump) {
-            dump->m = (int *)tmp_alloc(sizeof(int) * (1 + p->cap));
-            dump->used = dump->m + 1;
-            dump->beta = (double *)tmp_alloc(sizeof(double) * (2 * p->cap + 4));
-            dump->var = dump->beta + p->cap; dump->scalars = dump->var + p->cap;
-            out.m_out = dump->m; out.used_out = dump->used; out.beta_out = dump->beta; out.var_out = dump->var; out.scalars_out = dump->scalars;
+            dump->resize(n_fits, p->cap);
+            d_dump = (char *)tmp_alloc(DumpBuffers::bytes(n_fits, p->cap));
+            DumpBuffers::carve(d_dump, n_fits, p->cap, out);
         }
         Problem P;
         P.N = p->n; P.K = p->k; P.Kc = p->kc; P.n_folds = p->n_folds; P.epis = p->epis; P.prior = p->prior;
@@ -966,6 +1013,7 @@ int run_fits_impl(pareben_problem *p, int n_fits, const int *target, const int *
         CU(cudaMemcpyAsync(h_ints.data(), d_ints, sizeof(int) * 3 * n_fits, cudaMemcpyDeviceToHost, p->stream));
         double h_flops2[3] = {0, 0, 0};
         CU(cudaMemcpyAsync(h_flops2, p->d_flops, 3 * sizeof(double), cudaMemcpyDeviceToHost, p->stream));
+        if (dump) CU(cudaMemcpyAsync(dump->host.data(), d_dump, dump->host.size(), cudaMemcpyDeviceToHost, p->stream));
         CU(cudaStreamSynchronize(p->stream));
         const double h_flops = h_flops2[0];
         p->last_avoided = h_flops2[1];
@@ -979,17 +1027,13 @@ int run_fits_impl(pareben_problem *p, int n_fits, const int *target, const int *
             if (n_selected) n_selected[i] = h_ints[n_fits + i];
             if (n_iter) n_iter[i] = h_ints[2 * (size_t)n_fits + i];
         }
-        if (dump) {   // copy the dump to host-side mirrors allocated by the caller (reuse pointers)
-            int *hm = (int *)malloc(sizeof(int) * (1 + p->cap));
-            double *hb = (double *)malloc(sizeof(double) * (2 * p->cap + 4));
-            CU(cudaMemcpy(hm, dump->m, sizeof(int) * (1 + p->cap), cudaMemcpyDeviceToHost));
-            CU(cudaMemcpy(hb, dump->beta, sizeof(double) * (2 * p->cap + 4), cudaMemcpyDeviceToHost));
-            dump->m = hm; dump->used = hm + 1; dump->beta = hb; dump->var = hb + p->cap; dump->scalars = hb + 2 * p->cap;
-        }
         for (int i = 0; i < ns; i++) pool_give(p->device, scratch[i], scratch_bytes[i]);
     } catch (std::pair<int, std::string> &e) {
         for (int i = 0; i < ns; i++) pool_give(p->device, scratch[i], scratch_bytes[i]);
         return fail(e.first, e.second);
+    } catch (std::bad_alloc &) {
+        for (int i = 0; i < ns; i++) pool_give(p->device, scratch[i], scratch_bytes[i]);
+        return fail(PAREBEN_ENOMEM, "host allocation of the fit records failed");
     }
     return PAREBEN_OK;
 }
@@ -1119,19 +1163,75 @@ extern "C" int pareben_cv_grid(const double *basis, int n, int k, const double *
                                  shard, n_shards, fold_err, status, n_selected);
 }
 
+namespace {
+
+// Bound on the effects of one fit's record: the cached kernels' basis cap (the one in use once the slabs exist), or the
+// largest cap a streaming call can get; the binomial intercept slot is not an effect.
+int max_effects_of(const pareben_problem *p)
+{
+    if (p->streaming) return stream_cap_bound(p);
+    const int cap = p->d_slabs ? p->cap : cached_cap(p);
+    return p->prior == PAREBEN_BINOMIAL ? cap - 1 : cap;
+}
+
+}  // namespace
+
+extern "C" int pareben_max_effects(pareben_problem *p, int *max_effects)
+{
+    if (!p || !max_effects) return fail(PAREBEN_EINVAL, "pareben_max_effects: bad argument");
+    *max_effects = max_effects_of(p);
+    return PAREBEN_OK;
+}
+
+extern "C" int pareben_fit_batch(pareben_problem *p, int n_fits, const int *target, const int *fold, const double *alpha,
+                                 const double *lambda, int max_effects, int *n_effects, int *cand, double *beta, double *var,
+                                 double *scalars, int *status, double *fold_err)
+{
+    if (!p || n_fits < 0 || (n_fits > 0 && (!target || !fold || !alpha || !lambda)))
+        return fail(PAREBEN_EINVAL, "pareben_fit_batch: bad argument");
+    if (n_fits == 0) return PAREBEN_OK;
+    if (max_effects < max_effects_of(p))
+        return fail(PAREBEN_EINVAL, "pareben_fit_batch: max_effects is below pareben_max_effects (" + std::to_string(max_effects_of(p)) + ")");
+    if (max_effects > 0 && (!n_effects || !cand || !beta)) return fail(PAREBEN_EINVAL, "pareben_fit_batch: n_effects, cand and beta are required");
+    DumpBuffers dump;
+    std::vector<int> st;
+    std::vector<double> err;
+    try { st.resize(n_fits); err.resize(n_fits); } catch (std::bad_alloc &) { return fail(PAREBEN_ENOMEM, "pareben_fit_batch: host allocation failed"); }
+    const int rc = run_fits_impl(p, n_fits, target, fold, alpha, lambda, err.data(), st.data(), nullptr, nullptr, &dump);
+    if (rc != PAREBEN_OK) return rc;
+    for (int i = 0; i < n_fits; i++)
+        if (dump.m(i) < 0 || dump.m(i) > max_effects) return fail(PAREBEN_ECUDA, "pareben_fit_batch: a record has more effects than its stride");
+    const size_t me = (size_t)max_effects;
+    for (int i = 0; i < n_fits; i++) {
+        const int M = dump.m(i);
+        if (n_effects) n_effects[i] = M;
+        if (cand) { std::copy(dump.used(i), dump.used(i) + M, cand + i * me); std::fill(cand + i * me + M, cand + (i + 1) * me, 0); }
+        if (beta) { std::copy(dump.beta(i), dump.beta(i) + M, beta + i * me); std::fill(beta + i * me + M, beta + (i + 1) * me, 0.0); }
+        if (var) { std::copy(dump.var(i), dump.var(i) + M, var + i * me); std::fill(var + i * me + M, var + (i + 1) * me, 0.0); }
+        if (scalars) std::copy(dump.scalars(i), dump.scalars(i) + 4, scalars + 4 * (size_t)i);
+        if (status) status[i] = st[i];
+        if (fold_err) fold_err[i] = fold[i] == 0 ? 0.0 : err[i];      // an all-rows fit has no held-out rows to score
+    }
+    return PAREBEN_OK;
+}
+
+// The one-fit case of pareben_fit_batch, expanded into the reference's table layouts.
 extern "C" int pareben_fit(pareben_problem *p, double alpha, double lambda, double *beta_table, double *wald,
                            double *intercept, double *extra, int *status)
 {
     if (!p || !beta_table) return fail(PAREBEN_EINVAL, "pareben_fit: bad argument");
     if (p->n_folds != 0) return fail(PAREBEN_EINVAL, "pareben_fit needs a problem created with n_folds == 0");
     if (p->n_targets != 1) return fail(PAREBEN_EINVAL, "pareben_fit needs a problem with one response");
-    DumpBuffers dump;
-    int fold = 0, st = 0;
-    double err = 0;
-    int rc = run_fits_impl(p, 1, nullptr, &fold, &alpha, &lambda, &err, &st, nullptr, nullptr, &dump);
+    int me = 0;
+    pareben_max_effects(p, &me);
+    std::vector<int> used(me);           // one record: candidate ids in Used order, mu/scale, sigma_ii/scale^2
+    std::vector<double> beta(me), var(me);
+    double sc[4] = {0, 0, 0, 0};
+    const int target = 0, fold = 0;
+    int M = 0, st = 0;
+    const int rc = pareben_fit_batch(p, 1, &target, &fold, &alpha, &lambda, me, &M, used.data(), beta.data(), var.data(), sc, &st, nullptr);
     if (rc != PAREBEN_OK) return rc;
     const int k = p->k, kc = p->kc;
-    const int M = dump.m[0];
     if (p->prior == PAREBEN_GAUSSIAN) {
         const int ncol = p->epis ? 5 : 4;
         // loci columns (MainEff.c:87-91, NeFull2.c:100-134)
@@ -1139,33 +1239,32 @@ extern "C" int pareben_fit(pareben_problem *p, double alpha, double lambda, doub
         if (p->epis) { size_t kk = k; for (int i = 0; i < k - 1; i++) for (int j = i + 1; j < k; j++, kk++) { beta_table[kk] = i + 1; beta_table[(size_t)kc + kk] = j + 1; } }
         for (size_t z = (size_t)2 * kc; z < (size_t)ncol * kc; z++) beta_table[z] = 0;
         for (int i = 0; i < M; i++) {
-            const int c = dump.used[i] - 1;
-            beta_table[(size_t)2 * kc + c] = dump.beta[i];
-            beta_table[(size_t)3 * kc + c] = dump.var[i];
-            if (p->epis) beta_table[(size_t)4 * kc + c] = dump.used[i];
+            const int c = used[i] - 1;
+            beta_table[(size_t)2 * kc + c] = beta[i];
+            beta_table[(size_t)3 * kc + c] = var[i];
+            if (p->epis) beta_table[(size_t)4 * kc + c] = used[i];
         }
-        if (intercept) intercept[0] = dump.scalars[1];
+        if (intercept) intercept[0] = sc[1];
     } else {
         if (!p->epis) {      // k x 4 indexed by column id (NEmainEff.c:270-291, 364-371)
             for (int c = 0; c < k; c++) { beta_table[c] = c + 1; beta_table[(size_t)k + c] = c + 1; beta_table[(size_t)2 * k + c] = 0; beta_table[(size_t)3 * k + c] = 0; }
-            for (int i = 0; i < M; i++) { const int c = dump.used[i] - 1; beta_table[(size_t)2 * k + c] = dump.beta[i]; beta_table[(size_t)3 * k + c] = dump.var[i]; }
+            for (int i = 0; i < M; i++) { const int c = used[i] - 1; beta_table[(size_t)2 * k + c] = beta[i]; beta_table[(size_t)3 * k + c] = var[i]; }
         } else {             // compact 2k x 4 in Used order with decoded loci (NeFull.c:168-208)
             const int rows = 2 * k;
             for (size_t z = 0; z < (size_t)4 * rows; z++) beta_table[z] = 0;
             for (int i = 0; i < M && i < rows; i++) {
-                const int c = dump.used[i] - 1;
+                const int c = used[i] - 1;
                 int li = c, lj = c;
                 if (c >= k) { long long pp = (long long)c - k; int ii = 0; while ((long long)(ii + 1) * (2LL * k - (ii + 1) - 1) / 2 <= pp) ii++; li = ii; lj = (int)(pp - (long long)ii * (2LL * k - ii - 1) / 2) + ii + 1; }
                 beta_table[i] = li + 1; beta_table[(size_t)rows + i] = lj + 1;
-                beta_table[(size_t)2 * rows + i] = dump.beta[i]; beta_table[(size_t)3 * rows + i] = dump.var[i];
+                beta_table[(size_t)2 * rows + i] = beta[i]; beta_table[(size_t)3 * rows + i] = var[i];
             }
         }
-        if (intercept) { intercept[0] = dump.scalars[1]; intercept[1] = dump.scalars[2]; }
+        if (intercept) { intercept[0] = sc[1]; intercept[1] = sc[2]; }
     }
-    if (wald) wald[0] = dump.scalars[0];
-    if (extra) extra[0] = dump.scalars[3];
+    if (wald) wald[0] = sc[0];
+    if (extra) extra[0] = sc[3];
     if (status) status[0] = st;
-    free(dump.m); free(dump.beta);
     return PAREBEN_OK;
 }
 
