@@ -205,8 +205,9 @@ int pareben_last_counters(pareben_problem *p, double *flops, double *kernel_ms, 
  * the library builds it once per fold for every candidate (8 Kc^2 bytes per fold, when that fits in half of the free
  * device memory and the call has enough fits to amortise 2 N Kc^2 flops per fold; PAREBEN_GRAM=0 / 1 overrides the work
  * test) and all fits of the fold share it.  in_use: 1 when the problem runs that way; avoided_flops: the part of
- * pareben_last_counters' model flops that the last call did not have to execute; build_ms: time the last call spent
- * building the matrices (0 once they exist; it is included in that call's kernel_ms). */
+ * pareben_last_counters' model flops that the last call did not have to execute (binomial main-effect fits also skip the
+ * FullStat at the top of an outer iteration when the state is a fixed point of the posterior mode; its flops count here);
+ * build_ms: time the last call spent building the matrices (0 once they exist; it is included in that call's kernel_ms). */
 int pareben_last_gram_info(pareben_problem *p, int *in_use, double *avoided_flops, double *build_ms);
 /* Score contraction of the binomial main-effect fits (FullStat, ElasticNetBinaryNEmainEff.c:1693-1735).  tensor_core: 1 when
  * the problem computes it on the int8 tensor cores (every design entry an integer with |x| <= 11, exact to FP64 rounding),

@@ -298,7 +298,8 @@ class Problem:
 
     def gram_info(self):
         """(in use, model flops the last run_fits did not execute, ms the last run_fits spent building the matrices):
-        the Gram organisation of the Gaussian cached kernels (include/pareben.h, pareben_last_gram_info)."""
+        the Gram organisation of the Gaussian cached kernels (include/pareben.h, pareben_last_gram_info).  Binomial
+        main-effect fits report the FullStats they skip at a fixed point of the posterior mode as not executed."""
         use = np.zeros(1, np.int32); av = np.zeros(1); ms = np.zeros(1)
         _check(load().pareben_last_gram_info(self._h, _i(use), _d(av), _d(ms)))
         return bool(use[0]), float(av[0]), float(ms[0])

@@ -28,6 +28,7 @@ struct BinomState {
     int status;
     double flops;
     double tc_calls;  // score contractions run on the int8 tensor cores
+    bool at_mode;     // the last FullStat's posterior mode stopped on the gradient test at a point it had evaluated itself
 };
 
 // z = sum_j phi_j[h] mu[j] and z2 = the same for row h2, j ascending: two rows per thread keep twice the loads of the
@@ -69,7 +70,9 @@ __device__ inline double predictor_and_error(const Slab &s, int N, int M, const 
     return block_sum(err, sc);
 }
 
-// Returns true when eta / yv in memory belong to the final mu (the last evaluation was an accepted one).
+// Returns true when eta / yv in memory belong to the final mu (the last evaluation was an accepted one).  Sets b.at_mode
+// when, in addition, the loop stopped on the gradient test after a positive definite inverse: mu is then a fixed point, and
+// another call from the same mu and alpha repeats the last Newton step's arithmetic bit for bit and stops at once.
 template <bool EPIS>
 __device__ inline bool post_mode(Slab &s, BinomState &b, int N, const double *t, const Scratch &sc)
 {   // fEBCatPostMode*: Newton steps with step halving (NEmainEff.c:1808-2010, NeFull.c:998-1152)
@@ -82,6 +85,7 @@ __device__ inline bool post_mode(Slab &s, BinomState &b, int N, const double *t,
     double reg = 0;
     for (int i = 1; i < M; i++) reg = reg + s.alpha[i - 1] * s.mu[i] * s.mu[i] / 2;
     double total = reg + derr;
+    bool converged = false, pd = true;
     for (int it = 0; it < 25; it++) {
         const double err_log = total;
         double g0 = 0, h0 = 0;
@@ -122,7 +126,8 @@ __device__ inline bool post_mode(Slab &s, BinomState &b, int N, const double *t,
         else gram_mma(s.phi, N, LD, M, w, sc.sweep, put);
         for (int idx = threadIdx.x; idx < M * M; idx += T) s.sigma[idx] = s.H[idx];
         __syncthreads();
-        if (!spd_inverse_sweep(s.sigma, M, s.colk, sc, sc.sweep)) b.status |= ST_NOT_PD;
+        pd = spd_inverse_sweep(s.sigma, M, s.colk, sc, sc.sweep);
+        if (!pd) b.status |= ST_NOT_PD;
         int cnt = 0;
         for (int j = EPIS ? 0 : 1; j < M; j++) cnt += fabs(g[j]) < 1e-6;
         for (int k = threadIdx.x; k < M; k += T) {
@@ -131,7 +136,7 @@ __device__ inline bool post_mode(Slab &s, BinomState &b, int N, const double *t,
             dmu[k] = z;
         }
         __syncthreads();
-        if (cnt == (EPIS ? M : M - 1)) break;
+        if (cnt == (EPIS ? M : M - 1)) { converged = true; break; }
         double step = 1;
         while (step > 1.0 / 256) {
             for (int j = threadIdx.x; j < M; j += T) mun[j] = s.mu[j] + step * dmu[j];
@@ -151,6 +156,7 @@ __device__ inline bool post_mode(Slab &s, BinomState &b, int N, const double *t,
             __syncthreads();
         }
     }
+    b.at_mode = converged && current && pd;
     return current;                        // (IRLS work is not counted in the score-pass model)
 }
 
@@ -203,7 +209,7 @@ __device__ void binom_fit(const Problem &P, const FoldData &F, const Variant &v,
     const int N = F.ntr, K = P.K, Kc = P.Kc, cap = P.cap, T = blockDim.x, LD = phi_ld(N);   // cap counts the intercept slot
     const int lane_ = threadIdx.x & 31, wid_ = threadIdx.x >> 5, nw_ = T >> 5;
     const double *X = F.Xtr, *t = F.ytr, *scale = F.scale;
-    BinomState b; b.M = 2; b.n_unused = 0; b.status = 0; b.flops = 0; b.tc_calls = 0;
+    BinomState b; b.M = 2; b.n_unused = 0; b.status = 0; b.flops = 0; b.tc_calls = 0; b.at_mode = false;
     for (int j = threadIdx.x; j < cap + 1; j += T) { if (j < cap) s.grow[j] = j; s.alpha[j] = 0; s.mu[j] = 0; }
     __syncthreads();
     double vk = 1e-30, vk0, err = 1000, loglik = 0;
@@ -264,7 +270,19 @@ __device__ void binom_fit(const Problem &P, const FoldData &F, const Variant &v,
         __syncthreads();
         b.n_unused = block_compact(Kc, [&](int c) { return s.amap[c] < 0; }, s.unused, s.upos, 1, sc);
         const int initial = s.used[0];
-        binom_full_stat<EPIS, TC>(P, F, s, b, sV, sc);
+        // Every block of actions ends with a FullStat and nothing changes mu, alpha or PHI after it, so at iter > 1 the
+        // state is that of the last FullStat.  If its posterior mode stopped at a fixed point, FullStat would reproduce
+        // w, e, SIGMA, G, S_in and Q_in bit for bit: it is skipped (main effects; the Epis variant clamps the stored
+        // probabilities in place and recomputes them).  S_out/Q_out are refreshed as FullStat would (amap was rebuilt).
+        if (EPIS || iter <= 1 || !b.at_mode) binom_full_stat<EPIS, TC>(P, F, s, b, sV, sc);
+        else {
+            if (threadIdx.x == 0) {   // counted as binom_full_stat counts it, and reported as not executed (out.flops[1])
+                const double f = 2.0 * N * (double)Kc * (b.M + 2) + (double)Kc * (2.0 * b.M * b.M + b.M);
+                b.flops += f;
+                if (out.flops) atomicAdd(out.flops + 1, f);
+            }
+            refresh_out(s, b.M - 1, Kc);
+        }
         int selected = ACT_NONE, last = 0, n_update = 0, jj = -1, i_iter = 0;
         const int it_max = iter == 1 ? 10 : 100;
         loglik = 1e-30;

@@ -118,18 +118,65 @@ __device__ inline void tc_close(TcState &ts)
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(ts.tmem), "r"(TC_TMEM_COLS) : "memory");
 }
 
-// Digit planes of columns j0 .. j0 + ncols - 1 ([stage][column][16-row half][plane][16 rows]) and their scales.
-// val(j, h) is the FP64 value of column j at training row h.  A warp per column, a lane per four consecutive rows; the
-// digits are peeled off a 56-bit fixed-point integer (rounded once, every later step exact).
-template <class Val>
-__device__ inline void tc_digits(int j0, int ncols, int N, int nst, Val val, int8_t *__restrict__ planes, double *bscale)
+// Digit extraction stages a column in chunks of TC_DIG_ROWS training rows through shared memory (the ring is idle while
+// it runs): a lane issues the cp.async copies of its four consecutive rows of every 128-row group (TC_DIG_V values) at
+// once, so a chunk costs one trip to L2, and the column's maximum and its digits both read the staged copy.  Element k
+// of lane l sits at [32 k + l], so a warp's reads of one k are one contiguous 256-byte row.
+constexpr int TC_DIG_GROUPS = 4;
+constexpr int TC_DIG_V = 4 * TC_DIG_GROUPS;                   // values per lane and chunk
+constexpr int TC_DIG_ROWS = 128 * TC_DIG_GROUPS;              // rows per chunk
+constexpr int TC_DIG_WARPS = 8;                               // warps per block (FIT_T = 256 threads) the staging area serves
+static_assert((TC_DIG_WARPS + 1) * TC_DIG_ROWS * 8 <= TC_RING_BYTES, "the digit staging area must fit the ring");
+
+// 8-byte copy global -> shared, zero-filled when !valid (src is then not read)
+__device__ inline void cp_async8(double *dst, const double *src, bool valid)
+{
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 8, %2;" ::"r"(smem_u32(dst)), "l"(src), "r"(valid ? 8 : 0) : "memory");
+}
+__device__ inline void cp_async_wait_all() { asm volatile("cp.async.commit_group;\ncp.async.wait_group 0;" ::: "memory"); }
+
+// Digit planes of columns j0 .. j0 + ncols - 1 ([stage][column][16-row half][plane][16 rows]) and their scales.  Column
+// j < R is wv o col(j), column R is ev.  A warp per column, a lane per four consecutive rows of every 128-row group; the
+// digits are peeled off a 56-bit fixed-point integer (rounded once, every later step exact).  stage: shared memory for
+// TC_DIG_WARPS + 1 chunks.  When the rows fit one chunk (N <= 512), wv is staged once for the whole block and every
+// column is read once; longer columns take one pass over the chunks for the maximum and a second one for the digits
+// (which begins with the chunk still staged from the first), with wv read from global memory.
+template <class Col>
+__device__ inline void tc_digits(int j0, int ncols, int N, int nst, int R, Col col, const double *__restrict__ wv,
+                                 const double *__restrict__ ev, int8_t *__restrict__ planes, double *bscale, double *stage)
 {
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, nw = blockDim.x >> 5;
+    const int nrow = nst * TC_KS, nch = (nrow + TC_DIG_ROWS - 1) / TC_DIG_ROWS;
+    auto row = [&](int ch, int k) { return ch * TC_DIG_ROWS + 128 * (k >> 2) + 4 * lane + (k & 3); };
+    // this lane's rows of chunk ch of a -> d[32 k + lane], 0 past row N
+    auto stage_chunk = [&](double *d, const double *__restrict__ a, int ch) {
+#pragma unroll
+        for (int k = 0; k < TC_DIG_V; k++) { const int h = row(ch, k); cp_async8(d + 32 * k + lane, h < N ? a + h : a, h < N); }
+        cp_async_wait_all();
+    };
+    double *ws = stage, *cs = stage + (size_t)(1 + wid) * TC_DIG_ROWS;
+    if (nch == 1) {
+        if (wid == 0) stage_chunk(ws, wv, 0);
+        __syncthreads();
+    }
     for (int jl = wid; jl < ncols; jl += nw) {
         const int j = j0 + jl;
+        const bool prod = j < R;
+        const double *__restrict__ src = prod ? col(j) : ev;
+        auto val = [&](int ch, int k) -> double {              // the column's value at row(ch, k), staged
+            const double x = cs[32 * k + lane];
+            if (!prod) return x;
+            if (nch == 1) return ws[32 * k + lane] * x;
+            const int h = row(ch, k);
+            return h < N ? wv[h] * x : 0.0;
+        };
         double mx = 0.0;
         bool bad = false;
-        for (int h = lane; h < N; h += 32) { const double v = fabs(val(j, h)); if (!(v <= 1.7976931348623157e308)) bad = true; mx = fmax(mx, v); }
+        for (int ch = 0; ch < nch; ch++) {
+            stage_chunk(cs, src, ch);
+#pragma unroll
+            for (int k = 0; k < TC_DIG_V; k++) { const double a = fabs(val(ch, k)); if (!(a <= 1.7976931348623157e308)) bad = true; mx = fmax(mx, a); }
+        }
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, o));
         bad = __any_sync(0xffffffffu, bad);
@@ -142,30 +189,36 @@ __device__ inline void tc_digits(int j0, int ncols, int N, int nst, Val val, int
         // so both forms are one exact power-of-two scaling (rounded only on overflow) and agree bit for bit below 2^1022.
         if (lane == 0) bscale[jl] = bad ? __longlong_as_double(0x7ff8000000000000LL) : (live ? scalbn(1.0, ex - 1) : 0.0);
         int8_t *colp = planes + (size_t)jl * TC_COL_BYTES;
-        for (int p4 = 4 * lane; p4 < nst * TC_KS; p4 += 128) {
-            unsigned wout[TC_PLANES];
+        for (int ch = nch - 1; ch >= 0; ch--) {
+            if (ch < nch - 1) stage_chunk(cs, src, ch);
+#pragma unroll 1                                                // rolled: fewer spills in the fit kernel around it
+            for (int g = 0; g < TC_DIG_GROUPS; g++) {
+                const int p4 = row(ch, 4 * g);
+                if (p4 >= nrow) break;
+                unsigned wout[TC_PLANES];
 #pragma unroll
-            for (int s = 0; s < TC_PLANES; s++) wout[s] = 0u;
+                for (int s = 0; s < TC_PLANES; s++) wout[s] = 0u;
 #pragma unroll
-            for (int b = 0; b < 4; b++) {
-                const int h = p4 + b;
-                const long long q = (h < N && live) ? __double2ll_rn(val(j, h) * down) : 0LL;
-                // balanced base-128 digits, least significant first, in 32-bit arithmetic: the low 28 bits give four
-                // digits and a carry into the high part, which gives the other four
-                int lo = (int)(q & 0xfffffff), hi = (int)(q >> 28);
+                for (int b = 0; b < 4; b++) {
+                    // rows past N are staged as 0: their digits are 0
+                    const long long q = live ? __double2ll_rn(val(ch, 4 * g + b) * down) : 0LL;
+                    // balanced base-128 digits, least significant first, in 32-bit arithmetic: the low 28 bits give four
+                    // digits and a carry into the high part, which gives the other four
+                    int lo = (int)(q & 0xfffffff), hi = (int)(q >> 28);
 #pragma unroll
-                for (int s = TC_PLANES - 1; s >= 0; s--) {
-                    int &x = s >= 4 ? lo : hi;
-                    const int d = ((x + 64) & 127) - 64;        // in [-64, 63]
-                    x = (x - d) >> 7;                           // exact
-                    if (s == 4) hi += lo;                       // the carry (0 or 1)
-                    const int dig = s == 0 ? d + (x << 7) : d;  // the top digit takes what is left (|.| <= 64)
-                    wout[s] |= ((unsigned)dig & 0xffu) << (8 * b);
+                    for (int s = TC_PLANES - 1; s >= 0; s--) {
+                        int &x = s >= 4 ? lo : hi;
+                        const int d = ((x + 64) & 127) - 64;        // in [-64, 63]
+                        x = (x - d) >> 7;                           // exact
+                        if (s == 4) hi += lo;                       // the carry (0 or 1)
+                        const int dig = s == 0 ? d + (x << 7) : d;  // the top digit takes what is left (|.| <= 64)
+                        wout[s] |= ((unsigned)dig & 0xffu) << (8 * b);
+                    }
                 }
-            }
-            int8_t *dst = colp + (size_t)(p4 >> 5) * ncols * TC_COL_BYTES + ((p4 >> 4) & 1) * 128 + (p4 & 15);
+                int8_t *dst = colp + (size_t)(p4 >> 5) * ncols * TC_COL_BYTES + ((p4 >> 4) & 1) * 128 + (p4 & 15);
 #pragma unroll
-            for (int s = 0; s < TC_PLANES; s++) *reinterpret_cast<unsigned *>(dst + s * 16) = wout[s];
+                for (int s = 0; s < TC_PLANES; s++) *reinterpret_cast<unsigned *>(dst + s * 16) = wout[s];
+            }
         }
     }
 }
@@ -190,8 +243,9 @@ __device__ inline void tc_contract(const FoldData &F, int Kc, int R, Col col, De
         const bool first = j0 == 0;                             // the first pass also streams X o X for bb
         const int ncols = min(TC_COLS, ncol_all - j0), ncp = (ncols + 1) & ~1;
         __syncthreads();                                        // the previous pass's planes are fully consumed
-        tc_digits(j0, ncols, N, nst, [&](int j, int h) { return j < R ? wv[h] * col(j)[h] : ev[h]; }, planes, bscale);
+        tc_digits(j0, ncols, N, nst, R, col, wv, ev, planes, bscale, reinterpret_cast<double *>(ring));
         asm volatile("fence.proxy.async.global;" ::: "memory");     // the planes are read by the bulk copies
+        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // the digits were staged in the ring
         __syncthreads();
         // A slot holds ncp columns: with an odd column count the MMA (N = 8 ncp), and with one column the bb MMA (N = 16),
         // read one column's planes past the copied ones.  They stay inside the slot, and the accumulator columns they feed

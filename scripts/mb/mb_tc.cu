@@ -30,7 +30,7 @@ __global__ void __launch_bounds__(256, 2) mb_kernel(FoldData F, int Kc, int M, i
     long long t0 = clock64();
     for (int i = 0; i < reps; i++) {
         for (int j0 = 0; j0 < M + 1; j0 += TC_COLS)
-            tc_digits(j0, min(TC_COLS, M + 1 - j0), N, nst, [&](int j, int h) { return j < M ? w[h] * col(j)[h] : e[h]; }, planes, bscale);
+            tc_digits(j0, min(TC_COLS, M + 1 - j0), N, nst, M, col, w, e, planes, bscale, s_buf);
         __syncthreads();
     }
     long long t1 = clock64();
