@@ -4,7 +4,7 @@
 // Each entry takes host arrays, lays the training matrix out with the library's own layout kernels (layout.cuh) exactly
 // as pareben_problem_create does, runs ONE block with the fit kernels' resources (launch bounds, FIT_T threads, S_BUF_BYTES
 // of dynamic shared memory) on a private stream, copies the results back and frees every device buffer before it returns, on
-// success and on failure alike.  The tensor-core kernel allocates its tensor memory with tc_open and gives it back with
+// success and on failure alike (probe_call.cuh).  The tensor-core kernel allocates its tensor memory with tc_open and gives it back with
 // tc_close before it exits.
 //
 //   probe_tc          tc_contract (tc_contract.cuh): G[j][c] = x_c'(w o phi_j) / s_c for j < R, ze = X'e, bb = (X o X)'(w o phi_0)
@@ -18,64 +18,17 @@
 #include "../../pareben_b200/csrc/tc_contract.cuh"
 #include "../../pareben_b200/csrc/layout.cuh"
 #include "../../pareben_b200/csrc/fit_kernel.cuh"
+#include "probe_call.cuh"
 
 #include <cmath>
-#include <string>
 #include <vector>
 
 using namespace pareben;
 
 namespace {
 
-std::string g_err;
-
-// device buffers and the stream of one call, released in the destructor whatever path the call leaves by
-struct Call {
-    cudaStream_t stream = nullptr;
-    std::vector<void *> bufs;
-    cudaError_t err = cudaSuccess;
-    Call() { note(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking)); }
-    ~Call()
-    {
-        if (stream) cudaStreamSynchronize(stream);
-        for (void *p : bufs) cudaFree(p);
-        if (stream) cudaStreamDestroy(stream);
-    }
-    bool note(cudaError_t e)
-    {
-        if (e != cudaSuccess && err == cudaSuccess) { err = e; g_err = cudaGetErrorString(e); }
-        return err == cudaSuccess;
-    }
-    template <class T>
-    T *alloc(size_t n)
-    {
-        void *p = nullptr;
-        if (!note(cudaMalloc(&p, n * sizeof(T) + 16))) return nullptr;
-        bufs.push_back(p);
-        note(cudaMemsetAsync(p, 0, n * sizeof(T) + 16, stream));
-        return static_cast<T *>(p);
-    }
-    template <class T>
-    T *upload(const T *h, size_t n)
-    {
-        T *d = alloc<T>(n);
-        if (d && h && n) note(cudaMemcpyAsync(d, h, n * sizeof(T), cudaMemcpyHostToDevice, stream));
-        return d;
-    }
-    template <class T>
-    void download(T *h, const T *d, size_t n)
-    {
-        if (h && d && n && err == cudaSuccess) note(cudaMemcpyAsync(h, d, n * sizeof(T), cudaMemcpyDeviceToHost, stream));
-    }
-    int finish()
-    {
-        if (err == cudaSuccess) note(cudaGetLastError());
-        if (err == cudaSuccess) note(cudaStreamSynchronize(stream));
-        return (int)err;
-    }
-};
-
-int bad(const char *msg) { g_err = msg; return -1; }
+using probe::Call;
+using probe::bad;
 
 // the design as pareben_problem_create sees it: every entry an integer in [-127, 127], and the largest magnitude
 bool small_int_design(const double *X, size_t n, double &max_abs)
@@ -168,7 +121,7 @@ bool launch_setup(Call &cl, Kern kern)
 
 }  // namespace
 
-extern "C" const char *probe_last_error(void) { return g_err.c_str(); }
+extern "C" const char *probe_last_error(void) { return probe::last_error().c_str(); }
 
 // X: [N][K] row-major training rows (integers, |x| <= 11, N max|x|^2 64 < 2^31: the host predicate of the tensor-core
 // path).  phi: [R][N], column 0 all ones in a fit (bb reuses column 0's digit planes).  w, e: [N].

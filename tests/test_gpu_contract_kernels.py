@@ -1,8 +1,8 @@
 """GPU suite (-m gpu): the score contractions kernel by kernel, against exact references.
 
 A module fixture compiles tests/kernels/contract_probe.cu (the library's own headers, __graft_entry__.NVCC_FLAGS) into
-build/probe/ and loads it with ctypes.  The probe lays the design out with the library's layout kernels and runs one
-block of tc_contract or contract_x with the fit kernels' resources.
+build/probe/ and loads it with ctypes (kernel_probe.py).  The probe lays the design out with the library's layout
+kernels and runs one block of tc_contract or contract_x with the fit kernels' resources.
 
 * tc_contract (int8 tensor cores) must equal the numpy emulation of test_contract_reference.py bit for bit, and be
   within 2 N 2^-57 max|b| max|x| + |exact| 2^-51 of the exact value before the division by the column norm.
@@ -13,19 +13,16 @@ block of tc_contract or contract_x with the fit kernels' resources.
 Every assertion message names the kernel, the shape and the largest error/bound ratio.
 """
 import ctypes
-import os
-import subprocess
 
 import numpy as np
 import pytest
 
+import kernel_probe
 import test_contract_reference as ref
+from kernel_probe import bits_equal
 
 pytestmark = pytest.mark.gpu
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-PROBE_SRC = os.path.join(ROOT, "tests", "kernels", "contract_probe.cu")
-CSRC = os.path.join(ROOT, "pareben_b200", "csrc")
 U = 2.0 ** -53
 
 _d = ctypes.POINTER(ctypes.c_double)
@@ -34,19 +31,10 @@ _i = ctypes.POINTER(ctypes.c_int)
 
 @pytest.fixture(scope="module")
 def probe():
-    import shutil
-    import __graft_entry__ as ge
     import pareben_b200 as pb
     if pb.device_count() < 1:
         pytest.fail("no CUDA device: the -m gpu suite must run on the B200 box")
-    out_dir = os.path.join(ROOT, "build", "probe")
-    lib = os.path.join(out_dir, "libcontract_probe.so")
-    sources = [PROBE_SRC] + [os.path.join(CSRC, f) for f in os.listdir(CSRC)] + [os.path.join(ROOT, "__graft_entry__.py")]
-    if not ge._newer(lib, sources):
-        os.makedirs(out_dir, exist_ok=True)
-        nvcc = shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
-        subprocess.run([nvcc, *ge.NVCC_FLAGS, "--shared", "-o", lib, PROBE_SRC], check=True, cwd=out_dir)
-    L = ctypes.CDLL(lib)
+    L = kernel_probe.build_probe("contract_probe")
     L.probe_tc.argtypes = [ctypes.c_int, ctypes.c_int, _d, ctypes.c_int, _d, _d, _d, _d, _d, _d, _d]
     L.probe_contract_x.argtypes = [ctypes.c_int] * 5 + [_d, ctypes.c_int, _d, _d, _d, ctypes.c_int, _d, _d, _d, _d]
     L.probe_cand_map.argtypes = [ctypes.c_int, ctypes.c_int, _i, _i]
@@ -84,15 +72,6 @@ def run_cx(L, X, cols, epis=False, force_f64=False, n_aligned=None, w=None, e=No
                             _p(G), _p(bb), _p(ze), _p(sc))
     assert rc == 0, f"probe_contract_x: {rc} {L.probe_last_error().decode()}"
     return G, bb, ze, sc
-
-
-def bits_equal(a, b):
-    """Bitwise equal (so +0 and -0 differ); any NaN equals any NaN (payloads are not part of the result)."""
-    a = np.ascontiguousarray(a, np.float64); b = np.ascontiguousarray(b, np.float64)
-    if a.shape != b.shape:
-        return False
-    nan = np.isnan(a)
-    return np.array_equal(nan, np.isnan(b)) and np.array_equal(a[~nan].view(np.int64), b[~nan].view(np.int64))
 
 
 # ---------------------------------------------------------------------------------------------------------------------

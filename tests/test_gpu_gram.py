@@ -4,8 +4,9 @@ The candidate-cache row of a basis depends on the fold alone, so the library bui
 fold (fold_gram_kernel) and all fits of the fold share them; PAREBEN_GRAM=0 keeps the reference's organisation (one cache
 per fit, recomputed by every add and at the top of every outer iteration).  Both must give the same tables -- the same
 sums in a different summation order -- and both are checked against the oracle by the other GPU tests (which run with
-whichever organisation the work test picks).  Also here: the in-place SPD inverse at the sizes its three code paths
-take, against numpy, through a fit whose result depends on it.
+whichever organisation the work test picks).  The main-effect test reaches active sets of about 230, so its fits run
+the register and 8-wide panel paths of the SPD inverse and both forms of the quadratic forms; those kernels are tested
+on their own, at every path boundary, in test_gpu_linalg_kernels.py.
 """
 import os
 
@@ -49,8 +50,8 @@ def _both(pb, X, y, folds, n_folds, epis, fold, a, l):
 
 
 def test_gram_matches_per_fit_cache_main_effects(pb, bundled):
-    """Bundled 1000 x 481 Gaussian design, 10 folds, every 9th fit of the 4,000 (active sets up to ~230: all three
-    SPD-inverse paths, SIMT and tensor-core quadratic forms)."""
+    """Bundled 1000 x 481 Gaussian design, 10 folds, every 9th fit of the 4,000 (active sets up to ~230: the register
+    and 8-wide panel paths of the SPD inverse, SIMT and tensor-core quadratic forms)."""
     X, y, nf = bundled["BASIS"].astype(np.float64), bundled["y"], 10
     folds = pb.AssignToFolds(X, nf)
     grid = pb.BuildGrid(X, y, nf)
