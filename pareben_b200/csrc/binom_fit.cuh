@@ -76,33 +76,39 @@ __device__ inline double predictor_and_error(const Slab &s, int N, int M, const 
 template <bool EPIS>
 __device__ inline bool post_mode(Slab &s, BinomState &b, int N, const double *t, const Scratch &sc)
 {   // fEBCatPostMode*: Newton steps with step halving (NEmainEff.c:1808-2010, NeFull.c:998-1152)
-    PHASE(PH_IRLS_OTHER);      // includes the nested Gram/sweep phases (subtract them when reading the counters)
+    PHASE(PH_IRLS_OTHER);      // includes the nested IRLS phases (subtract them when reading the counters)
     const int M = b.M, T = blockDim.x, LD = phi_ld(N);
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, nw = T >> 5;
     double *yv = s.t, *e = s.e, *w = s.w1, *eta = s.w2, *g = s.gamma, *dmu = s.u, *mun = s.tmp;
-    double derr = predictor_and_error(s, N, M, s.mu, t, eta, yv, sc);
+    double derr, reg = 0;
+    {
+        PHASE(PH_IRLS_PRED);
+        derr = predictor_and_error(s, N, M, s.mu, t, eta, yv, sc);
+        for (int i = 1; i < M; i++) reg = reg + s.alpha[i - 1] * s.mu[i] * s.mu[i] / 2;
+    }
     bool current = true;
-    double reg = 0;
-    for (int i = 1; i < M; i++) reg = reg + s.alpha[i - 1] * s.mu[i] * s.mu[i] / 2;
     double total = reg + derr;
     bool converged = false, pd = true;
     for (int it = 0; it < 25; it++) {
         const double err_log = total;
         double g0 = 0, h0 = 0;
-        for (int h = threadIdx.x; h < N; h += T) {
-            double y = yv[h];
-            if (EPIS) { if (y < 1e-5) y = 1e-5; if (y > (1 - 1e-5)) y = 1 - 1e-5; yv[h] = y; }     // NeFull.c:1049-1050
-            const double eh = t[h] - y;
-            e[h] = eh; g0 += eh;
-            double bw = y * (1 - y);
-            if (!EPIS) { if (bw < 1e-10) bw = 1e-5; if (bw > 1e10) bw = 1e5; }                      // NEmainEff.c:1880-1882
-            else { if (bw < 1e-5) bw = 1e-3; if (bw > 1e5) bw = 1e3; }                              // NeFull.c:1054-1055
-            w[h] = bw; h0 += bw;
+        {
+            PHASE(PH_IRLS_DIR);
+            for (int h = threadIdx.x; h < N; h += T) {
+                double y = yv[h];
+                if (EPIS) { if (y < 1e-5) y = 1e-5; if (y > (1 - 1e-5)) y = 1 - 1e-5; yv[h] = y; }     // NeFull.c:1049-1050
+                const double eh = t[h] - y;
+                e[h] = eh; g0 += eh;
+                double bw = y * (1 - y);
+                if (!EPIS) { if (bw < 1e-10) bw = 1e-5; if (bw > 1e10) bw = 1e5; }                      // NEmainEff.c:1880-1882
+                else { if (bw < 1e-5) bw = 1e-3; if (bw > 1e5) bw = 1e3; }                              // NeFull.c:1054-1055
+                w[h] = bw; h0 += bw;
+            }
+            block_sum2(g0, h0, sc);
+            if (threadIdx.x == 0) g[0] = g0;
+            (void)h0;
+            __syncthreads();
         }
-        block_sum2(g0, h0, sc);
-        if (threadIdx.x == 0) g[0] = g0;
-        (void)h0;
-        __syncthreads();
         // gradient g_j = phi_j'e - alpha_j mu_j (one warp per column), then the Hessian PHI'B PHI + diag(0, alpha)
         // as a tiled Gram matrix; column 0 of PHI is the intercept's all-ones column, so H(0, k) = sum w phi_k
         // and H(0, 0) = sum w come out of the same pass (:1887-1919).
@@ -124,20 +130,27 @@ __device__ inline bool post_mode(Slab &s, BinomState &b, int N, const double *t,
         };
         if (fused) gram_pipe(s.phit, N, M, w, sc.sweep, put, e, [&](int j, double z) { if (j >= 1) g[j] = z - s.alpha[j - 1] * s.mu[j]; });   // row-major copy, pipelined
         else gram_mma(s.phi, N, LD, M, w, sc.sweep, put);
-        for (int idx = threadIdx.x; idx < M * M; idx += T) s.sigma[idx] = s.H[idx];
-        __syncthreads();
+        {
+            PHASE(PH_IRLS_COPY);
+            for (int idx = threadIdx.x; idx < M * M; idx += T) s.sigma[idx] = s.H[idx];
+            __syncthreads();
+        }
         pd = spd_inverse_sweep(s.sigma, M, s.colk, sc, sc.sweep);
         if (!pd) b.status |= ST_NOT_PD;
         int cnt = 0;
-        for (int j = EPIS ? 0 : 1; j < M; j++) cnt += fabs(g[j]) < 1e-6;
-        for (int k = threadIdx.x; k < M; k += T) {
-            double z = 0;
-            for (int L = 0; L < M; L++) z = fma(s.sigma[L * M + k], g[L], z);
-            dmu[k] = z;
+        {
+            PHASE(PH_IRLS_DIR);
+            for (int j = EPIS ? 0 : 1; j < M; j++) cnt += fabs(g[j]) < 1e-6;
+            for (int k = threadIdx.x; k < M; k += T) {
+                double z = 0;
+                for (int L = 0; L < M; L++) z = fma(s.sigma[L * M + k], g[L], z);
+                dmu[k] = z;
+            }
+            __syncthreads();
         }
-        __syncthreads();
         if (cnt == (EPIS ? M : M - 1)) { converged = true; break; }
         double step = 1;
+        PHASE(PH_IRLS_PRED);
         while (step > 1.0 / 256) {
             for (int j = threadIdx.x; j < M; j += T) mun[j] = s.mu[j] + step * dmu[j];
             __syncthreads();

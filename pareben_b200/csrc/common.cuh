@@ -155,7 +155,10 @@ __device__ inline Slab carve_slab(char *base, int cap, int nmax, int Kc, int tc)
 
 // ------------------------------------------------------------------------------------------
 // Optional per-phase cycle accounting (compile with -DPAREBEN_PHASE_TIMING; experiments only).
-enum : int { PH_VFILL = 0, PH_CONTRACT, PH_QUAD, PH_GRAM, PH_SWEEP, PH_IRLS_OTHER, PH_DELTA_ML, PH_ACTIONS, PH_LOGLIK, PH_OTHER, PH_COUNT };
+// PH_IRLS_OTHER contains the nested IRLS phases (PH_GRAM, PH_SWEEP, PH_IRLS_PRED, PH_IRLS_DIR, PH_IRLS_COPY) and
+// PH_SWEEP contains PH_SWEEP_LS (the register sweep's loads and stores); subtract them when reading the counters.
+enum : int { PH_VFILL = 0, PH_CONTRACT, PH_QUAD, PH_GRAM, PH_SWEEP, PH_IRLS_OTHER, PH_DELTA_ML, PH_ACTIONS, PH_LOGLIK, PH_OTHER,
+             PH_IRLS_PRED, PH_IRLS_DIR, PH_IRLS_COPY, PH_SWEEP_LS, PH_COUNT };
 #ifdef PAREBEN_PHASE_TIMING
 static __device__ unsigned long long g_phase_cycles[PH_COUNT];
 static __device__ unsigned long long g_phase_calls[PH_COUNT];

@@ -975,13 +975,16 @@ __device__ inline bool sweep_regs(double *a, int M, double *colbuf /* 128 double
 {
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     double r[NI][8];
+    {
+        PHASE(PH_SWEEP_LS);
 #pragma unroll
-    for (int ii = 0; ii < NI; ii++)
+        for (int ii = 0; ii < NI; ii++)
 #pragma unroll
-        for (int jj = 0; jj < 8; jj++) {
-            const int i = lane + 32 * ii, j = wid + 8 * jj;
-            r[ii][jj] = (i < M && j < M) ? a[(size_t)j * M + i] : 0.0;
-        }
+            for (int jj = 0; jj < 8; jj++) {
+                const int i = lane + 32 * ii, j = wid + 8 * jj;
+                r[ii][jj] = (i < M && j < M) ? a[(size_t)j * M + i] : 0.0;
+            }
+    }
     double *cur = colbuf, *nxt = colbuf + 64;
     __syncthreads();
     if (wid == 0) {                                   // column 0 lives in warp 0 (jj = 0)
@@ -1001,17 +1004,24 @@ __device__ inline bool sweep_regs(double *a, int M, double *colbuf /* 128 double
             const int j = wid + 8 * jj;
             if (j < M) {                                  // warp-uniform: whole columns beyond M are skipped
                 const double cj = cur[j];
+                if (j == k) {                             // the pivot column (warp-uniform branch)
 #pragma unroll
-                for (int ii = 0; ii < NI; ii++) {
-                    const int i = lane + 32 * ii;
-                    const double ci = ii == 0 ? ci0 : ci1;
-                    double v;
-                    if (i == k && j == k) v = ndinv;
-                    else if (i == k) v = cj * dinv;
-                    else if (j == k) v = ci * dinv;
-                    else v = fma(ci * cj, ndinv, r[ii][jj]);      // (ci*cj) is symmetric in (i, j): the result stays exactly symmetric
-                    r[ii][jj] = v;
-                    if (j == kn) nxt[i] = v;
+                    for (int ii = 0; ii < NI; ii++) {
+                        const double ci = ii == 0 ? ci0 : ci1;
+                        r[ii][jj] = lane + 32 * ii == k ? ndinv : ci * dinv;
+                    }
+                } else {                                  // the pivot row's entry, else the rank-1 update
+                    const double cjd = cj * dinv;
+#pragma unroll
+                    for (int ii = 0; ii < NI; ii++) {
+                        const double ci = ii == 0 ? ci0 : ci1;
+                        const double u = fma(ci * cj, ndinv, r[ii][jj]);  // (ci*cj) is symmetric in (i, j): the result stays exactly symmetric
+                        r[ii][jj] = lane + 32 * ii == k ? cjd : u;
+                    }
+                }
+                if (j == kn) {                            // publish the next pivot's column
+                    nxt[lane] = r[0][jj];
+                    if (NI > 1) nxt[lane + 32] = r[NI - 1][jj];
                 }
             }
         }
@@ -1019,6 +1029,7 @@ __device__ inline bool sweep_regs(double *a, int M, double *colbuf /* 128 double
         double *t = cur; cur = nxt; nxt = t;
     }
     if (ok) {
+        PHASE(PH_SWEEP_LS);
 #pragma unroll
         for (int ii = 0; ii < NI; ii++)
 #pragma unroll
@@ -1184,10 +1195,12 @@ __device__ inline void gram_pipe(const double *__restrict__ phit, int N, int M, 
                 const int hl = idx / cpr, q = idx - hl * cpr;
                 __pipeline_memcpy_async(dst + hl * NC + 2 * q, phit + (size_t)min(h0 + hl, N - 1) * PHIT_LD + 2 * q, 16);
             }
-            if (threadIdx.x < TR) {
-                const int h = h0 + (int)threadIdx.x;
-                wt[(t & 1) * 2 * GP_ROWS + threadIdx.x] = h < N ? (w ? w[h] : 1.0) : 0.0;
-                if (ev) et[(t & 1) * 2 * GP_ROWS + threadIdx.x] = h < N ? ev[h] : 0.0;
+            if (threadIdx.x < TR) {                              // w and ev ride in the same cp.async group (zero past N):
+                const int h = h0 + (int)threadIdx.x;              // a plain load here would stall these warps for an L2 round
+                double *wd = wt + (t & 1) * 2 * GP_ROWS + threadIdx.x;    // trip per tile, and the next barrier waits for them
+                if (w) __pipeline_memcpy_async(wd, w + min(h, N - 1), 8, h < N ? 0 : 8);
+                else *wd = h < N ? 1.0 : 0.0;
+                if (ev) __pipeline_memcpy_async(et + (t & 1) * 2 * GP_ROWS + threadIdx.x, ev + min(h, N - 1), 8, h < N ? 0 : 8);
             }
         }
         __pipeline_commit();

@@ -7,7 +7,8 @@ import pareben_b200 as pb
 lib = pb.load()
 lib.pareben_phase_cycles.restype = ctypes.c_int
 lib.pareben_phase_cycles.argtypes = [ctypes.POINTER(ctypes.c_ulonglong), ctypes.c_int]
-names = ["vfill", "contract", "quad", "gram", "sweep", "irls(all, incl. gram+sweep)", "delta_ml", "actions", "loglik/resid", "refresh(other)"]
+names = ["vfill", "contract", "quad", "gram", "sweep", "irls(all, incl. gram+sweep)", "delta_ml", "actions", "loglik/resid", "refresh(other)",
+         "  irls: predictor + line search", "  irls: weights, direction, tests", "  irls: H -> SIGMA copy", "  sweep: loads + stores"]
 g = np.load("tests/golden/inputs_bundled.npz")
 prior = sys.argv[1] if len(sys.argv) > 1 else "binomial"
 if prior == "binomial":
