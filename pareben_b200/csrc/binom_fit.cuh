@@ -17,8 +17,10 @@
 //    in-block symmetric sweep.
 #pragma once
 #include "common.cuh"
-#include "gauss_fit.cuh"
+#include "contract.cuh"
+#include "linalg.cuh"
 #include "tc_contract.cuh"
+#include "eben_step.cuh"
 
 namespace pareben {
 
@@ -220,7 +222,6 @@ __device__ void binom_fit(const Problem &P, const FoldData &F, const Variant &v,
                           double alpha_en, const FitTask &task, const FitOutputs &out, double *sV, const Scratch &sc)
 {
     const int N = F.ntr, K = P.K, Kc = P.Kc, cap = P.cap, T = blockDim.x, LD = phi_ld(N);   // cap counts the intercept slot
-    const int lane_ = threadIdx.x & 31, wid_ = threadIdx.x >> 5, nw_ = T >> 5;
     const double *X = F.Xtr, *t = F.ytr, *scale = F.scale;
     BinomState b; b.M = 2; b.n_unused = 0; b.status = 0; b.flops = 0; b.tc_calls = 0; b.at_mode = false;
     for (int j = threadIdx.x; j < cap + 1; j += T) { if (j < cap) s.grow[j] = j; s.alpha[j] = 0; s.mu[j] = 0; }
@@ -303,191 +304,148 @@ __device__ void binom_fit(const Problem &P, const FoldData &F, const Variant &v,
             i_iter++;
             const double logl0 = loglik;
             Decision d = delta_ml<EPIS, true>(s, b.M - 1, N, Kc, lambda, alpha_en, 0.0, 0.0, iter, i_iter, sc);
-            int nu = d.nu, worthwhile;
-            if (selected == ACT_TERM && !ini_removed && b.M > 2) nu = -1;             // :559-563
-            if (nu == -1 && ini_removed) { worthwhile = 0; selected = ACT_TERM; }
-            else if (nu == -1 && !ini_removed && b.M > 2) {                           // :570-579
-                worthwhile = 1; nu = initial - 1;
+            n_update = choose_block(s, v, d, b.M - 1, Kc, initial, selected, ini_removed, sc);
+            for (int iu = 0; iu < n_update; iu++) {
                 __syncthreads();
-                if (threadIdx.x == 0) { s.action[nu] = ACT_DEL; s.block[0] = nu; }
-                __syncthreads();
-                n_update = 1; ini_removed = 1; selected = ACT_DEL;
-            } else {
-                worthwhile = 1;
-                const int best_is_add = s.action[nu] == ACT_ADD, best_is_del = s.action[nu] == ACT_DEL;
-                double cutoff = d.best * (best_is_add ? v.n_add : 1.0);
-                if (cutoff < v.ml_delta) cutoff = v.ml_delta;
-                n_update = block_compact(Kc, [&](int c) { return s.dml[c] >= cutoff; }, s.block, nullptr, 0, sc);
-                if (best_is_del && n_update > 1) n_update = 1;                        // :607
-                if (n_update == 0) worthwhile = 0;
-            }
-            if (!worthwhile) selected = ACT_TERM;
-            if (worthwhile) {
-                for (int iu = 0; iu < n_update; iu++) {
+                const int nu = s.block[iu];
+                selected = s.action[nu];
+                const double new_alpha = s.aroot[nu];
+                { PHASE(PH_ACTIONS);
+                const bool need_sq = iu != n_update - 1;      // S/Q only matter to later actions of this block
+                find_slot(s, nu, b.M - 1, jj, selected, b.status);
+                if (selected == ACT_REEST && fabs(log(new_alpha) - log(s.alpha[jj])) <= v.reest_tol && !d.any_delete)
+                    selected = ACT_TERM;                                          // :663-670
+                const int M = b.M;
+                if (selected == ACT_REEST) {                                      // ActionRes*, :1127-1203
+                    const int j1 = jj + 1;
+                    const double old = s.alpha[jj];
+                    const double kappa = 1.0 / (s.sigma[j1 * M + j1] + 1.0 / (new_alpha - old));
+                    const double mujj = s.mu[j1];
+                    const double *sj = s.sigma + j1 * M;
                     __syncthreads();
-                    nu = s.block[iu];
-                    selected = s.action[nu];
-                    const double new_alpha = s.aroot[nu];
-                    { PHASE(PH_ACTIONS);
-                    const bool need_sq = iu != n_update - 1;      // S/Q only matter to later actions of this block
-                    if (selected == ACT_REEST || selected == ACT_DEL) {
-                        const int a = s.amap[nu];
-                        if (a >= 0) jj = a;                        // stale jj kept when the search fails (:629-636)
-                        if (jj < 0 || jj >= b.M - 1) { b.status |= ST_NOT_PD; selected = ACT_TERM; }
+                    if (threadIdx.x == 0) s.alpha[jj] = new_alpha;
+                    mu_reest(s.mu, M, sj, mujj, kappa);
+                    sigma_reest(s.sigma, s.sigma_new, M, j1, kappa);
+                    __syncthreads();
+                    { double *tp = s.sigma; s.sigma = s.sigma_new; s.sigma_new = tp; }
+                    if (need_sq) {   // reads the UPDATED row j1 (the copy precedes the loop, :1166, 1191)
+                        const double *sn = s.sigma + j1 * M;
+                        cache_dot(s, M, Kc, sn, [&](int c, double z) {
+                            s.S_in[c] += z * z * kappa;
+                            s.Q_in[c] += mujj * kappa * z;
+                        });
+                        if (threadIdx.x == 0) b.flops += 2.0 * Kc * (double)M;
                     }
-                    if (selected == ACT_REEST && fabs(log(new_alpha) - log(s.alpha[jj])) <= v.reest_tol && !d.any_delete)
-                        selected = ACT_TERM;                                          // :663-670
-                    const int M = b.M;
-                    if (selected == ACT_REEST) {                                      // ActionRes*, :1127-1203
-                        const int j1 = jj + 1;
-                        const double old = s.alpha[jj];
-                        const double kappa = 1.0 / (s.sigma[j1 * M + j1] + 1.0 / (new_alpha - old));
-                        const double mujj = s.mu[j1];
-                        const double *sj = s.sigma + j1 * M;
-                        __syncthreads();
-                        if (threadIdx.x == 0) s.alpha[jj] = new_alpha;
-                        for (int i = threadIdx.x; i < M; i += T) s.mu[i] += -mujj * kappa * sj[i];
-                        for (int j = wid_; j < M; j += nw_)                      // warps own columns, lanes rows: no integer division
-                            for (int i = lane_; i < M; i += 32) {
-                                const int idx = j * M + i;
-                                s.sigma_new[idx] = s.sigma[idx] - kappa * sj[i] * sj[j];
-                            }
-                        __syncthreads();
-                        { double *tp = s.sigma; s.sigma = s.sigma_new; s.sigma_new = tp; }
-                        if (need_sq) {   // reads the UPDATED row j1 (the copy precedes the loop, :1166, 1191)
-                            const double *sn = s.sigma + j1 * M;
-                            cache_dot(s, M, Kc, sn, [&](int c, double z) {
-                                s.S_in[c] += z * z * kappa;
-                                s.Q_in[c] += mujj * kappa * z;
-                            });
-                            if (threadIdx.x == 0) b.flops += 2.0 * Kc * (double)M;
-                        }
-                    } else if (selected == ACT_ADD) {                                 // ActionAdd*, :830-1003
-                        const int n_used = M - 1;
-                        if (n_used + 1 > cap - 1) { b.status |= ST_CAP; selected = ACT_TERM; }
-                        else {
-                            {
-                                Cand<EPIS> cd(nu, K);
-                                const double sc_nu = scale[nu], isc = 1 / sc_nu;
-                                for (int h = threadIdx.x; h < N; h += T) {
-                                    const double x = cd.at(X + (size_t)h * K);
-                                    s.phinew[h] = EPIS ? x / sc_nu : x * isc;         // NeFull.c:253-262 vs NEmainEff.c:643-646
-                                }
-                            }
-                            __syncthreads();
-                            const int grow_new = s.grow[M];
-                            if (need_sq) {
-                                contract_x<EPIS>(F, K, Kc, 1, 0,
-                                    [&](int) -> const double * { return s.phinew; },
-                                    [&](int, bool &dv) -> double * { dv = true; return s.G + (size_t)grow_new * Kc; }, sV, s.w1);
-                            }
-                            {   // tmp = PHI' (w o phi_new), one warp per active column
-                                const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, nw = T >> 5;
-                                for (int i = wid; i < M; i += nw) {
-                                    const double *p = s.phi + (size_t)i * LD;
-                                    double z = 0;
-                                    for (int h = lane; h < N; h += 32) z = fma(p[h], s.w1[h] * s.phinew[h], z);
-                                    z = warp_sum(z);
-                                    if (lane == 0) s.tmp[i] = z;
-                                }
-                            }
-                            __syncthreads();
-                            for (int i = threadIdx.x; i < M; i += T) {
-                                double z = 0;
-                                for (int j = 0; j < M; j++) z = fma(s.sigma[i * M + j], s.tmp[j], z);
-                                s.u[i] = z;
-                            }
-                            for (int h = N + threadIdx.x; h < LD; h += T) s.phi[(size_t)M * LD + h] = 0;
+                } else if (selected == ACT_ADD) {                                 // ActionAdd*, :830-1003
+                    const int n_used = M - 1;
+                    if (n_used + 1 > cap - 1) { b.status |= ST_CAP; selected = ACT_TERM; }
+                    else {
+                        {
+                            Cand<EPIS> cd(nu, K);
+                            const double sc_nu = scale[nu], isc = 1 / sc_nu;
                             for (int h = threadIdx.x; h < N; h += T) {
-                                s.phi[(size_t)M * LD + h] = s.phinew[h];
-                                if (M < PHIT_LD) s.phit[(size_t)h * PHIT_LD + M] = s.phinew[h];
+                                const double x = cd.at(X + (size_t)h * K);
+                                s.phinew[h] = EPIS ? x / sc_nu : x * isc;         // NeFull.c:253-262 vs NEmainEff.c:643-646
                             }
-                            const double s_ii = 1.0 / (new_alpha + s.S_in[nu]);
-                            const double mu_i = s_ii * s.Q_in[nu];
-                            __syncthreads();
-                            if (threadIdx.x == 0) { s.alpha[n_used] = new_alpha; s.mu[M] = mu_i; }
-                            for (int i = threadIdx.x; i < M; i += T) s.mu[i] += -mu_i * s.u[i];
-                            const int M1 = M + 1;
-                            for (int j = wid_; j < M1; j += nw_)
-                                for (int i = lane_; i < M1; i += 32) {
-                                    double val;
-                                    if (i < M && j < M) val = s.sigma[j * M + i] + (s_ii * s.u[i]) * s.u[j];
-                                    else if (i == M && j == M) val = s_ii;
-                                    else val = -s_ii * s.u[i < M ? i : j];
-                                    s.sigma_new[j * M1 + i] = val;
-                                }
-                            if (need_sq) {
-                                cache_dot(s, M, Kc, s.u, [&](int c, double z) {
-                                    const double mci = s.G[(size_t)grow_new * Kc + c] - z;
-                                    s.S_in[c] -= mci * mci * s_ii;
-                                    s.Q_in[c] -= mu_i * mci;
-                                });
-                            }
-                            __syncthreads();
-                            if (threadIdx.x == 0) {
-                                s.used[n_used] = nu + 1;
-                                s.amap[nu] = n_used;
-                                const int p = s.upos[nu], nun = b.n_unused - 1;
-                                if (p < nun) { const int lastc = s.unused[nun] - 1; s.unused[p] = lastc + 1; s.upos[lastc] = p; }
-                                if (need_sq) b.flops += 2.0 * N * (double)Kc + 2.0 * Kc * (double)M;
-                            }
-                            { double *tp = s.sigma; s.sigma = s.sigma_new; s.sigma_new = tp; }
-                            b.n_unused--;
-                            b.M = M + 1;
                         }
-                    } else if (selected == ACT_DEL) {                                 // ActionDel*, :1010-1121
-                        const int j1 = jj + 1, lastj = M - 1;
-                        const double *sj = s.sigma + j1 * M;
-                        const double sjj = sj[j1];
-                        const double mujj = s.mu[j1];
-                        const double al_last = s.alpha[lastj - 1];
                         __syncthreads();
-                        for (int i = threadIdx.x; i < M; i += T) s.mu[i] = s.mu[i] - mujj * sj[i] / sjj;
+                        const int grow_new = s.grow[M];
                         if (need_sq) {
-                            cache_dot(s, M, Kc, sj, [&](int c, double z) {
-                                s.S_in[c] += z * z / sjj;
-                                s.Q_in[c] += z * mujj / sjj;
-                            });
-                            if (threadIdx.x == 0) b.flops += 2.0 * Kc * (double)M;
+                            contract_x<EPIS>(F, K, Kc, 1, 0,
+                                [&](int) -> const double * { return s.phinew; },
+                                [&](int, bool &dv) -> double * { dv = true; return s.G + (size_t)grow_new * Kc; }, sV, s.w1);
                         }
-                        for (int j = wid_; j < lastj; j += nw_) {
-                            const int sjx = (j == j1) ? lastj : j;
-                            for (int i = lane_; i < lastj; i += 32) {
-                                const int si = (i == j1) ? lastj : i;
-                                s.sigma_new[j * lastj + i] = EPIS ? s.sigma[sjx * M + si] - sj[si] / sjj * sj[sjx]      // NeFull.c:1612
-                                                                  : s.sigma[sjx * M + si] - sj[si] * sj[sjx] / sjj;     // NEmainEff.c:1069
+                        {   // tmp = PHI' (w o phi_new), one warp per active column
+                            const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, nw = T >> 5;
+                            for (int i = wid; i < M; i += nw) {
+                                const double *p = s.phi + (size_t)i * LD;
+                                double z = 0;
+                                for (int h = lane; h < N; h += 32) z = fma(p[h], s.w1[h] * s.phinew[h], z);
+                                z = warp_sum(z);
+                                if (lane == 0) s.tmp[i] = z;
                             }
                         }
+                        __syncthreads();
+                        for (int i = threadIdx.x; i < M; i += T) {
+                            double z = 0;
+                            for (int j = 0; j < M; j++) z = fma(s.sigma[i * M + j], s.tmp[j], z);
+                            s.u[i] = z;
+                        }
+                        for (int h = N + threadIdx.x; h < LD; h += T) s.phi[(size_t)M * LD + h] = 0;
                         for (int h = threadIdx.x; h < N; h += T) {
-                            if (j1 != lastj) {
-                                const double pv = s.phi[(size_t)lastj * LD + h];
-                                s.phi[(size_t)j1 * LD + h] = pv;
-                                if (j1 < PHIT_LD) s.phit[(size_t)h * PHIT_LD + j1] = pv;
-                            }
-                            if (lastj < PHIT_LD) s.phit[(size_t)h * PHIT_LD + lastj] = 0;     // vacated slot back to zero
+                            s.phi[(size_t)M * LD + h] = s.phinew[h];
+                            if (M < PHIT_LD) s.phit[(size_t)h * PHIT_LD + M] = s.phinew[h];
+                        }
+                        const double s_ii = 1.0 / (new_alpha + s.S_in[nu]);
+                        const double mu_i = s_ii * s.Q_in[nu];
+                        __syncthreads();
+                        if (threadIdx.x == 0) s.alpha[n_used] = new_alpha;
+                        mu_add(s.mu, M, s.u, mu_i);
+                        sigma_add(s.sigma, s.sigma_new, M, s.u, s_ii);
+                        if (need_sq) {
+                            cache_dot(s, M, Kc, s.u, [&](int c, double z) {
+                                const double mci = s.G[(size_t)grow_new * Kc + c] - z;
+                                s.S_in[c] -= mci * mci * s_ii;
+                                s.Q_in[c] -= mu_i * mci;
+                            });
                         }
                         __syncthreads();
                         if (threadIdx.x == 0) {
-                            if (j1 != lastj) {
-                                s.alpha[jj] = al_last;
-                                s.mu[j1] = s.mu[lastj];
-                                const int gr = s.grow[j1]; s.grow[j1] = s.grow[lastj]; s.grow[lastj] = gr;
-                            }
-                            const int moved = s.used[lastj - 1];
-                            s.used[jj] = moved;
-                            s.amap[nu] = -1;
-                            if (jj != lastj - 1) s.amap[moved - 1] = jj;
-                            s.unused[b.n_unused] = nu + 1; s.upos[nu] = b.n_unused;
+                            s.used[n_used] = nu + 1;
+                            s.amap[nu] = n_used;
+                            const int p = s.upos[nu], nun = b.n_unused - 1;
+                            if (p < nun) { const int lastc = s.unused[nun] - 1; s.unused[p] = lastc + 1; s.upos[lastc] = p; }
+                            if (need_sq) b.flops += 2.0 * N * (double)Kc + 2.0 * Kc * (double)M;
                         }
                         { double *tp = s.sigma; s.sigma = s.sigma_new; s.sigma_new = tp; }
-                        b.n_unused++;
-                        b.M = M - 1;
-                        if (nu + 1 == initial) ini_removed = 1;                       // :744
+                        b.n_unused--;
+                        b.M = M + 1;
+                    }
+                } else if (selected == ACT_DEL) {                                 // ActionDel*, :1010-1121
+                    const int j1 = jj + 1, lastj = M - 1;
+                    const double *sj = s.sigma + j1 * M;
+                    const double sjj = sj[j1];
+                    const double mujj = s.mu[j1];
+                    const double al_last = s.alpha[lastj - 1];
+                    __syncthreads();
+                    if (need_sq) {
+                        cache_dot(s, M, Kc, sj, [&](int c, double z) {
+                            s.S_in[c] += z * z / sjj;
+                            s.Q_in[c] += z * mujj / sjj;
+                        });
+                        if (threadIdx.x == 0) b.flops += 2.0 * Kc * (double)M;
+                    }
+                    sigma_delete<EPIS>(s.sigma, s.sigma_new, M, j1, nullptr);    // NeFull.c:1612 vs NEmainEff.c:1069
+                    mu_delete(s.mu, M, sj, sjj, mujj);
+                    for (int h = threadIdx.x; h < N; h += T) {
+                        if (j1 != lastj) {
+                            const double pv = s.phi[(size_t)lastj * LD + h];
+                            s.phi[(size_t)j1 * LD + h] = pv;
+                            if (j1 < PHIT_LD) s.phit[(size_t)h * PHIT_LD + j1] = pv;
+                        }
+                        if (lastj < PHIT_LD) s.phit[(size_t)h * PHIT_LD + lastj] = 0;     // vacated slot back to zero
                     }
                     __syncthreads();
+                    if (threadIdx.x == 0) {
+                        if (j1 != lastj) {
+                            s.alpha[jj] = al_last;
+                            s.mu[j1] = s.mu[lastj];
+                            const int gr = s.grow[j1]; s.grow[j1] = s.grow[lastj]; s.grow[lastj] = gr;
+                        }
+                        const int moved = s.used[lastj - 1];
+                        s.used[jj] = moved;
+                        s.amap[nu] = -1;
+                        if (jj != lastj - 1) s.amap[moved - 1] = jj;
+                        s.unused[b.n_unused] = nu + 1; s.upos[nu] = b.n_unused;
                     }
-                    if (iu == n_update - 1) binom_full_stat<EPIS, TC>(P, F, s, b, sV, sc);          // after the last action of the block (:749-762)
+                    { double *tp = s.sigma; s.sigma = s.sigma_new; s.sigma_new = tp; }
+                    b.n_unused++;
+                    b.M = M - 1;
+                    if (nu + 1 == initial) ini_removed = 1;                       // :744
                 }
+                __syncthreads();
+                }
+                if (iu == n_update - 1) binom_full_stat<EPIS, TC>(P, F, s, b, sV, sc);          // after the last action of the block (:749-762)
             }
             if (selected == ACT_TERM && ini_removed) last = 1;
             if ((i_iter == it_max && b.M == 2) || i_iter > it_max) last = 1;
@@ -544,29 +502,9 @@ __device__ void binom_fit(const Problem &P, const FoldData &F, const Variant &v,
     if (F.nte > 0 && !isfinite(ll)) b.status |= ST_NONFINITE;      // (no held-out rows in an all-rows fit: nothing to score)
     if (threadIdx.x == 0) {
         const int o = task.out_index;
-        if (out.fold_err) out.fold_err[o] = ll;
-        if (out.status) out.status[o] = b.status;
-        if (out.n_selected) out.n_selected[o] = nsel;
-        if (out.n_iter) out.n_iter[o] = iter;
-        if (out.flops) { atomicAdd(out.flops, b.flops); if (b.tc_calls > 0) atomicAdd(out.flops + 2, b.tc_calls); }
-        if (out.m_out) {          // full-model record of fit o (pareben_fit_batch); slot 0 is the intercept
-            out.m_out[o] = M - 1;
-            double wd = 0;
-            for (int i = 0; i < M; i++) {
-                double z = 0;
-                for (int j = 0; j < M; j++) z += s.mu[j] * s.H[i * M + j];
-                wd += z * s.mu[i];
-            }
-            const size_t r = (size_t)o * out.dump_ld;
-            for (int i = 1; i < M; i++) {
-                const int c = s.used[i - 1] - 1;
-                out.used_out[r + i - 1] = s.used[i - 1];
-                out.beta_out[r + i - 1] = s.mu[i] / scale[c];
-                out.var_out[r + i - 1] = s.sigma[i * M + i] / (scale[c] * scale[c]);
-            }
-            out.scalars_out[4 * (size_t)o + 0] = wd; out.scalars_out[4 * (size_t)o + 1] = s.mu[0];
-            out.scalars_out[4 * (size_t)o + 2] = s.sigma[0]; out.scalars_out[4 * (size_t)o + 3] = loglik;
-        }
+        write_fit_outputs(out, o, ll, b.status, nsel, iter, b.flops, 0, b.tc_calls);
+        if (out.m_out)            // slot 0 is the intercept
+            write_record(out, o, M, 1, s.mu, s.H, s.sigma, s.used, [&](int k) { return scale[s.used[k] - 1]; }, s.mu[0], s.sigma[0], loglik);
     }
     __syncthreads();
 }

@@ -358,7 +358,7 @@ static void ensure_slabs(pareben_problem *p)
     {
         // Block size: measured on B200 (config 2 / bundled Gaussian): 256 threads x 2 blocks per SM beats
         // 128 x 4 (-5 % / -43 %) and 64 x 8 (-40 % / -70 %) (measured with an earlier build that had a run-time block size).
-        p->threads = FIT_THREADS_HOST;     // gram_tiled() maps 16 x 16 register blocks onto exactly 256 threads
+        p->threads = FIT_THREADS_HOST;     // sweep_regs() and the fused gram_pipe() run only at exactly 256 threads
         static int occ_cache[5] = {0, 0, 0, 0, 0};
         int &occ = occ_cache[p->tc ? 4 : (p->prior == PAREBEN_BINOMIAL ? 2 : 0) + (p->epis ? 1 : 0)];
         if (!occ) {

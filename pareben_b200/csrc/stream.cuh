@@ -37,6 +37,7 @@
 //                           delta-ML and appends to the fit's ADD list; nothing of length Kc is ever stored.
 #pragma once
 #include "common.cuh"
+#include "eben_step.cuh"
 
 namespace pareben {
 
@@ -86,15 +87,10 @@ struct StreamFit {
 //              (need = n_add * best; thr only ever grows: atomicMax on its bit pattern).
 __device__ inline double lub_of(double q2, double sl, double l1, double l2)
 {   // upper bound of delta-ML at Q^2 = q2; +inf where the closed form cannot be evaluated (keeps the candidate)
-    const double a = sl - q2 + 2 * l1 + l2;
-    if (!(a < 0)) return 0.0;
-    const double b = (sl + l2) * (sl + 4 * l1 + l2);
-    const double gmm = 2 * l1 * (sl + l2) * (sl + l2);
-    const double dl = b * b - 4 * a * gmm;
-    if (!(dl > 0)) return INFINITY;
-    const double r = (-b - sqrt(dl)) / (2 * a);
+    if (!(add_a(sl, q2, l1, l2) < 0)) return 0.0;
+    double r, L;
+    if (!add_root(sl, q2, l1, l2, r, L)) return INFINITY;
     if (!(r > 0)) return INFINITY;
-    const double L = (log(r / (r + sl + l2)) + q2 / (r + sl + l2)) * 0.5 - l1 / r;
     return L == L ? L : INFINITY;
 }
 

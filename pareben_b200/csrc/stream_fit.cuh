@@ -11,7 +11,8 @@
 //   * column norms are computed when a column enters the model (exact sums for genotype codes).
 #pragma once
 #include "stream.cuh"
-#include "gauss_fit.cuh"
+#include "linalg.cuh"
+#include "eben_step.cuh"
 
 namespace pareben {
 
@@ -125,17 +126,7 @@ stream_advance_kernel(Problem P, Variant v, StreamFit *fits, int n_fits, StreamS
                 if (threadIdx.x == 0) s.ascale[0] = sc0;
                 for (int h = threadIdx.x; h < LD; h += T) s.phi[h] = h < N ? s.phinew[h] * isc : 0.0;
                 __syncthreads();
-                const double var = block_var(s.t, N, sc);
-                if (!EPIS) s.beta = 1 / (var * 0.01 + 1e-10);
-                else { double sd = sqrt(var); if (sd < 1e-6) sd = 1e-6; s.beta = 1 / ((sd * 0.1) * (sd * 0.1)); }
-                double p = 0, q = 0;
-                for (int h = threadIdx.x; h < N; h += T) { p = fma(s.phi[h], s.phi[h], p); q = fma(s.phi[h], s.t[h], q); }
-                block_sum2(p, q, sc);
-                p *= s.beta; q *= s.beta;
-                double a = p * p / (q * q - p);
-                if (a < 0) a = v.init_alpha_max;
-                if (a > v.init_alpha_max) a = v.init_alpha_max;
-                if (threadIdx.x == 0) s.alpha[0] = a;
+                gauss_start<EPIS>(s.phi, s.t, N, v, s.beta, s.alpha, sc);
             }
             __syncthreads();
             for (int j = threadIdx.x; j < cap; j += T) s.gamma[j] = 0;               // gamma is Calloc'ed per call (:344)
@@ -233,29 +224,19 @@ stream_advance_kernel(Problem P, Variant v, StreamFit *fits, int n_fits, StreamS
                 const double si = s.s_in[j], qi = s.beta_s * s.q_in[j];
                 const double aj = s.alpha[j];
                 const double den = aj - si;
-                const double qo = aj * qi / den, so = aj * si / den;
+                const double qo = aj * qi / den, so = aj * si / den, q2 = qo * qo;
                 double d_ml = 0; int act = ACT_NONE;
-                const double a = so - qo * qo + 2 * l1 + l2;
-                const double b = (so + l2) * (so + 4 * l1 + l2);
-                const double gmm = 2 * l1 * (so + l2) * (so + l2);
-                const double dl = b * b - 4 * a * gmm;
-                if (a < 0 && dl > 0) {
-                    const double r = (-b - sqrt(dl)) / (2 * a);
-                    const double L = (log(r / (r + so + l2)) + qo * qo / (r + so + l2)) * 0.5 - l1 / r;
+                double r, L;
+                if (add_root(so, q2, l1, l2, r, L)) {
                     if (L > 0) {
                         s.aroot_in[j] = r + l2;
                         act = ACT_REEST;
-                        const double o = aj - l2;
-                        d_ml = 0.5 * (log(r * (o + so + l2) / (o * (r + so + l2))) +
-                                      qo * qo * (1 / (r + so + l2) - 1 / (o + so + l2))) -
-                               l1 * (1 / r - 1 / o);
+                        d_ml = reest_gain(so, q2, l1, l2, r, aj);
                     }
                 } else if (M0 > 1) {
                     f_del = 1;
                     act = ACT_DEL;
-                    const double o = aj - l2;
-                    const double L = (log(o / (o + so + l2)) + qo * qo / (o + so + l2)) * 0.5 - l1 / o;
-                    d_ml = -L;
+                    d_ml = delete_gain(so, q2, l1, l2, aj);
                 }
                 s.dml_in[j] = d_ml; s.act_in[j] = act;
             }
@@ -370,12 +351,8 @@ stream_advance_kernel(Problem P, Variant v, StreamFit *fits, int n_fits, StreamS
                         const double *sj = s.sigma + jj * M;
                         __syncthreads();
                         if (threadIdx.x == 0) s.alpha[jj] = new_alpha;
-                        for (int i = threadIdx.x; i < M; i += T) s.mu[i] += -mujj * kappa * sj[i];
-                        for (int j = wid_; j < M; j += nw_)
-                            for (int i = lane_; i < M; i += 32) {
-                                const int idx = j * M + i;
-                                s.sigma_new[idx] = s.sigma[idx] - kappa * sj[i] * sj[j];
-                            }
+                        sigma_reest(s.sigma, s.sigma_new, M, jj, kappa);
+                        mu_reest(s.mu, M, sj, mujj, kappa);
                         updated = true;
                     } else if (s.selected == ACT_ADD) {                                    // ActionAdd*, :1585-1723
                         if (M + 1 > cap) { s.status |= ST_CAP; s.selected = ACT_TERM; }
@@ -431,17 +408,8 @@ stream_advance_kernel(Problem P, Variant v, StreamFit *fits, int n_fits, StreamS
                             const double mu_i = s_ii * Q_nu;
                             __syncthreads();
                             if (threadIdx.x == 0) { s.alpha[M] = new_alpha; s.ascale[M] = sc_nu; }
-                            for (int i = threadIdx.x; i < M; i += T) s.mu[i] += -mu_i * s.u[i];
-                            if (threadIdx.x == 0) s.mu[M] = mu_i;
-                            const int M1 = M + 1;
-                            for (int j = wid_; j < M1; j += nw_)
-                                for (int i = lane_; i < M1; i += 32) {
-                                    double val;
-                                    if (i < M && j < M) val = s.sigma[j * M + i] + (s_ii * s.u[i]) * s.u[j];
-                                    else if (i == M && j == M) val = s_ii;
-                                    else val = -s_ii * s.u[i < M ? i : j];
-                                    s.sigma_new[j * M1 + i] = val;
-                                }
+                            mu_add(s.mu, M, s.u, mu_i);
+                            sigma_add(s.sigma, s.sigma_new, M, s.u, s_ii);
                             __syncthreads();
                             if (threadIdx.x == 0) s.used[M] = nu + 1;
                             s.M = M + 1;
@@ -454,7 +422,7 @@ stream_advance_kernel(Problem P, Variant v, StreamFit *fits, int n_fits, StreamS
                         const double sjj = sj[jj];
                         const double al_last = s.alpha[lastj], sc_last = s.ascale[lastj];
                         __syncthreads();
-                        for (int i = threadIdx.x; i < M; i += T) s.mu[i] = s.mu[i] - mujj * sj[i] / sjj;
+                        mu_delete(s.mu, M, sj, sjj, mujj);
                         __syncthreads();
                         // the remainder of the deleted weight stays in the reference's Q array: carry it in d
                         const double mu_drop = s.mu[jj];
@@ -462,21 +430,8 @@ stream_advance_kernel(Problem P, Variant v, StreamFit *fits, int n_fits, StreamS
                             s.d[h] = fma(mu_drop, s.phi[(size_t)jj * LD + h], s.d[h]);
                             s.phi[(size_t)jj * LD + h] = s.phi[(size_t)lastj * LD + h];
                         }
-                        if (jj != lastj) {                                                 // PHI'PHI: last row/column into slot jj
-                            for (int i = threadIdx.x; i < lastj; i += T) {
-                                if (i == jj) s.ptp[(size_t)jj * cap + jj] = s.ptp[(size_t)lastj * cap + lastj];
-                                else { s.ptp[(size_t)i * cap + jj] = s.ptp[(size_t)i * cap + lastj]; s.ptp[(size_t)jj * cap + i] = s.ptp[(size_t)lastj * cap + i]; }
-                            }
-                        }
-                        for (int i = threadIdx.x; i < M; i += T) s.colk[i] = sj[i] / sjj;
-                        __syncthreads();
-                        for (int j = wid_; j < lastj; j += nw_) {
-                            const int sjx = (j == jj) ? lastj : j;
-                            for (int i = lane_; i < lastj; i += 32) {
-                                const int si = (i == jj) ? lastj : i;
-                                s.sigma_new[j * lastj + i] = s.sigma[sjx * M + si] - s.colk[si] * sj[sjx];
-                            }
-                        }
+                        ptp_move_last(s.ptp, cap, jj, lastj);
+                        sigma_delete<true>(s.sigma, s.sigma_new, M, jj, s.colk);
                         __syncthreads();
                         // the basis that leaves is the one in slot jj: not candidate nu when the forced removal's search of Used
                         // failed (gauss_fit.cuh, delete action) -- it is then in neither list until the next outer iteration
@@ -572,49 +527,13 @@ stream_advance_kernel(Problem P, Variant v, StreamFit *fits, int n_fits, StreamS
 
     // ---------------- hold-out score (R/GetModelError.R:6-32) ----------------
     const int M = s.M;
-    __syncthreads();
-    for (int i = threadIdx.x; i < M; i += T) s.tmp[i] = s.mu[i] / s.ascale[i];              // Beta[,3] (:221)
-    __syncthreads();
-    double sse = 0;
-    for (int h = threadIdx.x; h < F.nte; h += T) {
-        const double *xr = F.Xte + (size_t)h * K;
-        double pred = 0;
-        for (int i = 0; i < M; i++) {
-            const double w = s.tmp[i];
-            if (w != 0) { Cand<EPIS> cd(s.used[i] - 1, K); pred = fma(cd.at(xr), w, pred); }
-        }
-        const double r = F.yte[h] - (s.b + pred);
-        sse = fma(r, r, sse);
-    }
-    sse = block_sum(sse, sc);
-    int nsel = 0;
-    for (int i = 0; i < M; i++) nsel += s.tmp[i] != 0;
-    if (!isfinite(sse)) s.status |= ST_NONFINITE;
+    auto norm = [&](int i) { return s.ascale[i]; };
+    int nsel;
+    const double sse = gauss_holdout_sse<EPIS>(F, K, M, s.mu, s.used, s.b, s.tmp, norm, nsel, s.status, sc);
     if (threadIdx.x == 0) {
         const int o = s.out_index;
-        if (out.fold_err) out.fold_err[o] = sse;
-        if (out.status) out.status[o] = s.status;
-        if (out.n_selected) out.n_selected[o] = nsel;
-        if (out.n_iter) out.n_iter[o] = s.iter;
-        if (out.flops) atomicAdd(out.flops, s.flops);
-        if (out.m_out) {          // full-model record of fit o (pareben_fit_batch)
-            out.m_out[o] = M;
-            double wd = 0;        // Wald score mu'H mu with H read at leading dimension M (:206-215)
-            for (int i = 0; i < M; i++) {
-                double z = 0;
-                for (int j = 0; j < M; j++) z += s.mu[j] * s.H[i * M + j];
-                wd += z * s.mu[i];
-            }
-            const size_t r = (size_t)o * out.dump_ld;
-            for (int i = 0; i < M; i++) {
-                out.used_out[r + i] = s.used[i];
-                out.beta_out[r + i] = s.mu[i] / s.ascale[i];
-                out.var_out[r + i] = s.sigma[i * M + i] / (s.ascale[i] * s.ascale[i]);
-            }
-            out.scalars_out[4 * (size_t)o + 0] = wd; out.scalars_out[4 * (size_t)o + 1] = s.b;
-            out.scalars_out[4 * (size_t)o + 2] = 0;
-            out.scalars_out[4 * (size_t)o + 3] = 1 / (s.beta + 1e-10);
-        }
+        write_fit_outputs(out, o, sse, s.status, nsel, s.iter, s.flops, 0, 0);
+        if (out.m_out) write_record(out, o, M, 0, s.mu, s.H, s.sigma, s.used, norm, s.b, 0, 1 / (s.beta + 1e-10));
         s.phase = SP_DONE;
         G = s;
     }

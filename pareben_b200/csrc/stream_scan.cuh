@@ -24,7 +24,8 @@
 // the advance kernel filters with the exact cutoff and sorts, so the result does not depend on the schedule).
 #pragma once
 #include "stream.cuh"
-#include "gauss_fit.cuh"
+#include "contract.cuh"
+#include "eben_step.cuh"
 
 namespace pareben {
 
@@ -51,13 +52,8 @@ __device__ inline double scan_decide(StreamFit *fit, int c, double so, double qo
 {
     const double l1 = fit->l1, l2 = fit->l2;
     for (int h = 0; h < fit->n_hidden; h++) if (fit->hidden[h] == c) return 0.0;       // in neither Used nor Unused
-    const double a = so - qo * qo + 2 * l1 + l2;
-    const double b = (so + l2) * (so + 4 * l1 + l2);
-    const double gm = 2 * l1 * (so + l2) * (so + l2);
-    const double dl = b * b - 4 * a * gm;
-    if (!(a < 0 && dl > 0)) return 0.0;
-    const double r = (-b - sqrt(dl)) / (2 * a);
-    const double L = (log(r / (r + so + l2)) + qo * qo / (r + so + l2)) * 0.5 - l1 / r;
+    double r = 0, L = 0;
+    if (!add_root(so, qo * qo, l1, l2, r, L)) return 0.0;
     if (!(L > 0)) return 0.0;
     if (GAUSS_MAIN) fit->any_add = 1;
     if (!(L >= fit->ml_delta)) return 0.0;

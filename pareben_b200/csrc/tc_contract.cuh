@@ -25,7 +25,7 @@
 // The MMA issue order, and with it every sum, depends on the row index only: exact duplicate columns tie exactly.
 #pragma once
 #include "common.cuh"
-#include "gauss_fit.cuh"
+#include "contract.cuh"
 
 namespace pareben {
 

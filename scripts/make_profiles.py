@@ -66,7 +66,7 @@ def func_starts(path):
         m = re.match(r"^(?:__device__|static __device__)\s+(?:inline\s+)?[\w:<> \*&]+?\s+(\w+)\s*\(", ln)
         if m: out.append((i, m.group(1)))
     return out
-starts = {f: func_starts(os.path.join(ROOT, "pareben_b200", "csrc", f)) for f in ("gauss_fit.cuh", "binom_fit.cuh", "common.cuh", "fit_kernel.cuh", "stream_scan.cuh", "stream_fit.cuh", "stream.cuh")}
+starts = {f: func_starts(os.path.join(ROOT, "pareben_b200", "csrc", f)) for f in ("gauss_fit.cuh", "binom_fit.cuh", "contract.cuh", "linalg.cuh", "eben_step.cuh", "common.cuh", "fit_kernel.cuh", "stream_scan.cuh", "stream_fit.cuh", "stream.cuh")}
 def region(f, line):
     best = f"{f}:(top)"
     for ln, nm in starts.get(f, []):

@@ -1,6 +1,6 @@
 // Microbenchmark of the tensor-core contraction in isolation (experiments only).
 // build: nvcc -gencode arch=compute_100a,code=sm_100a -O3 -fmad=false -std=c++17 -I../../pareben_b200/csrc -o mb_contract2 mb_contract2.cu
-#include "gauss_fit.cuh"
+#include "contract.cuh"
 #include <cstdio>
 #include <cstdlib>
 #include <vector>

@@ -5,7 +5,7 @@
 // each phase behind a barrier.  Prints cycles per call for M in {8, 24, 40, 56}.
 //   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -fmad=false -std=c++17 -o mb_linalg mb_linalg.cu
 #include "../../pareben_b200/csrc/common.cuh"
-#include "../../pareben_b200/csrc/gauss_fit.cuh"
+#include "../../pareben_b200/csrc/linalg.cuh"
 #include "../../pareben_b200/csrc/fit_kernel.cuh"
 #include <cstdio>
 #include <vector>

@@ -8,13 +8,13 @@
 // tc_close before it exits.
 //
 //   probe_tc          tc_contract (tc_contract.cuh): G[j][c] = x_c'(w o phi_j) / s_c for j < R, ze = X'e, bb = (X o X)'(w o phi_0)
-//   probe_contract_x  contract_x (gauss_fit.cuh), the form chosen as a fit chooses it: by R, ldt and whether bb is wanted
+//   probe_contract_x  contract_x (contract.cuh), the form chosen as a fit chooses it: by R, ldt and whether bb is wanted
 //   probe_cand_map    Cand<true>: candidate index -> loci (i, j) of the Epis numbering
 //
 // Return value: 0, a negative number for arguments the contraction does not accept (probe_last_error says which), or a
 // positive cudaError_t.
 #include "../../pareben_b200/csrc/common.cuh"
-#include "../../pareben_b200/csrc/gauss_fit.cuh"
+#include "../../pareben_b200/csrc/contract.cuh"
 #include "../../pareben_b200/csrc/tc_contract.cuh"
 #include "../../pareben_b200/csrc/layout.cuh"
 #include "../../pareben_b200/csrc/fit_kernel.cuh"

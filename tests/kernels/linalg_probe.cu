@@ -1,4 +1,4 @@
-// linalg_probe.cu -- test-only entry points into the dense linear algebra of a fit (gauss_fit.cuh), built by
+// linalg_probe.cu -- test-only entry points into the dense linear algebra of a fit (linalg.cuh, contract.cuh), built by
 // tests/test_gpu_linalg_kernels.py into its own shared library (libpareben.so gains nothing).
 //
 // Each entry copies host arrays into guarded device buffers (probe_call.cuh), runs ONE block with the fit kernels'
@@ -17,7 +17,8 @@
 // Return value: 0, -1 for arguments the kernel does not accept, -2 when a kernel wrote into a guard region
 // (probe_last_error says which), or a positive cudaError_t.
 #include "../../pareben_b200/csrc/common.cuh"
-#include "../../pareben_b200/csrc/gauss_fit.cuh"
+#include "../../pareben_b200/csrc/contract.cuh"
+#include "../../pareben_b200/csrc/linalg.cuh"
 #include "../../pareben_b200/csrc/fit_kernel.cuh"
 #include "probe_call.cuh"
 

@@ -148,7 +148,7 @@ def fma_exact(a, b, c):
 
 
 def div_by(a, b):
-    """gauss_fit.cuh div_by(a, b, 1/b): q = a r, then fma(fma(-q, b, a), r, q)."""
+    """contract.cuh div_by(a, b, 1/b): q = a r, then fma(fma(-q, b, a), r, q)."""
     r = 1.0 / b
     q = a * r
     return fma_exact(fma_exact(-q, b, a), r, q)

@@ -1,6 +1,6 @@
 """CPU references for the dense linear algebra of a fit (no GPU needed).
 
-tests/test_gpu_linalg_kernels.py holds the kernels of gauss_fit.cuh to three kinds of reference built here:
+tests/test_gpu_linalg_kernels.py holds the kernels of linalg.cuh and contract.cuh to three kinds of reference built here:
 
 * Bit-exact C restatements (tests/kernels/linalg_ref.c, gcc -ffp-contract=off) of the kernels whose arithmetic is plain
   IEEE double in a fixed order: sweep_regs, sweep_core, quad_forms_simt<8>, gram_pipe, cache_dot, sym_matvec_row.
